@@ -17,7 +17,11 @@ through the product's scene driver (lfsr_b200.scene.SceneRunner - what train.tes
   cpu_baseline         the reference algorithm on the host cores (oracle port)
 N > 1: every rank runs its own scenes for `value` (weak scaling, no data-path collective).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model NAME] [--quick]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model NAME] [--quick] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed headline step of --impl ours returned (rank 0): sr.npy (float32 SR mosaic),
+metric_sums.npy (float64 per-view sums of squared error and SSIM) and psnr_ssim.npy (float64). Inputs and weights are
+seeded, so two builds run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -62,7 +66,12 @@ def parse():
     ap.add_argument("--quick", action="store_true", help="headline + parity + roofline only (no configs / eager / sustained legs)")
     ap.add_argument("--no-tc", action="store_true", help="keep every conv on the fp32 CUDA-core kernels")
     ap.add_argument("--sustained-s", type=float, default=5.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (at most 64 MB in all)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def scene_side(batch: int) -> int:
@@ -178,6 +187,9 @@ def run_reference(a):
     if rank != 0:
         return
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if a.dump_outputs:
+        print("[bench] --dump-outputs is ignored with --impl reference (it times a smaller sample of the workload)",
+              file=sys.stderr)
     patches = 16           # bounded sample: a 4x4-patch scene per step (~1.5 s of host work on the GPU box)
     import lfsr_b200
     torch.manual_seed(1234)                                  # the product arm's weights: seeded constructor-default init
@@ -209,6 +221,32 @@ def cuda_time(fn, iters: int, warmup: int = 1, sync=None):
     e1.record()
     torch.cuda.synchronize()
     return e0.elapsed_time(e1) / iters
+
+
+DUMP_BUDGET = 64 * 10 ** 6
+DUMP_HEADER = 4096          # room left for each .npy header
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Write each float32 / float64 array as out_dir/<name>.npy, smallest first, within DUMP_BUDGET bytes in all. An array
+    larger than what is left is replaced by a fixed sample of its flattened elements (RandomState(0), sorted indices): the
+    same arguments give the same sample, so the files of two builds stay comparable."""
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BUDGET
+    written = {}
+    for name, arr in sorted(arrays.items(), key=lambda kv: kv[1].nbytes):
+        arr = np.ascontiguousarray(arr)
+        assert arr.dtype in (np.float32, np.float64), (name, arr.dtype)
+        keep = (left - DUMP_HEADER) // arr.itemsize
+        if keep <= 0:
+            raise ValueError(f"--dump-outputs: no room left for {name}")
+        if arr.size > keep:
+            idx = np.sort(np.random.RandomState(0).choice(arr.size, keep, replace=False))
+            arr = arr.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+        left -= arr.nbytes + DUMP_HEADER
+        written[name] = list(arr.shape)
+    return written
 
 
 def measure_tf32_peak(dev, n: int = 8192):
@@ -363,6 +401,13 @@ def main():
     ms_total, launches = timed(step_resident, a.steps, max(a.warmup, 3))
     clocks = sampler.stop() if sampler else None
     value = a.batch * world * a.steps / (ms_total * 1e-3)
+    # slot 0 now holds the last timed step's outputs; the e2e leg below reuses it
+    if a.dump_outputs and rank == 0:
+        acc = slot0["acc"].cpu().numpy()
+        written = dump_outputs(a.dump_outputs, {
+            "sr": slot0["mosaic"].cpu().numpy(), "metric_sums": acc,
+            "psnr_ssim": np.array(runner.metrics_from_sums(acc), dtype=np.float64)})
+        print(f"[bench] outputs of the last timed step -> {a.dump_outputs}: {written}", file=sys.stderr)
 
     # ---- e2e: host LR + host HR in, host SR mosaic + (psnr, ssim) out, through SceneRunner.submit/result ----
     pending = []

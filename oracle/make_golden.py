@@ -128,7 +128,7 @@ def main():
     assert abs(p_ref - p_or) < 1e-6 and abs(s_ref - s_or) < 1e-7
     pipe["met_label"], pipe["met_out"] = lab, noisy
     pipe["met_psnr"], pipe["met_ssim"] = np.float64(p_ref), np.float64(s_ref)
-    np.savez_compressed(os.path.join(gold, "pipeline.npz"), **pipe)
+    weights.save_pipeline_golden(pipe)
 
     # ---- utils/imresize.py (SURVEY 8f-3): the reference function on seeded arrays ---------------------
     import utils.imresize as RI  # the reference's

@@ -23,6 +23,25 @@ GOLDEN_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file
 GAIN = {"MyEfficientLFNet": 0.7, "EPIT": 0.6, "DistgSSR": 0.6, "LF_InterNet": 0.55, "MyEfficientLFNetV4_5": 0.7}
 
 
+# the patch-pipeline goldens of make_golden.py, split by key prefix so that every file stays under 1 MB
+PIPELINE_GOLDENS = {"pipeline.npz": ("div_",),                   # LFdivide
+                    "pipeline_tail.npz": ("int_", "met_")}       # LFintegrate, cal_metrics
+
+
+def save_pipeline_golden(pipe: dict) -> None:
+    assert all(k.startswith(sum(PIPELINE_GOLDENS.values(), ())) for k in pipe), "a key without a file"
+    for fname, prefixes in PIPELINE_GOLDENS.items():
+        np.savez_compressed(os.path.join(GOLDEN_DIR, fname), **{k: v for k, v in pipe.items() if k.startswith(prefixes)})
+
+
+def load_pipeline_golden() -> dict:
+    out = {}
+    for fname in PIPELINE_GOLDENS:
+        with np.load(os.path.join(GOLDEN_DIR, fname)) as g:
+            out.update({k: g[k] for k in g.files})
+    return out
+
+
 def spec_path(model: str, scale: int) -> str:
     return os.path.join(GOLDEN_DIR, f"{model}_x{scale}.spec.json")
 

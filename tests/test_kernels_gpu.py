@@ -8,7 +8,7 @@ import lfsr_b200
 from lfsr_b200 import kernels as K
 from lfsr_b200 import _native as N
 from opref import RefOps
-from oracle import lf_oracle
+from oracle import lf_oracle, weights
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -72,8 +72,8 @@ def test_divide_integrate_edge_geometries(ops, A, h0, w0, P, S, s):
             lfsr_b200.lfutils.LFdivide(torch.zeros(5 * bad[0], 5 * bad[1], device=DEV), 5, bad[2], bad[3])
 
 
-def test_divide_integrate_goldens(ops, golden_dir):
-    g = np.load(f"{golden_dir}/pipeline.npz")
+def test_divide_integrate_goldens(ops):
+    g = weights.load_pipeline_golden()
     for (h0, w0) in ((32, 32), (47, 61), (64, 40)):
         scene = g[f"div_{h0}x{w0}_scene"]
         got = lfsr_b200.lfutils.LFdivide(torch.from_numpy(scene).to(DEV), 5, 32, 16).cpu().numpy()
@@ -456,8 +456,8 @@ def test_epit_basictrans_fused(ops, B, hv):
         assert err <= 1.5e-3 * scale, (pi, err, scale)          # 1e-3 + half an fp16 ulp of the output
 
 
-def test_metrics_vs_oracle_and_golden(ops, golden_dir):
-    g = np.load(f"{golden_dir}/pipeline.npz")
+def test_metrics_vs_oracle_and_golden(ops):
+    g = weights.load_pipeline_golden()
     lab, noisy = g["met_label"], g["met_out"]
 
     class MA:

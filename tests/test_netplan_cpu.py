@@ -76,7 +76,7 @@ def test_cpu_input_without_backend_raises():
         net(torch.zeros(1, 1, 40, 40))
 
 
-def test_oracle_imresize_matches_reference_golden():
+def test_oracle_imresize_matches_reference_golden(monkeypatch):
     """oracle.lf_oracle.imresize == outputs of the unmodified utils/imresize.py (oracle/make_golden.py, SURVEY 8f-3), and
     the product's host-side contribution tables equal the oracle's"""
     from oracle import lf_oracle
@@ -90,11 +90,12 @@ def test_oracle_imresize_matches_reference_golden():
         w0, i0 = lf_oracle.imresize_contributions(n_in, n_out, sc, m)
         w1, i1 = lfsr_b200.lfutils.resize_contributions(n_in, n_out, sc, m)
         assert np.array_equal(w0, w1) and np.array_equal(i0, i1)
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)        # host inputs go to the GPU when there is one
     with pytest.raises(lfsr_b200.LfsrError):
         lfsr_b200.lfutils.imresize(np.zeros((8, 8)), scalar_scale=2)        # no CPU fallback
 
 
-def test_oracle_colour_tail_and_bmp_writer(tmp_path):
+def test_oracle_colour_tail_and_bmp_writer(tmp_path, monkeypatch):
     """oracle colour tail == the reference's (committed golden); write_bmp == Pillow's bytes (host logic, no GPU)"""
     from oracle import lf_oracle
     g = np.load(f"{weights.GOLDEN_DIR}/colour_tail.npz")
@@ -102,5 +103,6 @@ def test_oracle_colour_tail_and_bmp_writer(tmp_path):
     p = tmp_path / "v.bmp"
     lfsr_b200.lfutils.write_bmp(str(p), g["views"][1, 3])
     assert np.array_equal(np.frombuffer(p.read_bytes(), dtype=np.uint8), g["bmp_view_1_3"])
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)        # host inputs go to the GPU when there is one
     with pytest.raises(lfsr_b200.LfsrError):
         lfsr_b200.lfutils.sai_to_rgb8_views(torch.zeros(10, 10), torch.zeros(2, 10, 10), 5)

@@ -14,8 +14,8 @@ SIZES = ((32, 32), (47, 61), (64, 40))
 
 @pytest.mark.parametrize("h0,w0", SIZES)
 def test_lfdivide_lfintegrate_equal_reference_outputs(h0, w0):
-    """utils/utils.py:152-178 through the reference itself -> pipeline.npz; bit-exact (pure indexing)"""
-    g = np.load(f"{GOLD}/pipeline.npz")
+    """utils/utils.py:152-178 through the reference itself -> pipeline.npz, pipeline_tail.npz; bit-exact (pure indexing)"""
+    g = weights.load_pipeline_golden()
     scene = g[f"div_{h0}x{w0}_scene"]
     sub = lf_oracle.lfdivide(scene, 5, 32, 16)
     assert sub.shape == tuple(g[f"div_{h0}x{w0}_shape"])
@@ -29,7 +29,7 @@ def test_lfdivide_lfintegrate_equal_reference_outputs(h0, w0):
 
 def test_cal_metrics_equal_reference_outputs():
     """utils/utils.py:91-134 (skimage restated on scipy): PSNR / SSIM of the reference run on the same pair"""
-    g = np.load(f"{GOLD}/pipeline.npz")
+    g = weights.load_pipeline_golden()
     p, s, pv, sv = lf_oracle.cal_metrics(g["met_label"][0, 0], g["met_out"][0, 0], 5)
     assert abs(p - float(g["met_psnr"])) < 1e-6 and abs(s - float(g["met_ssim"])) < 1e-7
     assert pv.shape == (5, 5) and sv.shape == (5, 5)
