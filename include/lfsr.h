@@ -122,6 +122,25 @@ int lfsr_divide_rows(const float* scene, float* patches, int ang, int h0, int w0
 int lfsr_integrate_rows(const float* patches, float* out, int ang, int pz, int stride, int h, int w,
                         int num_u, int num_v, int u_begin, int u_end, void* stream);
 
+/* ---- x8 geometric self-ensemble (no counterpart in the reference) ---------------------- */
+/* The 8 flips / transposes of one patch mosaic M [(a1 P), (a2 P)] of side L; on the SAI mosaic they reverse an angular
+ * axis together with its spatial axis, or swap (u, h) with (v, w), so the epipolar geometry is kept. For t in 0..7 with
+ * b0 = t & 1, b1 = (t >> 1) & 1, b2 = (t >> 2) & 1:
+ *     T_t(M):  m = M;  if b0: m = m[::-1, :];  if b1: m = m[:, ::-1];  if b2: m = m.T
+ * and T_t^-1 applies the same steps in reverse order. The ensemble of a patch with network F is, in fp32 without FMA
+ * contraction, Y = ((T_0^-1 F(T_0 X) + T_1^-1 F(T_1 X)) + ... + T_7^-1 F(T_7 X)) * 0.125.
+ *
+ * lfsr_divide_rows_d8: lfsr_divide_rows (same geometry checks and accept / reject rule) that writes the 8 variants of
+ * every patch of rows [u_begin, u_end): patches [(u_end - u_begin) * numV][8][A*P][A*P], patch-major, t = T_t(patch).
+ * Bit-exact (a pure gather). */
+int lfsr_divide_rows_d8(const float* scene, float* patches, int ang, int h0, int w0, int patch, int stride,
+                        int u_begin, int u_end, void* stream);
+/* lfsr_integrate_rows_d8: patches8 [(u_end - u_begin) * num_v][8][A*pz][A*pz] holds F(T_t X) of each patch (pointing at
+ * patch (u_begin, 0), variant 0); writes the LFintegrate of the per-patch ensembles Y into rows [u_begin, u_end) of the
+ * mosaic, with the row-shard semantics of lfsr_integrate_rows. Each mosaic pixel is written once (no atomics). */
+int lfsr_integrate_rows_d8(const float* patches8, float* out, int ang, int pz, int stride, int h, int w,
+                           int num_u, int num_v, int u_begin, int u_end, void* stream);
+
 /* ---- interpolation residual ---------------------------------------------------------- */
 /* F.interpolate(mode='bicubic'|'bilinear', align_corners=False) as called at
  * MyEfficientLFNet.py:88-90 (bicubic, whole mosaic), EPIT.py:164-169 (bicubic, per view),

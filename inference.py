@@ -36,7 +36,8 @@ def main(args):
             for Lr_SAI_y, _hr, cbcr, data_info, lf_name in loader:
                 ang = int(data_info[0][0].item())
                 sr = _scene.super_resolve_scene(net, Lr_SAI_y.squeeze().to(device), ang, args.scale_factor,
-                                                args.patch_size_for_test, args.stride_for_test, args.minibatch)
+                                                args.patch_size_for_test, args.stride_for_test, args.minibatch,
+                                                self_ensemble=bool(getattr(args, "self_ensemble", 0)))
                 _write_views(save_dir, lf_name[0], sr, cbcr, args.angRes_out)
                 print("scene %s -> %s" % (lf_name[0], save_dir))
 

@@ -88,6 +88,8 @@ SIGNATURES = {
     "lfsr_divide": (_I, [_P, _P, _I, _I, _I, _I, _I, _P]),
     "lfsr_divide_rows": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "lfsr_integrate_rows": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "lfsr_divide_rows_d8": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "lfsr_integrate_rows_d8": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
     "lfsr_interp": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "lfsr_ycbcr_to_rgb8": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
     "lfsr_resample_f64": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),

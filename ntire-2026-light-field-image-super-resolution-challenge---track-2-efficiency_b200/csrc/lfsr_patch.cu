@@ -78,6 +78,169 @@ integrate_kernel(const float* __restrict__ patches, float* __restrict__ out, int
   }
 }
 
+// ---- x8 geometric self-ensemble (include/lfsr.h: lfsr_divide_rows_d8 / lfsr_integrate_rows_d8) ----------------------
+// Variant t of an L x L patch mosaic M (b0 = t & 1, b1 = t & 2, b2 = t & 4): flip rows, flip columns, transpose, in that
+// order. So T_t(M)[y][x] = b2 ? M[f0(x)][f1(y)] : M[f0(y)][f1(x)] with f0 / f1 the row / column flip when b0 / b1 is set,
+// and T_t^-1(Z)[r][c] = b2 ? Z[f1(c)][f0(r)] : Z[f0(r)][f1(c)].
+
+// divide_kernel with the variant folded into the source index: blockIdx.y walks (patch, t) pairs in output order, so the
+// stores stay dense float4 runs; the scene reads of the transposing variants walk a column of the (L2-resident) LR scene
+__global__ void __launch_bounds__(256)
+divide_d8_kernel(const float* __restrict__ scene, float* __restrict__ patches, int A, int h0, int w0, int P, int S,
+                 int bdr, int numV, int u_begin, int nvar) {
+  const int L = A * P;
+  const int row4 = L >> 2;
+  const int per_patch4 = L * row4;
+  const int sw = A * w0;
+  for (int vidx = blockIdx.y; vidx < nvar; vidx += gridDim.y) {
+    const int pidx = vidx >> 3, t = vidx & 7;
+    const bool b0 = t & 1, b1 = t & 2, b2 = t & 4;
+    const int n2 = pidx % numV;
+    const int n1 = pidx / numV + u_begin;
+    // scene offset of patch-mosaic row r / column c (divide_kernel's index math, split by axis)
+    auto row_off = [&](int r) {
+      if (b0) r = L - 1 - r;
+      const int a1 = r / P, y = r - a1 * P;
+      return (a1 * h0 + mirror(n1 * S + y - bdr, h0)) * sw;
+    };
+    auto col_off = [&](int c) {
+      if (b1) c = L - 1 - c;
+      const int a2 = c / P, x = c - a2 * P;
+      return a2 * w0 + mirror(n2 * S + x - bdr, w0);
+    };
+    float4* dst = reinterpret_cast<float4*>(patches) + (size_t)vidx * per_patch4;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < per_patch4; i += gridDim.x * blockDim.x) {
+      const int py = i / row4;
+      const int px = (i - py * row4) << 2;
+      float4 v;
+      if (b2) {
+        const int c = col_off(py);
+        v.x = __ldg(scene + row_off(px) + c);
+        v.y = __ldg(scene + row_off(px + 1) + c);
+        v.z = __ldg(scene + row_off(px + 2) + c);
+        v.w = __ldg(scene + row_off(px + 3) + c);
+      } else {
+        const float* src = scene + row_off(py);
+        v.x = __ldg(src + col_off(px));
+        v.y = __ldg(src + col_off(px + 1));
+        v.z = __ldg(src + col_off(px + 2));
+        v.w = __ldg(src + col_off(px + 3));
+      }
+      dst[i] = v;
+    }
+  }
+}
+
+constexpr int D8_TILE = 32;
+
+// One CTA = a 32 x 32 tile of one view (a1, a2) of the stitched mosaic. Each output pixel (Y, X) of the view sits at row
+// r(Y), column c(X) of patch (Y / ss, X / ss); the kernel averages T_t^-1(F_t)[r][c] over t. The four non-transposing
+// variants are read row-wise straight from global memory (float4 when VEC == 4; reversed quads for b1). The four transposing
+// ones read Z_t[f1(c)][f0(r)], a column walk, so each is staged through a padded shared tile: lanes run along Y, which is
+// contiguous in Z_t's row, and the tile is read back along X. Sums run in t order with __fadd_rn, then __fmul_rn by 1/8.
+template <int VEC>
+__global__ void __launch_bounds__(256)
+integrate_d8_kernel(const float* __restrict__ patches8, float* __restrict__ out, int A, int pz, int ss, int h, int w,
+                    int numV, int u_begin, int y_begin, int y_count, int tiles_x, int tiles_y) {
+  __shared__ float tile[4][D8_TILE][D8_TILE + 1];      // [t - 4][Y][X]
+  const int L = A * pz;
+  const size_t LL = (size_t)L * L;
+  const int bdr = (pz - ss) / 2;
+  const int a2 = blockIdx.x / tiles_x, X0 = (blockIdx.x - a2 * tiles_x) * D8_TILE;
+  const int a1 = blockIdx.y / tiles_y, Y0 = y_begin + (blockIdx.y - a1 * tiles_y) * D8_TILE;
+  const int y_end = y_begin + y_count;
+  const int lane = threadIdx.x & 31, wy = threadIdx.x >> 5;
+  // patch (n1, n2) variant 0 and the in-patch row / column of view pixel (Y, X)
+  auto patch_base = [&](int Y, int X) {
+    return patches8 + ((size_t)(Y / ss - u_begin) * numV + X / ss) * 8 * LL;
+  };
+  auto prow = [&](int Y) { return a1 * pz + bdr + Y % ss; };
+  auto pcol = [&](int X) { return a2 * pz + bdr + X % ss; };
+
+  // stage the transposing variants: element (Y0 + lane, X0 + wy + 8k) of T_t^-1(Z_t) = Z_t[f1(c)][f0(r)]
+  {
+    const int Y = Y0 + lane;
+    const int r = prow(Y);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const int xl = wy + 8 * k, X = X0 + xl;
+      if (Y < y_end && X < w) {
+        const float* base = patch_base(Y, X);
+        const int c = pcol(X);
+#pragma unroll
+        for (int t = 4; t < 8; ++t) {
+          const int zr = (t & 2) ? L - 1 - c : c, zc = (t & 1) ? L - 1 - r : r;
+          tile[t - 4][lane][xl] = __ldg(base + t * LL + (size_t)zr * L + zc);
+        }
+      }
+    }
+  }
+  __syncthreads();
+
+  const size_t ow = (size_t)A * w;
+  if (VEC == 4) {
+    // thread = one float4 of X in one row: 8 threads per tile row, 32 rows
+    const int yl = threadIdx.x >> 3, xl = (threadIdx.x & 7) * 4;
+    const int Y = Y0 + yl, X = X0 + xl;
+    if (Y < y_end && X < w) {                                    // w % 4 == 0: the whole quad is inside
+      const float* base = patch_base(Y, X);
+      const int r = prow(Y), c = pcol(X);
+      float4 acc;
+#pragma unroll
+      for (int t = 0; t < 8; ++t) {
+        float4 v;
+        if (t < 4) {
+          const int zr = (t & 1) ? L - 1 - r : r;
+          if (t & 2) {                                           // columns L-1-c-3 .. L-1-c, read as one quad, reversed
+            const float4 q = __ldg(reinterpret_cast<const float4*>(base + t * LL + (size_t)zr * L + (L - 4 - c)));
+            v = make_float4(q.w, q.z, q.y, q.x);
+          } else {
+            v = __ldg(reinterpret_cast<const float4*>(base + t * LL + (size_t)zr * L + c));
+          }
+        } else {
+          const float* s = tile[t - 4][yl] + xl;
+          v = make_float4(s[0], s[1], s[2], s[3]);
+        }
+        if (t == 0) {
+          acc = v;
+        } else {
+          acc.x = __fadd_rn(acc.x, v.x);
+          acc.y = __fadd_rn(acc.y, v.y);
+          acc.z = __fadd_rn(acc.z, v.z);
+          acc.w = __fadd_rn(acc.w, v.w);
+        }
+      }
+      acc = make_float4(__fmul_rn(acc.x, 0.125f), __fmul_rn(acc.y, 0.125f), __fmul_rn(acc.z, 0.125f),
+                        __fmul_rn(acc.w, 0.125f));
+      *reinterpret_cast<float4*>(out + (size_t)(a1 * h + Y) * ow + (size_t)a2 * w + X) = acc;
+    }
+  } else {
+    // thread = one X (lane) in rows wy + 8k
+    const int X = X0 + lane;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const int yl = wy + 8 * k, Y = Y0 + yl;
+      if (Y < y_end && X < w) {
+        const float* base = patch_base(Y, X);
+        const int r = prow(Y), c = pcol(X);
+        float acc = 0.f;
+#pragma unroll
+        for (int t = 0; t < 8; ++t) {
+          float v;
+          if (t < 4) {
+            const int zr = (t & 1) ? L - 1 - r : r, zc = (t & 2) ? L - 1 - c : c;
+            v = __ldg(base + t * LL + (size_t)zr * L + zc);
+          } else {
+            v = tile[t - 4][yl][lane];
+          }
+          acc = t == 0 ? v : __fadd_rn(acc, v);
+        }
+        out[(size_t)(a1 * h + Y) * ow + (size_t)a2 * w + X] = __fmul_rn(acc, 0.125f);
+      }
+    }
+  }
+}
+
 
 }  // namespace lfsr
 
@@ -88,12 +251,13 @@ extern "C" int lfsr_abi_version(void) { return LFSR_ABI_VERSION; }
 extern "C" int lfsr_built_for_sm100a(void) { return 1; }
 extern "C" uint64_t lfsr_launch_count(void) { return g_launches.load(); }
 
-extern "C" int lfsr_divide_rows(const float* scene, float* patches, int ang, int h0, int w0, int patch,
-                                int stride, int u_begin, int u_end, void* stream) {
-  LFSR_REQUIRE(scene && patches, "lfsr_divide: null pointer");
+// geometry checks + accept / reject rule shared by lfsr_divide_rows and lfsr_divide_rows_d8; sets bdr / numV
+static int divide_check(const float* scene, const float* patches, int ang, int h0, int w0, int patch, int stride,
+                        int u_begin, int u_end, const char* what, int* bdr_out, int* numv_out) {
+  LFSR_REQUIRE(scene && patches, "%s: null pointer", what);
   LFSR_REQUIRE(ang > 0 && h0 > 0 && w0 > 0 && patch > 0 && stride > 0 && patch >= stride,
-               "lfsr_divide: bad geometry A=%d h0=%d w0=%d P=%d S=%d", ang, h0, w0, patch, stride);
-  LFSR_REQUIRE(patch % 4 == 0, "lfsr_divide: patch size %d must be a multiple of 4", patch);
+               "%s: bad geometry A=%d h0=%d w0=%d P=%d S=%d", what, ang, h0, w0, patch, stride);
+  LFSR_REQUIRE(patch % 4 == 0, "%s: patch size %d must be a multiple of 4", what, patch);
   const int bdr = (patch - stride) / 2;
   const int numU = (h0 + 2 * bdr - 1) / stride, numV = (w0 + 2 * bdr - 1) / stride;
   // The reference pads bdr above and bdr + stride - 1 below out of ONE mirrored copy of the view (ImageExtend,
@@ -107,10 +271,20 @@ extern "C" int lfsr_divide_rows(const float* scene, float* patches, int ang, int
     return n >= bdr && windows >= 1 && windows == want;
   };
   LFSR_REQUIRE(tiles(h0, numU) && tiles(w0, numV),
-               "lfsr_divide: %dx%d views cannot be tiled with patch %d / stride %d (the reference's LFdivide raises too)", h0,
+               "%s: %dx%d views cannot be tiled with patch %d / stride %d (the reference's LFdivide raises too)", what, h0,
                w0, patch, stride);
-  LFSR_REQUIRE(0 <= u_begin && u_begin <= u_end && u_end <= numU, "lfsr_divide: row shard [%d,%d) outside [0,%d)",
+  LFSR_REQUIRE(0 <= u_begin && u_begin <= u_end && u_end <= numU, "%s: row shard [%d,%d) outside [0,%d)", what,
                u_begin, u_end, numU);
+  *bdr_out = bdr;
+  *numv_out = numV;
+  return LFSR_OK;
+}
+
+extern "C" int lfsr_divide_rows(const float* scene, float* patches, int ang, int h0, int w0, int patch,
+                                int stride, int u_begin, int u_end, void* stream) {
+  int bdr = 0, numV = 0;
+  const int st = divide_check(scene, patches, ang, h0, w0, patch, stride, u_begin, u_end, "lfsr_divide", &bdr, &numV);
+  if (st != LFSR_OK) return st;
   if (u_begin == u_end) return LFSR_OK;
   const int npatch = (u_end - u_begin) * numV;
   const int per_patch4 = (ang * patch) * (ang * patch / 4);
@@ -118,6 +292,21 @@ extern "C" int lfsr_divide_rows(const float* scene, float* patches, int ang, int
   divide_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(scene, patches, ang, h0, w0, patch, stride, bdr, numV, u_begin,
                                                         npatch);
   return check_launch("divide_kernel");
+}
+
+extern "C" int lfsr_divide_rows_d8(const float* scene, float* patches, int ang, int h0, int w0, int patch,
+                                   int stride, int u_begin, int u_end, void* stream) {
+  int bdr = 0, numV = 0;
+  const int st = divide_check(scene, patches, ang, h0, w0, patch, stride, u_begin, u_end, "lfsr_divide_rows_d8", &bdr,
+                              &numV);
+  if (st != LFSR_OK) return st;
+  if (u_begin == u_end) return LFSR_OK;
+  const int nvar = (u_end - u_begin) * numV * 8;
+  const int per_patch4 = (ang * patch) * (ang * patch / 4);
+  dim3 grid(ceil_div(per_patch4, 256 * 4), nvar < 32768 ? nvar : 32768);
+  divide_d8_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(scene, patches, ang, h0, w0, patch, stride, bdr, numV, u_begin,
+                                                           nvar);
+  return check_launch("divide_d8_kernel");
 }
 
 extern "C" int lfsr_divide(const float* scene, float* patches, int ang, int h0, int w0, int patch, int stride,
@@ -128,21 +317,34 @@ extern "C" int lfsr_divide(const float* scene, float* patches, int ang, int h0, 
   return lfsr_divide_rows(scene, patches, ang, h0, w0, patch, stride, 0, numU, stream);
 }
 
+// geometry checks shared by lfsr_integrate_rows and lfsr_integrate_rows_d8: the output rows [y_begin, y_begin + y_count)
+// of every view that the shard covers (y_count == 0: nothing to do) and whether the float4 path applies
+static int integrate_check(const float* patches, const float* out, int ang, int pz, int stride, int h, int w, int num_u,
+                           int num_v, int u_begin, int u_end, const char* what, int* y_begin_out, int* y_count_out,
+                           bool* vec_out) {
+  LFSR_REQUIRE(patches && out, "%s: null pointer", what);
+  LFSR_REQUIRE(ang > 0 && pz >= stride && stride > 0 && h > 0 && w > 0, "%s: bad geometry", what);
+  LFSR_REQUIRE(h <= num_u * stride && w <= num_v * stride,
+               "%s: output %dx%d larger than the stitched grid %dx%d", what, h, w, num_u * stride, num_v * stride);
+  LFSR_REQUIRE(0 <= u_begin && u_begin <= u_end && u_end <= num_u, "%s: bad row shard", what);
+  const int y_begin = u_begin * stride;
+  const int y_end = u_end * stride < h ? u_end * stride : h;
+  const int bdr = (pz - stride) / 2;
+  *y_begin_out = y_begin;
+  *y_count_out = y_end > y_begin ? y_end - y_begin : 0;
+  *vec_out = (w % 4 == 0) && (stride % 4 == 0) && (pz % 4 == 0) && (bdr % 4 == 0) &&
+             ((uintptr_t)patches % 16 == 0) && ((uintptr_t)out % 16 == 0);
+  return LFSR_OK;
+}
+
 extern "C" int lfsr_integrate_rows(const float* patches, float* out, int ang, int pz, int stride, int h, int w,
                                    int num_u, int num_v, int u_begin, int u_end, void* stream) {
-  LFSR_REQUIRE(patches && out, "lfsr_integrate: null pointer");
-  LFSR_REQUIRE(ang > 0 && pz >= stride && stride > 0 && h > 0 && w > 0, "lfsr_integrate: bad geometry");
-  LFSR_REQUIRE(h <= num_u * stride && w <= num_v * stride,
-               "lfsr_integrate: output %dx%d larger than the stitched grid %dx%d", h, w, num_u * stride,
-               num_v * stride);
-  LFSR_REQUIRE(0 <= u_begin && u_begin <= u_end && u_end <= num_u, "lfsr_integrate: bad row shard");
-  int y_begin = u_begin * stride;
-  int y_end = u_end * stride < h ? u_end * stride : h;
-  if (y_end <= y_begin) return LFSR_OK;
-  const int y_count = y_end - y_begin;
-  const int bdr = (pz - stride) / 2;
-  const bool vec = (w % 4 == 0) && (stride % 4 == 0) && (pz % 4 == 0) && (bdr % 4 == 0) &&
-                   ((uintptr_t)patches % 16 == 0) && ((uintptr_t)out % 16 == 0);
+  int y_begin = 0, y_count = 0;
+  bool vec = false;
+  const int st = integrate_check(patches, out, ang, pz, stride, h, w, num_u, num_v, u_begin, u_end, "lfsr_integrate",
+                                 &y_begin, &y_count, &vec);
+  if (st != LFSR_OK) return st;
+  if (y_count == 0) return LFSR_OK;
   const int rows = ang * y_count;
   if (vec) {
     dim3 grid(ceil_div(ang * (w / 4), 256), rows < 32768 ? rows : 32768);
@@ -154,6 +356,26 @@ extern "C" int lfsr_integrate_rows(const float* patches, float* out, int ang, in
                                                                 y_begin, y_count);
   }
   return check_launch("integrate_kernel");
+}
+
+extern "C" int lfsr_integrate_rows_d8(const float* patches8, float* out, int ang, int pz, int stride, int h, int w,
+                                      int num_u, int num_v, int u_begin, int u_end, void* stream) {
+  int y_begin = 0, y_count = 0;
+  bool vec = false;
+  const int st = integrate_check(patches8, out, ang, pz, stride, h, w, num_u, num_v, u_begin, u_end,
+                                 "lfsr_integrate_rows_d8", &y_begin, &y_count, &vec);
+  if (st != LFSR_OK) return st;
+  if (y_count == 0) return LFSR_OK;
+  const int tiles_x = ceil_div(w, D8_TILE), tiles_y = ceil_div(y_count, D8_TILE);
+  LFSR_REQUIRE((long long)ang * tiles_y <= 65535, "lfsr_integrate_rows_d8: %d view rows per shard is too many", y_count);
+  dim3 grid(ang * tiles_x, ang * tiles_y);
+  if (vec)
+    integrate_d8_kernel<4><<<grid, 256, 0, (cudaStream_t)stream>>>(patches8, out, ang, pz, stride, h, w, num_v, u_begin,
+                                                                   y_begin, y_count, tiles_x, tiles_y);
+  else
+    integrate_d8_kernel<1><<<grid, 256, 0, (cudaStream_t)stream>>>(patches8, out, ang, pz, stride, h, w, num_v, u_begin,
+                                                                   y_begin, y_count, tiles_x, tiles_y);
+  return check_launch("integrate_d8_kernel");
 }
 
 

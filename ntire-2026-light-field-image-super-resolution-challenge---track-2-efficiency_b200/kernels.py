@@ -161,6 +161,16 @@ class CudaOps:
         N.check(self.lib.lfsr_integrate_rows(patches.data_ptr(), out.data_ptr(), ang, pz, stride, h, w, num_u, num_v,
                                              u0, u1, self._stream(out)), "lfsr_integrate_rows")
 
+    def divide_rows_d8(self, scene, patches, ang, h0, w0, patch, stride, u0, u1):
+        """the 8 self-ensemble variants of every patch of rows [u0, u1): patches [n][8][A*P][A*P] (include/lfsr.h)"""
+        N.check(self.lib.lfsr_divide_rows_d8(scene.data_ptr(), patches.data_ptr(), ang, h0, w0, patch, stride, u0, u1,
+                                             self._stream(scene)), "lfsr_divide_rows_d8")
+
+    def integrate_rows_d8(self, patches8, out, ang, pz, stride, h, w, num_u, num_v, u0, u1):
+        """LFintegrate of the per-patch means of the 8 un-transformed SR variants in patches8 [n][8][A*pz][A*pz]"""
+        N.check(self.lib.lfsr_integrate_rows_d8(patches8.data_ptr(), out.data_ptr(), ang, pz, stride, h, w, num_u, num_v,
+                                                u0, u1, self._stream(out)), "lfsr_integrate_rows_d8")
+
     def interp(self, x, out, n, h, w, scale, mode, block_h, block_w):
         N.check(self.lib.lfsr_interp(x.data_ptr(), out.data_ptr(), n, h, w, scale, mode, block_h, block_w,
                                      self._stream(x)), "lfsr_interp")

@@ -47,11 +47,14 @@ class SceneRunner:
     world/rank row sharding of the patch grid (defaults: torch.distributed state); `group` is the process group of the
                all-gather
     depth      scenes in flight through submit()/result()
+    self_ensemble  x8 geometric self-ensemble per patch (include/lfsr.h, lfsr_divide_rows_d8): the network runs on the 8
+               flips / transposes of every patch mosaic, the un-transformed outputs are averaged before LFintegrate. Each
+               forward covers the 8 variants of whole patch-grid rows; `minibatch` still counts network patches
     """
 
     def __init__(self, net, ang: int, scale: int, h0: int, w0: int, patch: int = 32, stride: int = 16, minibatch: int = 64,
                  device=None, ops=None, world: Optional[int] = None, rank: Optional[int] = None, group=None,
-                 depth: int = 2, with_metrics: bool = True):
+                 depth: int = 2, with_metrics: bool = True, self_ensemble: bool = False):
         self.net, self.ang, self.scale, self.h0, self.w0 = net, int(ang), int(scale), int(h0), int(w0)
         self.patch, self.stride = int(patch), int(stride)
         self.ops = ops or getattr(net, "_ops", None) or K.default_ops()
@@ -76,13 +79,16 @@ class SceneRunner:
         self.hs_cov, self.ws_cov = min(self.hs, self.num_u * self.ss), min(self.ws, self.num_v * self.ss)
         if (self.hs_cov, self.ws_cov) != (self.hs, self.ws):
             raise ValueError("SceneRunner: the patch grid does not cover the scene (non-overlapping patches)")
-        n_own = (self.u1 - self.u0) * self.num_v
-        self.rows_per_mb = max(1, int(minibatch) // self.num_v) if self.num_v <= int(minibatch) else 0
+        self.self_ensemble = bool(self_ensemble)
+        self.nvar = 8 if self.self_ensemble else 1            # network patches per source patch
+        row = self.nvar * self.num_v                          # network patches per patch-grid row
+        n_own = (self.u1 - self.u0) * row
+        self.rows_per_mb = max(1, int(minibatch) // row) if row <= int(minibatch) else 0
         self.minibatch = int(minibatch)
         f32 = dict(dtype=torch.float32, device=self.dev)
         self.sub = torch.empty((max(n_own, 1), 1, ang * patch, ang * patch), **f32)
         # a patch-grid row wider than the minibatch is super-resolved in pieces into this row buffer
-        self.row_sr = torch.empty((self.num_v, 1, ang * self.pz, ang * self.pz), **f32) if self.rows_per_mb == 0 else None
+        self.row_sr = torch.empty((row, 1, ang * self.pz, ang * self.pz), **f32) if self.rows_per_mb == 0 else None
         self.depth = max(1, int(depth))
         self.with_metrics = with_metrics
         self.slots = []
@@ -123,21 +129,25 @@ class SceneRunner:
         """the hot path on tensors already in HBM; everything is enqueued on the current stream, nothing syncs."""
         ops, A = self.ops, self.ang
         u0, u1 = self.u0, self.u1
+        if self.self_ensemble:
+            divide, integrate = ops.divide_rows_d8, ops.integrate_rows_d8
+        else:
+            divide, integrate = ops.divide_rows, ops.integrate_rows
+        row = self.nvar * self.num_v
         if u1 > u0:
-            ops.divide_rows(lr_dev, self.sub, A, self.h0, self.w0, self.patch, self.stride, u0, u1)
+            divide(lr_dev, self.sub, A, self.h0, self.w0, self.patch, self.stride, u0, u1)
             if self.rows_per_mb:
                 for r in range(u0, u1, self.rows_per_mb):
                     r1 = min(r + self.rows_per_mb, u1)
-                    x = self.sub[(r - u0) * self.num_v:(r1 - u0) * self.num_v]
+                    x = self.sub[(r - u0) * row:(r1 - u0) * row]
                     y = self._forward(x)
-                    ops.integrate_rows(y, mosaic, A, self.pz, self.ss, self.hs, self.ws, self.num_u, self.num_v, r, r1)
+                    integrate(y, mosaic, A, self.pz, self.ss, self.hs, self.ws, self.num_u, self.num_v, r, r1)
             else:
                 for r in range(u0, u1):
-                    for c in range(0, self.num_v, self.minibatch):
-                        c1 = min(c + self.minibatch, self.num_v)
-                        self.row_sr[c:c1] = self.net(self.sub[(r - u0) * self.num_v + c:(r - u0) * self.num_v + c1], [A, A])
-                    ops.integrate_rows(self.row_sr, mosaic, A, self.pz, self.ss, self.hs, self.ws, self.num_u, self.num_v,
-                                       r, r + 1)
+                    for c in range(0, row, self.minibatch):
+                        c1 = min(c + self.minibatch, row)
+                        self.row_sr[c:c1] = self.net(self.sub[(r - u0) * row + c:(r - u0) * row + c1], [A, A])
+                    integrate(self.row_sr, mosaic, A, self.pz, self.ss, self.hs, self.ws, self.num_u, self.num_v, r, r + 1)
         if gather and self.world > 1:
             self.gather_stripes(mosaic)
         if hr_dev is not None and acc is not None:
@@ -265,36 +275,38 @@ class _NullCtx:
 
 
 def runner_for(net, ang, scale, h0, w0, patch=32, stride=16, minibatch=64, device=None, ops=None, group=None,
-               world=None, rank=None) -> SceneRunner:
+               world=None, rank=None, self_ensemble=False) -> SceneRunner:
     """the SceneRunner of this geometry, cached on the network (dropped with the network)."""
     w_, r_ = _dist_state(group)
     world = w_ if world is None else world
     rank = r_ if rank is None else rank
     cache = net.__dict__.setdefault("_scene_runners", {})
-    key = (ang, scale, h0, w0, patch, stride, minibatch, str(device), id(ops), world, rank, id(group))
+    key = (ang, scale, h0, w0, patch, stride, minibatch, str(device), id(ops), world, rank, id(group), bool(self_ensemble))
     r = cache.get(key)
     if r is None:
         if len(cache) >= 4:                    # scenes of a dataset come in a few sizes; do not hoard HBM
             cache.pop(next(iter(cache)))
-        r = cache[key] = SceneRunner(net, ang, scale, h0, w0, patch, stride, minibatch, device, ops, world, rank, group)
+        r = cache[key] = SceneRunner(net, ang, scale, h0, w0, patch, stride, minibatch, device, ops, world, rank, group,
+                                     self_ensemble=bool(self_ensemble))
     return r
 
 
 def super_resolve_rows(net, lr_sai: torch.Tensor, ang: int, scale: int, patch: int = 32, stride: int = 16,
-                       minibatch: int = 64, rows=None, out_mosaic: torch.Tensor = None, ops=None) -> torch.Tensor:
+                       minibatch: int = 64, rows=None, out_mosaic: torch.Tensor = None, ops=None,
+                       self_ensemble: bool = False) -> torch.Tensor:
     """SR of the patch-grid rows `rows` of one scene; returns the full-size SAI mosaic
-    [(a1 h s), (a2 w s)] with only the owned stripes written."""
+    [(a1 h s), (a2 w s)] with only the owned stripes written. self_ensemble: see SceneRunner."""
     H, W = lr_sai.shape
     h0, w0 = H // ang, W // ang
     dev = lr_sai.device
     _, num_u, _ = U.divide_geometry(h0, w0, patch, stride)
-    r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops, world=1, rank=0)
+    r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops, world=1, rank=0, self_ensemble=self_ensemble)
     if out_mosaic is None:
         out_mosaic = torch.zeros((ang * h0 * scale, ang * w0 * scale), dtype=torch.float32, device=dev)
     saved = (r.u0, r.u1)
     r.u0, r.u1 = (0, num_u) if rows is None else rows
-    if (r.u1 - r.u0) * r.num_v > r.sub.shape[0]:
-        r.sub = torch.empty(((r.u1 - r.u0) * r.num_v,) + tuple(r.sub.shape[1:]), dtype=torch.float32, device=dev)
+    if (r.u1 - r.u0) * r.nvar * r.num_v > r.sub.shape[0]:
+        r.sub = torch.empty(((r.u1 - r.u0) * r.nvar * r.num_v,) + tuple(r.sub.shape[1:]), dtype=torch.float32, device=dev)
     try:
         r.run_resident(lr_sai.to(torch.float32).contiguous(), out_mosaic, gather=False)
     finally:
@@ -303,14 +315,14 @@ def super_resolve_rows(net, lr_sai: torch.Tensor, ang: int, scale: int, patch: i
 
 
 def super_resolve_scene(net, lr_sai: torch.Tensor, ang: int, scale: int, patch: int = 32, stride: int = 16,
-                        minibatch: int = 64, group=None, ops=None) -> torch.Tensor:
+                        minibatch: int = 64, group=None, ops=None, self_ensemble: bool = False) -> torch.Tensor:
     """Full scene; when a process group is given (or torch.distributed is initialised with
     world_size > 1) each rank computes its row band and the bands are all-gathered. Returns a device mosaic owned by the
-    caller."""
+    caller. self_ensemble: see SceneRunner."""
     H, W = lr_sai.shape
     h0, w0 = H // ang, W // ang
     dev = lr_sai.device
-    r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops, group)
+    r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops, group, self_ensemble=self_ensemble)
     mosaic = torch.empty((r.H, r.W), dtype=torch.float32, device=dev)
     ctx = torch.cuda.device(dev) if dev.type == "cuda" else _NullCtx()
     with ctx:
@@ -334,9 +346,10 @@ def gather_stripes(mosaic: torch.Tensor, ang: int, h: int, w: int, ss: int, num_
 
 
 def test_scene(net, lr_sai, hr_sai, ang: int, scale: int, patch: int = 32, stride: int = 16, minibatch: int = 64,
-               ops=None):
+               ops=None, self_ensemble: bool = False):
     """(psnr, ssim, sr_mosaic) for one scene - the body of train.test()'s loop on the device. lr/hr may be host or device
-    tensors; sr_mosaic is a device tensor that stays valid until the next scene of the same geometry is submitted twice."""
+    tensors; sr_mosaic is a device tensor that stays valid until the next scene of the same geometry is submitted twice.
+    self_ensemble: see SceneRunner."""
     lr_sai = lr_sai.reshape(lr_sai.shape[-2:])
     hr_sai = hr_sai.reshape(hr_sai.shape[-2:])
     H, W = lr_sai.shape
@@ -347,6 +360,6 @@ def test_scene(net, lr_sai, hr_sai, ang: int, scale: int, patch: int = 32, strid
         dev = lr_sai.device
     if lr_sai.is_cuda:
         dev = lr_sai.device
-    r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops)
+    r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops, self_ensemble=self_ensemble)
     psnr, ssim, sr = r.result(r.submit(lr_sai, hr_sai, readback=False))
     return psnr, ssim, sr

@@ -2,7 +2,7 @@
 reference's option.py:4-34 (including its `type=bool` quirk: any non-empty string is True, so the
 random-init path needs --use_pre_ckpt ''), parsed at import time like the reference because
 utils/utils.py and the entry points do `from option import args`.
-Additive flags (not in the reference): --synthetic, --minibatch."""
+Additive flags (not in the reference): --synthetic, --synthetic_size, --minibatch, --self_ensemble."""
 import argparse
 
 _FLAGS = [
@@ -32,6 +32,7 @@ _FLAGS = [
     ("--synthetic", dict(type=int, default=0, help="run on N seeded synthetic scenes instead of h5 files")),
     ("--synthetic_size", dict(type=int, default=64, help="view height/width of the synthetic LR scenes")),
     ("--minibatch", dict(type=int, default=64, help="patches per forward on the device path")),
+    ("--self_ensemble", dict(type=int, default=0, help="1: x8 flip/transpose self-ensemble per patch (8x the forwards)")),
 ]
 
 parser = argparse.ArgumentParser()

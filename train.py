@@ -32,7 +32,8 @@ def test(test_loader, device, net, args, save_dir=None):
         lr, hr = Lr_SAI_y.squeeze(), Hr_SAI_y.squeeze()
         with torch.no_grad():
             psnr, ssim, sr = _scene.test_scene(net, lr, hr, ang, args.scale_factor, args.patch_size_for_test,
-                                               args.stride_for_test, getattr(args, "minibatch", 64))
+                                               args.stride_for_test, getattr(args, "minibatch", 64),
+                                               self_ensemble=bool(getattr(args, "self_ensemble", 0)))
         psnrs.append(psnr)
         ssims.append(ssim)
         names.append(LF_name[0])
