@@ -30,6 +30,17 @@ def shard_rows(num_u: int, world: int, rank: int):
     return lo, lo + base + (1 if rank < extra else 0)
 
 
+def assign_scenes(n: int, world: int, rank: int):
+    """(own, tail) of a dataset of n scenes on `world` ranks. `own`: the scenes rank runs alone as single-GPU runs, i in
+    [0, world * (n // world)) with i % world == rank (full rounds, no communication). `tail`: the remaining n % world
+    scenes, each row-sharded over all ranks; rank i % world keeps its result. Both lists ascend and every tail index is
+    above every full-round index, so own + tail is the rank's run order and follows dataset order."""
+    if n < 0 or world < 1 or not 0 <= rank < world:
+        raise ValueError(f"assign_scenes: n={n}, world={world}, rank={rank}")
+    full = world * (n // world)
+    return list(range(rank, full, world)), list(range(full, n))
+
+
 def _dist_state(group=None):
     import torch.distributed as dist
     if dist.is_available() and dist.is_initialized():
@@ -315,14 +326,17 @@ def super_resolve_rows(net, lr_sai: torch.Tensor, ang: int, scale: int, patch: i
 
 
 def super_resolve_scene(net, lr_sai: torch.Tensor, ang: int, scale: int, patch: int = 32, stride: int = 16,
-                        minibatch: int = 64, group=None, ops=None, self_ensemble: bool = False) -> torch.Tensor:
+                        minibatch: int = 64, group=None, ops=None, self_ensemble: bool = False, world: Optional[int] = None,
+                        rank: Optional[int] = None) -> torch.Tensor:
     """Full scene; when a process group is given (or torch.distributed is initialised with
     world_size > 1) each rank computes its row band and the bands are all-gathered. Returns a device mosaic owned by the
-    caller. self_ensemble: see SceneRunner."""
+    caller. world/rank override the group's (world=1, rank=0: the whole scene on this rank, no exchange).
+    self_ensemble: see SceneRunner."""
     H, W = lr_sai.shape
     h0, w0 = H // ang, W // ang
     dev = lr_sai.device
-    r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops, group, self_ensemble=self_ensemble)
+    r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops, group, world, rank,
+                   self_ensemble=self_ensemble)
     mosaic = torch.empty((r.H, r.W), dtype=torch.float32, device=dev)
     ctx = torch.cuda.device(dev) if dev.type == "cuda" else _NullCtx()
     with ctx:
@@ -346,10 +360,10 @@ def gather_stripes(mosaic: torch.Tensor, ang: int, h: int, w: int, ss: int, num_
 
 
 def test_scene(net, lr_sai, hr_sai, ang: int, scale: int, patch: int = 32, stride: int = 16, minibatch: int = 64,
-               ops=None, self_ensemble: bool = False):
+               ops=None, self_ensemble: bool = False, world: Optional[int] = None, rank: Optional[int] = None):
     """(psnr, ssim, sr_mosaic) for one scene - the body of train.test()'s loop on the device. lr/hr may be host or device
     tensors; sr_mosaic is a device tensor that stays valid until the next scene of the same geometry is submitted twice.
-    self_ensemble: see SceneRunner."""
+    world/rank: see super_resolve_scene. self_ensemble: see SceneRunner."""
     lr_sai = lr_sai.reshape(lr_sai.shape[-2:])
     hr_sai = hr_sai.reshape(hr_sai.shape[-2:])
     H, W = lr_sai.shape
@@ -360,6 +374,7 @@ def test_scene(net, lr_sai, hr_sai, ang: int, scale: int, patch: int = 32, strid
         dev = lr_sai.device
     if lr_sai.is_cuda:
         dev = lr_sai.device
-    r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops, self_ensemble=self_ensemble)
+    r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops, world=world, rank=rank,
+                   self_ensemble=self_ensemble)
     psnr, ssim, sr = r.result(r.submit(lr_sai, hr_sai, readback=False))
     return psnr, ssim, sr

@@ -20,14 +20,19 @@ class SyntheticTestSet:
     def __len__(self):
         return self.n
 
-    def __iter__(self):
+    def __getitem__(self, i):
+        if not 0 <= i < self.n:
+            raise IndexError(i)
         A, s, h = self.args.angRes_in, self.args.scale_factor, self.size
+        rs = np.random.RandomState(1000 + i)
+        lr = torch.from_numpy(rs.random_sample((1, A * h, A * h)).astype(np.float32))
+        hr = torch.from_numpy(rs.random_sample((1, A * h * s, A * h * s)).astype(np.float32))
+        cbcr = torch.full((2, A * h * s, A * h * s), 0.5)
+        return _batch1(lr, hr, cbcr, A, self.args.angRes_out, "synthetic_%02d" % i)
+
+    def __iter__(self):
         for i in range(self.n):
-            rs = np.random.RandomState(1000 + i)
-            lr = torch.from_numpy(rs.random_sample((1, A * h, A * h)).astype(np.float32))
-            hr = torch.from_numpy(rs.random_sample((1, A * h * s, A * h * s)).astype(np.float32))
-            cbcr = torch.full((2, A * h * s, A * h * s), 0.5)
-            yield _batch1(lr, hr, cbcr, A, self.args.angRes_out, "synthetic_%02d" % i)
+            yield self[i]
 
 
 class H5TestSet:
@@ -46,22 +51,27 @@ class H5TestSet:
     def __len__(self):
         return len(self.files)
 
-    def __iter__(self):
+    def __getitem__(self, i):
+        """reads only the i-th file (a rank of a multi-GPU run opens just the scenes it runs)"""
         import h5py
-        for fn in self.files:
-            with h5py.File(os.path.join(self.root, fn), "r") as hf:
-                lr = np.array(hf.get("Lr_SAI_y")).T
-                hr = np.array(hf.get("Hr_SAI_y")).T
-                cb = np.array(hf.get("Sr_SAI_cbcr"), dtype="single")
-            if cb.ndim == 3:
-                cb = np.transpose(cb, (2, 1, 0))
-            elif cb.ndim == 0 or cb.size == 0:
-                cb = np.zeros((hr.shape[0], hr.shape[1], 2), np.float32)
-            elif cb.ndim == 2:
-                cb = cb[..., None]
-            to_t = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32))
-            yield _batch1(to_t(lr)[None], to_t(hr)[None], to_t(cb).permute(2, 0, 1).contiguous(), self.args.angRes_in,
-                          self.args.angRes_out, fn.split(".")[0])
+        fn = self.files[i]
+        with h5py.File(os.path.join(self.root, fn), "r") as hf:
+            lr = np.array(hf.get("Lr_SAI_y")).T
+            hr = np.array(hf.get("Hr_SAI_y")).T
+            cb = np.array(hf.get("Sr_SAI_cbcr"), dtype="single")
+        if cb.ndim == 3:
+            cb = np.transpose(cb, (2, 1, 0))
+        elif cb.ndim == 0 or cb.size == 0:
+            cb = np.zeros((hr.shape[0], hr.shape[1], 2), np.float32)
+        elif cb.ndim == 2:
+            cb = cb[..., None]
+        to_t = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32))
+        return _batch1(to_t(lr)[None], to_t(hr)[None], to_t(cb).permute(2, 0, 1).contiguous(), self.args.angRes_in,
+                       self.args.angRes_out, fn.split(".")[0])
+
+    def __iter__(self):
+        for i in range(len(self.files)):
+            yield self[i]
 
 
 def MultiTestSetDataLoader(args):
