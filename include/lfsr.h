@@ -156,6 +156,26 @@ int lfsr_interp(const float* in, float* out, int n, int h, int w, int scale, int
 int lfsr_ycbcr_to_rgb8(const float* y, const float* cb, const float* cr, unsigned char* rgb, int ang, int h, int w,
                        const double* mat_inv255, const double* offset, void* stream);
 
+/* ---- View preparation (input side; BasicLFSR's Generate_Data_for_Test.py / _for_inference.py as recorded in DESIGN.md
+ * row f-7: the generator scripts are not in this tree, so parity with them is unpinned). Per scene of U x V RGB views
+ * (U, V >= A = angRes), with s = scale_factor:
+ *   views   the central A x A: u0 = (U - A) // 2, v0 = (V - A) // 2;
+ *   crop    every view top-left to H' = H - H mod s, W' = W - W mod s; x = uint8 / 255.0 in fp64, in [0, 1];
+ *   colour  rgb2ycbcr term by term, each operation rounded, no FMA (a term's sign is folded into its constant):
+ *             Y  = ((((65.481 R + 128.553 G) + 24.966 B) +  16) / 255
+ *             Cb = ((((-37.797 R + -74.203 G) + 112.0 B) + 128) / 255
+ *             Cr = ((((112.0 R + -93.786 G) + -18.214 B) + 128) / 255
+ *   ground-truth views (test.py): Hr_SAI_y = Y(x); lr_rgb = imresize(x, 1/s) per view (fp64 float path);
+ *             Lr_SAI_y = Y(lr_rgb); Sr_SAI_cbcr = CbCr(imresize(lr_rgb, s));
+ *   LR views (inference.py): Lr_SAI_y = Y(x); Sr_SAI_cbcr = CbCr(imresize(x, s)); no HR.
+ * Outputs are SAI mosaics [(u h), (v w)] cast to fp32 round-to-nearest, Sr_SAI_cbcr as [2][(u h)][(v w)].
+ *
+ * lfsr_rgb_to_ycbcr_mosaic: views [ang][ang][h][w][3], uint8 (is_u8 = 1; divided by 255.0 in the kernel) or fp64 in
+ * [0, 1] (is_u8 = 0) -> the colour step above into fp32 mosaics [(ang h)][(ang w)]. y, or cb and cr together, may be NULL
+ * to skip that output; at least one is written. Bit-exact to the numpy statement. */
+int lfsr_rgb_to_ycbcr_mosaic(const void* views, int is_u8, float* y, float* cb, float* cr, int ang, int h, int w,
+                             void* stream);
+
 /* One separable pass of the reference's MATLAB-style imresize (utils/imresize.py:57-102 `resizeAlongDim`), fp64:
  * out[a][i][b] = sum_p weights[i][p] * in[a][indices[i][p]][b] over a tensor viewed as [outer][in_len][inner]
  * -> [outer][out_len][inner]; weights / border-reflected indices per output sample as imresize.py:32-55 builds them. */

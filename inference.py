@@ -29,7 +29,7 @@ def run(args, device, rank):
     _, _, result_dir = create_dir(args)
     result_dir = result_dir.joinpath("TEST")
     result_dir.mkdir(exist_ok=True)
-    test_names, test_loaders, n_scenes = MultiTestSetDataLoader(args)
+    test_names, test_loaders, n_scenes = MultiTestSetDataLoader(args, views="lr")
     log("The number of test data is: %d" % n_scenes)
     MODEL = importlib.import_module("model." + args.task + "." + args.model_name)
     net = MODEL.get_model(args)

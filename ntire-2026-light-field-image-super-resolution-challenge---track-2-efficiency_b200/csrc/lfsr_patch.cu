@@ -419,3 +419,59 @@ extern "C" int lfsr_ycbcr_to_rgb8(const float* y, const float* cb, const float* 
   lfsr::ycbcr_rgb8_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(y, cb, cr, rgb, ang, h, w, cm);
   return lfsr::check_launch("ycbcr_rgb8_kernel");
 }
+
+
+// ---- input side of the light-field preparation (include/lfsr.h, "View preparation"): RGB views -> Y / CbCr mosaics -------
+// BasicLFSR's rgb2ycbcr term by term: Y = (((65.481 R + 128.553 G) + 24.966 B) + 16) / 255 and likewise Cb, Cr with the
+// signs folded into the constants (exact), every multiply / add / divide rounded on its own (no FMA contraction), cast
+// to fp32 round-to-nearest. uint8 views are divided by 255 here in fp64 first. One thread per mosaic pixel in mosaic
+// order, so the fp32 stores coalesce; the a1 a2 h w -> (a1 h)(a2 w) rearrange is folded into the load address.
+namespace lfsr {
+__device__ __forceinline__ double view_value(const unsigned char* p) { return __ddiv_rn((double)*p, 255.0); }
+__device__ __forceinline__ double view_value(const double* p) { return *p; }
+
+__device__ __forceinline__ float ycbcr_term(double r, double g, double b, double kr, double kg, double kb, double off) {
+  const double s = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(kr, r), __dmul_rn(kg, g)), __dmul_rn(kb, b)), off);
+  return __double2float_rn(__ddiv_rn(s, 255.0));
+}
+
+template <class T>
+__global__ void __launch_bounds__(256)
+rgb_ycbcr_mosaic_kernel(const T* __restrict__ views, float* __restrict__ y, float* __restrict__ cb, float* __restrict__ cr,
+                        int ang, int h, int w) {
+  const int W = ang * w;
+  const long long total = (long long)ang * h * W;
+  for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
+    const int X = (int)(t % W), Y = (int)(t / W);
+    const int u = Y / h, yy = Y - u * h, v = X / w, xx = X - v * w;
+    const T* src = views + ((((long long)u * ang + v) * h + yy) * w + xx) * 3;
+    const double r = view_value(src), g = view_value(src + 1), b = view_value(src + 2);
+    if (y) y[t] = ycbcr_term(r, g, b, 65.481, 128.553, 24.966, 16.0);
+    if (cb) {
+      cb[t] = ycbcr_term(r, g, b, -37.797, -74.203, 112.0, 128.0);
+      cr[t] = ycbcr_term(r, g, b, 112.0, -93.786, -18.214, 128.0);
+    }
+  }
+}
+}  // namespace lfsr
+
+extern "C" int lfsr_rgb_to_ycbcr_mosaic(const void* views, int is_u8, float* y, float* cb, float* cr, int ang, int h, int w,
+                                        void* stream) {
+  LFSR_REQUIRE(views, "lfsr_rgb_to_ycbcr_mosaic: null views");
+  LFSR_REQUIRE(y || cb, "lfsr_rgb_to_ycbcr_mosaic: no output (need Y, CbCr or both)");
+  LFSR_REQUIRE((cb == nullptr) == (cr == nullptr), "lfsr_rgb_to_ycbcr_mosaic: cb and cr go together");
+  LFSR_REQUIRE(ang > 0 && h > 0 && w > 0, "lfsr_rgb_to_ycbcr_mosaic: bad geometry ang=%d h=%d w=%d", ang, h, w);
+  LFSR_REQUIRE((long long)ang * h < (1LL << 31) && (long long)ang * w < (1LL << 31),
+               "lfsr_rgb_to_ycbcr_mosaic: mosaic %lldx%lld too large", (long long)ang * h, (long long)ang * w);
+  const long long total = (long long)ang * h * ang * w;
+  long long blocks = (total + 255) / 256;
+  if (blocks > 148LL * 32) blocks = 148LL * 32;
+  if (is_u8) {
+    lfsr::rgb_ycbcr_mosaic_kernel<unsigned char><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(
+        (const unsigned char*)views, y, cb, cr, ang, h, w);
+  } else {
+    lfsr::rgb_ycbcr_mosaic_kernel<double><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>((const double*)views, y, cb, cr,
+                                                                                          ang, h, w);
+  }
+  return lfsr::check_launch("rgb_ycbcr_mosaic_kernel");
+}

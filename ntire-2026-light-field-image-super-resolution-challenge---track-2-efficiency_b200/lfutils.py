@@ -194,31 +194,56 @@ def imresize(I, scalar_scale=None, method="bicubic", output_shape=None, mode="ve
     else:
         scale = [1.0 * output_shape[0] / H, 1.0 * output_shape[1] / W]
         out_size = [int(output_shape[0]), int(output_shape[1])]
-    lib = N.load()
     cur = t.to(dev).to(torch.float64)
     if cur.dim() == 2:
         cur = cur[:, :, None]
-    cur = cur.contiguous()
-    stream = torch.cuda.current_stream(dev).cuda_stream
-    for dim in np.argsort(np.array(scale)):
-        dim = int(dim)
-        w, ind = resize_contributions(cur.shape[dim], out_size[dim], scale[dim], method)
-        wd, idd = torch.from_numpy(w).to(dev), torch.from_numpy(ind).to(dev)
-        shape = list(cur.shape)
-        outer = 1 if dim == 0 else shape[0]
-        inner = shape[1] * shape[2] if dim == 0 else shape[2]
-        in_len = shape[dim]
-        shape[dim] = out_size[dim]
-        out = torch.empty(shape, dtype=torch.float64, device=dev)
-        N.check(lib.lfsr_resample_f64(cur.data_ptr(), out.data_ptr(), wd.data_ptr(), idd.data_ptr(), outer, in_len, out_size[dim],
-                                      inner, w.shape[1], stream), "lfsr_resample_f64")
-        cur = out.clamp_(0, 255).round_() if is_u8 else out
+    cur = _resample_passes(cur[None], scale, out_size, method, is_u8)[0]
     if is_u8:
         cur = cur.to(torch.uint8)
     if t.dim() == 2:
         cur = cur[:, :, 0]
     cur = cur.to(home)
     return cur.numpy() if as_numpy else cur
+
+
+def _resample_passes(cur: torch.Tensor, scale, out_size, method: str, is_u8: bool = False) -> torch.Tensor:
+    """the two separable passes of imresize over a batch of images: fp64 [N, H, W, C] on the device -> [N, H', W', C].
+    The dimension with the smaller scale goes first (rows first on a tie); one lfsr_resample_f64 launch per pass covers
+    all N images: rows as [N][H][W*C], columns as [N*H'][W][C]. Each output sample is the same tap-order sum as for
+    a single image, so the batch is bit-identical to N separate calls."""
+    dev = cur.device
+    lib = N.load()
+    cur = cur.contiguous()
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    for dim in np.argsort(np.array(scale)):
+        dim = int(dim)
+        w, ind = resize_contributions(cur.shape[dim + 1], out_size[dim], scale[dim], method)
+        wd, idd = torch.from_numpy(w).to(dev), torch.from_numpy(ind).to(dev)
+        shape = list(cur.shape)
+        outer = shape[0] if dim == 0 else shape[0] * shape[1]
+        inner = shape[2] * shape[3] if dim == 0 else shape[3]
+        in_len = shape[dim + 1]
+        shape[dim + 1] = out_size[dim]
+        out = torch.empty(shape, dtype=torch.float64, device=dev)
+        N.check(lib.lfsr_resample_f64(cur.data_ptr(), out.data_ptr(), wd.data_ptr(), idd.data_ptr(), outer, in_len, out_size[dim],
+                                      inner, w.shape[1], stream), "lfsr_resample_f64")
+        cur = out.clamp_(0, 255).round_() if is_u8 else out
+    return cur
+
+
+def imresize_views(views: torch.Tensor, scalar_scale: float, method: str = "bicubic") -> torch.Tensor:
+    """imresize(view, scalar_scale) of every view of a light field at once: fp64 [..., H, W, C] on the device (the
+    leading dimensions, e.g. the A x A views, are flattened) -> fp64 [..., ceil(s H), ceil(s W), C], bit-identical to
+    calling imresize on each view (the float path; uint8 views go through imresize one by one)."""
+    if not views.is_cuda:
+        raise N.LfsrError("lfsr_b200 needs a CUDA device (sm_100a); there is no CPU fallback for this path")
+    if views.dtype != torch.float64 or views.dim() < 3:
+        raise ValueError(f"imresize_views expects fp64 [..., H, W, C] views, got {tuple(views.shape)} {views.dtype}")
+    lead, (H, W, C) = views.shape[:-3], views.shape[-3:]
+    scale = [float(scalar_scale)] * 2
+    out_size = [int(np.ceil(scale[0] * H)), int(np.ceil(scale[1] * W))]
+    out = _resample_passes(views.reshape(-1, H, W, C), scale, out_size, method)
+    return out.reshape(*lead, *out.shape[1:])
 
 
 # ---- colour / BMP tail of test() (train.py:329-341) -------------------------------------------------------------------------
@@ -248,6 +273,89 @@ def sai_to_rgb8_views(sr_y: torch.Tensor, sr_cbcr: torch.Tensor, angRes: int) ->
                                         W // angRes, inv255.ctypes.data, offset.ctypes.data,
                                         torch.cuda.current_stream(dev).cuda_stream), "lfsr_ycbcr_to_rgb8")
     return out
+
+
+# ---- input side: RGB views -> the Lr_SAI_y / Hr_SAI_y / Sr_SAI_cbcr tensors of a test set (include/lfsr.h) ------------------
+def rgb_to_ycbcr_mosaic(views: torch.Tensor, angRes: int, y: bool = True, cbcr: bool = True):
+    """views [a1, a2, h, w, 3] (or [a1*a2, h, w, 3]) on the device, uint8 or fp64 in [0, 1] -> (Y mosaic [(a1 h), (a2 w)],
+    CbCr mosaics [2, (a1 h), (a2 w)]) in fp32, BasicLFSR's term-by-term rgb2ycbcr in one kernel; an output that is not
+    asked for is None."""
+    if not views.is_cuda:
+        raise N.LfsrError("lfsr_b200 needs a CUDA device (sm_100a); there is no CPU fallback for this path")
+    if views.dtype not in (torch.uint8, torch.float64):
+        raise ValueError(f"views must be uint8 or float64, got {views.dtype}")
+    h, w, c = views.shape[-3:]
+    if c != 3 or views.numel() != angRes * angRes * h * w * 3:
+        raise ValueError(f"expected {angRes}x{angRes} RGB views, got {tuple(views.shape)}")
+    if not (y or cbcr):
+        raise ValueError("rgb_to_ycbcr_mosaic: ask for Y, CbCr or both")
+    src = views.contiguous()
+    dev = src.device
+    oy = torch.empty((angRes * h, angRes * w), dtype=torch.float32, device=dev) if y else None
+    oc = torch.empty((2, angRes * h, angRes * w), dtype=torch.float32, device=dev) if cbcr else None
+    ptr = lambda t: None if t is None else t.data_ptr()
+    N.check(N.load().lfsr_rgb_to_ycbcr_mosaic(src.data_ptr(), int(src.dtype == torch.uint8), ptr(oy),
+                                              None if oc is None else oc[0].data_ptr(), None if oc is None else oc[1].data_ptr(),
+                                              angRes, h, w, torch.cuda.current_stream(dev).cuda_stream),
+            "lfsr_rgb_to_ycbcr_mosaic")
+    return oy, oc
+
+
+def central_views(rgb8: np.ndarray, angRes: int, scale: int) -> np.ndarray:
+    """the views the preparation uses, as a host view (no copy): the central angRes x angRes of a [U, V, H, W, 3] grid,
+    each cropped top-left to a multiple of `scale` in height and width."""
+    a = np.asarray(rgb8)
+    if a.ndim != 5 or a.shape[-1] != 3:
+        raise ValueError(f"expected RGB views [U, V, H, W, 3], got {a.shape}")
+    U, V, H, W, _ = a.shape
+    if U < angRes or V < angRes:
+        raise ValueError(f"a {U}x{V} grid of views has no central {angRes}x{angRes}")
+    hc, wc = H - H % scale, W - W % scale
+    if hc == 0 or wc == 0:
+        raise ValueError(f"views of {H}x{W} are smaller than the scale factor {scale}")
+    u0, v0 = (U - angRes) // 2, (V - angRes) // 2
+    return a[u0:u0 + angRes, v0:v0 + angRes, :hc, :wc]
+
+
+_U8_TO_UNIT = {}
+
+
+def _unit(x8: torch.Tensor) -> torch.Tensor:
+    """uint8 -> fp64 k / 255.0, exactly numpy's astype('double') / 255.0: a 256-entry table of correctly rounded quotients
+    (a division by a scalar in torch may become a multiplication by its reciprocal)."""
+    lut = _U8_TO_UNIT.get(x8.device)
+    if lut is None:
+        lut = _U8_TO_UNIT[x8.device] = torch.from_numpy(np.arange(256, dtype=np.float64) / 255.0).to(x8.device)
+    return lut.index_select(0, x8.reshape(-1).to(torch.int32)).view(x8.shape)
+
+
+def prepare_views(rgb8, angRes: int, scale: int, kind: str = "hr"):
+    """RGB views of one scene -> (Lr_SAI_y, Hr_SAI_y or None, Sr_SAI_cbcr) as fp32 mosaics on the current CUDA device,
+    by the recipe of include/lfsr.h. rgb8: host uint8 [U, V, H, W, 3]. kind="hr": the views are ground truth (test.py),
+    the LR input is their bicubic x1/scale; kind="lr": the views are the LR input (inference.py) and there is no HR.
+    The cropped central views cross PCIe once (3 bytes per pixel, from pinned memory); the rest runs on the device."""
+    if kind not in ("hr", "lr"):
+        raise ValueError(f"kind must be 'hr' or 'lr', got {kind!r}")
+    a = np.asarray(rgb8)
+    if a.dtype != np.uint8:
+        raise ValueError(f"prepare_views takes uint8 views, got {a.dtype}")
+    if not torch.cuda.is_available():
+        raise N.LfsrError("lfsr_b200 needs a CUDA device (sm_100a); there is no CPU fallback for this path")
+    dev = torch.device("cuda", torch.cuda.current_device())
+    crop = central_views(a, angRes, scale)
+    host = torch.empty(crop.shape, dtype=torch.uint8, pin_memory=True)
+    host.numpy()[...] = crop
+    x8 = host.to(dev, non_blocking=True)
+    A = angRes
+    if kind == "hr":
+        hr_y, _ = rgb_to_ycbcr_mosaic(x8, A, cbcr=False)
+        lr_rgb = imresize_views(_unit(x8), 1.0 / scale)
+        lr_y, _ = rgb_to_ycbcr_mosaic(lr_rgb, A, cbcr=False)
+    else:
+        hr_y, lr_rgb = None, _unit(x8)
+        lr_y, _ = rgb_to_ycbcr_mosaic(x8, A, cbcr=False)
+    _, sr_cbcr = rgb_to_ycbcr_mosaic(imresize_views(lr_rgb, float(scale)), A, y=False)
+    return lr_y, hr_y, sr_cbcr
 
 
 def write_bmp(path, img) -> None:

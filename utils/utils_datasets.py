@@ -1,9 +1,15 @@
 """Test-set loaders for the entry points (the reference's utils/utils_datasets.py:61-136 on the
 inference path). Disk I/O is outside the accelerated path (SURVEY 2 #12): this module only has to
 yield the same 5-tuples `(Lr_SAI_y[1,1,AH,AW], Hr_SAI_y, Sr_SAI_cbcr, [angRes_in, angRes_out], [name])`
-the reference's DataLoader(batch_size=1) yields. h5 datasets need h5py; `--synthetic N` produces
-seeded scenes so the whole entry point can run without any dataset."""
+the reference's DataLoader(batch_size=1) yields. Three sources, chosen by MultiTestSetDataLoader:
+- `--synthetic N`: seeded scenes, so the whole entry point can run without any dataset;
+- h5 files under <path_for_test>/SR_AxA_sx/<data_name>/ (BasicLFSR's prepared test sets; needs h5py);
+- light fields stored as view images, <path_for_test>/<data_name>/<scene>/View_u_v.{png,bmp} with 0-based u, v (the
+  layout inference.py writes). They are decoded with Pillow on the host and prepared on the GPU
+  (lfsr_b200.lfutils.prepare_views: central A x A views, crop, rgb2ycbcr, bicubic LR / SR colour), so no offline
+  generator step is needed: test.py reads them as ground truth, inference.py as LR input."""
 import os
+import re
 
 import numpy as np
 import torch
@@ -74,11 +80,133 @@ class H5TestSet:
             yield self[i]
 
 
-def MultiTestSetDataLoader(args):
+_VIEW_FILE = re.compile(r"View_(\d+)_(\d+)\.(png|bmp)$", re.IGNORECASE)
+
+
+def _scene_dirs(path):
+    """sub-directories of `path` that hold at least one View_u_v image, sorted by name."""
+    if not os.path.isdir(path):
+        return []
+    out = []
+    for d in sorted(os.listdir(path)):
+        full = os.path.join(path, d)
+        if os.path.isdir(full) and any(_VIEW_FILE.match(f) for f in os.listdir(full)):
+            out.append(d)
+    return out
+
+
+def _check_rgb8(im, fn):
+    """8-bit RGB only: Pillow also opens 48-bit PNGs as mode RGB, so look at the raw mode of the encoded data too."""
+    if im.mode != "RGB":
+        raise ValueError(f"{fn}: mode {im.mode} is not supported (8-bit RGB views only)")
+    for tile in getattr(im, "tile", None) or []:
+        args = tile[3] if len(tile) > 3 else None
+        raw = args[0] if isinstance(args, tuple) and args else args
+        if isinstance(raw, str) and (";16" in raw or ";15" in raw):
+            raise ValueError(f"{fn}: 16-bit samples are not supported (8-bit RGB views only)")
+
+
+def read_views(scene_dir, ang):
+    """the central ang x ang views of one scene folder of View_u_v.{png,bmp} images -> uint8 [ang, ang, H, W, 3].
+    Every view of the grid must be present, 8-bit RGB and of one size (headers only are read for the views outside
+    the centre); only the central views are decoded. Raises ValueError naming the file and the problem."""
+    from PIL import Image
+    files = {}
+    for f in sorted(os.listdir(scene_dir)):
+        m = _VIEW_FILE.match(f)
+        if m:
+            key = (int(m.group(1)), int(m.group(2)))
+            if key in files:
+                raise ValueError(f"{os.path.join(scene_dir, f)}: view {key} is stored twice "
+                                 f"(also {os.path.basename(files[key])})")
+            files[key] = os.path.join(scene_dir, f)
+    if not files:
+        raise ValueError(f"{scene_dir}: no View_u_v.png or View_u_v.bmp images")
+    U = max(u for u, _ in files) + 1
+    V = max(v for _, v in files) + 1
+    for u in range(U):
+        for v in range(V):
+            if (u, v) not in files:
+                raise ValueError(f"{os.path.join(scene_dir, 'View_%d_%d.png|bmp' % (u, v))}: view is missing "
+                                 f"from the {U}x{V} grid")
+    if U < ang or V < ang:
+        raise ValueError(f"{scene_dir}: a {U}x{V} grid of views is smaller than angRes {ang}x{ang}")
+    size = None
+    for (u, v), fn in sorted(files.items()):
+        with Image.open(fn) as im:
+            _check_rgb8(im, fn)
+            if size is None:
+                size, first = im.size, fn
+            elif im.size != size:
+                raise ValueError(f"{fn}: view is {im.size[0]}x{im.size[1]} (WxH) but {first} is {size[0]}x{size[1]}")
+    u0, v0 = (U - ang) // 2, (V - ang) // 2
+    out = np.empty((ang, ang, size[1], size[0], 3), dtype=np.uint8)
+    for i in range(ang):
+        for j in range(ang):
+            with Image.open(files[(u0 + i, v0 + j)]) as im:
+                out[i, j] = np.asarray(im)
+    return out
+
+
+def prepare_views(rgb8, ang, scale, kind):
+    """the device preparation (a module attribute, so that tests on machines without a GPU can substitute the oracle)."""
+    from lfsr_b200 import lfutils
+    return lfutils.prepare_views(rgb8, ang, scale, kind)
+
+
+class ViewsTestSet:
+    """one dataset directory <path_for_test>/<data_name>/ of scene folders of View_u_v.{png,bmp} images. kind="hr":
+    the views are ground truth (test.py: LR input = their bicubic x1/s); kind="lr": the views are the LR input
+    (inference.py; Hr_SAI_y is an empty tensor). Yields the batch-1 5-tuple with the tensors on the current CUDA device;
+    __getitem__ decodes only the scene asked for."""
+
+    def __init__(self, args, data_name, kind):
+        if kind not in ("hr", "lr"):
+            raise ValueError(f"kind must be 'hr' or 'lr', got {kind!r}")
+        self.args, self.kind = args, kind
+        self.root = os.path.join(args.path_for_test, data_name)
+        self.scenes = _scene_dirs(self.root)
+
+    def __len__(self):
+        return len(self.scenes)
+
+    def __getitem__(self, i):
+        if not 0 <= i < len(self.scenes):
+            raise IndexError(i)
+        A, s = self.args.angRes_in, self.args.scale_factor
+        rgb8 = read_views(os.path.join(self.root, self.scenes[i]), A)
+        lr, hr, cbcr = prepare_views(rgb8, A, s, self.kind)
+        if hr is None:
+            hr = lr.new_empty((0, 0))
+        return _batch1(lr[None], hr[None], cbcr, A, self.args.angRes_out, self.scenes[i])
+
+    def __iter__(self):
+        for i in range(len(self)):
+            yield self[i]
+
+
+def MultiTestSetDataLoader(args, views=None):
+    """(dataset names, loaders, total scenes). --synthetic N wins; then BasicLFSR's h5 layout
+    <path_for_test>/SR_AxA_sx/<data_name>/*.h5 if that directory exists (or `views` is None); otherwise light fields
+    stored as view images, <path_for_test>/<data_name>/<scene>/View_u_v.{png,bmp}, read as `views` = "hr" (ground
+    truth, test.py) or "lr" (LR input, inference.py)."""
     if getattr(args, "synthetic", 0) > 0:
         ds = SyntheticTestSet(args, args.synthetic, args.synthetic_size)
         return ["Synthetic"], [ds], len(ds)
     base = os.path.join(args.path_for_test, "SR_%dx%d_%dx" % (args.angRes_in, args.angRes_in, args.scale_factor))
-    names = sorted(os.listdir(base)) if args.data_name == "ALL" else [args.data_name]
-    loaders = [H5TestSet(args, n) for n in names]
-    return names, loaders, sum(len(d) for d in loaders)
+    if views is None or os.path.isdir(base):
+        names = sorted(os.listdir(base)) if args.data_name == "ALL" else [args.data_name]
+        loaders = [H5TestSet(args, n) for n in names]
+        return names, loaders, sum(len(d) for d in loaders)
+    root = args.path_for_test
+    if args.data_name == "ALL":
+        names = [d for d in sorted(os.listdir(root)) if _scene_dirs(os.path.join(root, d))] if os.path.isdir(root) else []
+    else:
+        names = [args.data_name]
+    loaders = [ViewsTestSet(args, n, views) for n in names]
+    n_scenes = sum(len(d) for d in loaders)
+    if n_scenes == 0:
+        raise FileNotFoundError(
+            f"no test data under {root}: expected either h5 files in {base}/<data_name>/ or scene folders of "
+            f"View_u_v.png|bmp images in {os.path.join(root, '<data_name>')}/<scene>/ (data_name {args.data_name})")
+    return names, loaders, n_scenes
