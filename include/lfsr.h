@@ -182,6 +182,29 @@ int lfsr_rgb_to_ycbcr_mosaic(const void* views, int is_u8, float* y, float* cb, 
 int lfsr_resample_f64(const double* in, double* out, const double* weights, const int32_t* indices, int outer,
                       int in_len, int out_len, int inner, int taps, void* stream);
 
+/* ---- Angular window tiling (no counterpart in the reference; DESIGN.md row f-8): every view of a light field larger than
+ * the A x A a network was trained for (A = angRes), off by default (--full_grid 1).
+ *   grid     N = min(U, V) of a U x V grid of views; the central N x N by the rule of "View preparation" (u0 = (U - N) // 2,
+ *            v0 = (V - N) // 2); N >= A. Square only: the metric and colour kernels take one angular size.
+ *   origins  along each angular axis, for a stride t with 1 <= t <= A - 1 when N > A (default t = A - 1, the fewest windows
+ *            that cover the grid): 0, t, 2t, ... while < N - A, then N - A. N = A: the single origin 0. E.g. N = 9, A = 5:
+ *            {0, 4}; N = 14, A = 5: {0, 4, 8, 9}.
+ *   windows  the pairs (o_u, o_v) in row-major order of (o_u, o_v); that order is the summation order.
+ *   window   the LR Y mosaic of views [o_u, o_u + A) x [o_v, o_v + A) through the scene pipeline unchanged (LFdivide ->
+ *            forward -> LFintegrate, with the x8 self-ensemble when it is on) -> an SR window mosaic [(A hs), (A ws)].
+ *   merge    SR view (u, v) of the N x N mosaic = (((W_k1 + W_k2) + ...) + W_kc) / c over the windows k1 < k2 < ... that
+ *            contain it, c their count: fp32 sums with __fadd_rn, one __fdiv_rn by (float)c; c = 1 is a plain copy. This is
+ *            what torch's fp32 `a + b` then `/ c` (c as a tensor: a Python scalar divisor may become a reciprocal multiply)
+ *            computes, bit for bit.
+ *
+ * lfsr_window_accumulate: merges one SR window mosaic `win` [(ang h)][(ang w)] into the N x N mosaic `grid` [(n h)][(n w)] at
+ * view offset (o_u, o_v). host_modes[a1 * ang + a2] (a host array of ang * ang) is the step for window view (a1, a2):
+ * 0 = store (the first window over that view), 1 = add, c >= 2 = add then divide by c (the last of its c windows). So the
+ * merge needs no zeroing and no normalising pass. float4 loads and stores when w % 4 == 0. LFSR_ERR_INVALID for n < ang,
+ * ang > 16, a window outside the grid, overlapping mosaics or a mode outside [0, min(ang, n - ang + 1)^2]. */
+int lfsr_window_accumulate(const float* win, float* grid, int ang, int n, int h, int w, int o_u, int o_v,
+                           const int32_t* host_modes, void* stream);
+
 /* ---- convolutions --------------------------------------------------------------------- */
 /* fp32 CUDA-core implicit GEMM; weights packed [kh*kw][cin][cout]. */
 int lfsr_conv2d_f32(const lfsr_tensor* in, const float* w_packed, const lfsr_tensor* out,

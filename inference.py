@@ -4,7 +4,9 @@ metrics; writes View_i_j.bmp per scene. The reference's fvcore FLOP probe (:117-
 there (wrapped in try/except) and is not reproduced.
 
 Under torchrun (WORLD_SIZE > 1) each dataset is split across the ranks like test.py's (train.rank_scenes); every
-View_i_j.bmp is written once, by the rank that owns its scene, and only rank 0 prints."""
+View_i_j.bmp is written once, by the rank that owns its scene, and only rank 0 prints. With --full_grid 1 every view of
+the central N x N of each light field is super-resolved with overlapping angRes x angRes windows
+(scene.super_resolve_grid) and N^2 View_i_j.bmp are written."""
 import importlib
 
 import torch
@@ -13,7 +15,7 @@ from utils.utils import create_dir
 from utils.utils_datasets import MultiTestSetDataLoader
 from lfsr_b200 import scene as _scene
 from test import broadcast_weights, finish_distributed, init_distributed, load_checkpoint
-from train import _write_views, dist_world, gather_in_order, rank_scenes
+from train import _write_views, dist_world, gather_in_order, grid_size, rank_scenes
 
 
 def main(args):
@@ -40,6 +42,7 @@ def run(args, device, rank):
     net = net.to(device).eval()
     broadcast_weights(net)
     world, _ = dist_world()
+    full_grid = bool(getattr(args, "full_grid", 0))
     with torch.no_grad():
         for name, loader in zip(test_names, test_loaders):
             save_dir = result_dir.joinpath(name)
@@ -48,11 +51,19 @@ def run(args, device, rank):
             for i, solo, owner, (Lr_SAI_y, _hr, cbcr, data_info, lf_name) in rank_scenes(loader, world, rank):
                 ang = int(data_info[0][0].item())
                 shard = dict(world=1, rank=0) if solo else {}
-                sr = _scene.super_resolve_scene(net, Lr_SAI_y.squeeze().to(device), ang, args.scale_factor,
-                                                args.patch_size_for_test, args.stride_for_test, args.minibatch,
-                                                self_ensemble=bool(getattr(args, "self_ensemble", 0)), **shard)
+                if full_grid:
+                    views = grid_size(data_info)
+                    sr = _scene.super_resolve_grid(net, Lr_SAI_y.squeeze().to(device), views, args.angRes_in,
+                                                   args.scale_factor, args.patch_size_for_test, args.stride_for_test,
+                                                   args.minibatch, ang_stride=getattr(args, "ang_stride", 0) or None,
+                                                   self_ensemble=bool(getattr(args, "self_ensemble", 0)), **shard)
+                else:
+                    views = args.angRes_out
+                    sr = _scene.super_resolve_scene(net, Lr_SAI_y.squeeze().to(device), ang, args.scale_factor,
+                                                    args.patch_size_for_test, args.stride_for_test, args.minibatch,
+                                                    self_ensemble=bool(getattr(args, "self_ensemble", 0)), **shard)
                 if owner:
-                    _write_views(save_dir, lf_name[0], sr, cbcr, args.angRes_out)
+                    _write_views(save_dir, lf_name[0], sr, cbcr, views)
                     written.append((i, lf_name[0]))
                     if world == 1:
                         print("scene %s -> %s" % (lf_name[0], save_dir))

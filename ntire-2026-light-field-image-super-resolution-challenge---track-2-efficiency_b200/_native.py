@@ -94,6 +94,7 @@ SIGNATURES = {
     "lfsr_ycbcr_to_rgb8": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
     "lfsr_resample_f64": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "lfsr_rgb_to_ycbcr_mosaic": (_I, [_P, _I, _P, _P, _P, _I, _I, _I, _P]),
+    "lfsr_window_accumulate": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _P, _P]),
     "lfsr_conv2d_f32": (_I, [_TP, _P, _TP, C.POINTER(ConvDesc), _P]),
     "lfsr_dwconv_f32": (_I, [_TP, _P, _P, _P, _TP, _I, _I, _I, _I, _I, C.c_float, _P]),
     "lfsr_dwconv_multi": (_I, [_TP, _TP, C.POINTER(DwBranch), _I, _P]),

@@ -475,3 +475,82 @@ extern "C" int lfsr_rgb_to_ycbcr_mosaic(const void* views, int is_u8, float* y, 
   }
   return lfsr::check_launch("rgb_ycbcr_mosaic_kernel");
 }
+
+
+// ---- angular window tiling (include/lfsr.h, "Angular window tiling"): one SR window mosaic [(A h), (A w)] merged into the
+// N x N SR mosaic [(N h), (N w)] at view offset (o_u, o_v). Per view of the window a mode: 0 = store, 1 = add, c >= 2 = add,
+// then divide by c (the last window over that view). Sums with __fadd_rn, the mean with one __fdiv_rn: fp32 `a + b` and
+// `a / c` in torch give the same bits. One thread = VEC consecutive x of one view row, in window-mosaic order, so the window
+// reads are dense; a window row lands as one contiguous run of the grid row (views o_v .. o_v + A - 1 are adjacent there).
+namespace lfsr {
+constexpr int WIN_MAX_ANG = 16;
+struct WinModes { int m[WIN_MAX_ANG * WIN_MAX_ANG]; };
+
+__device__ __forceinline__ float win_merge(float acc, float v, int mode) {
+  const float s = __fadd_rn(acc, v);
+  return mode == 1 ? s : __fdiv_rn(s, (float)mode);
+}
+
+template <int VEC>
+__global__ void __launch_bounds__(256)
+window_accumulate_kernel(const float* __restrict__ win, float* __restrict__ grid, int A, int N, int h, int w, int o_u,
+                         int o_v, WinModes md) {
+  const int wv = w / VEC;
+  for (int Y = blockIdx.y; Y < A * h; Y += gridDim.y) {
+    const int a1 = Y / h, y = Y - a1 * h;
+    const float* src = win + (size_t)Y * A * w;
+    float* dst = grid + ((size_t)(o_u + a1) * h + y) * ((size_t)N * w) + (size_t)o_v * w;
+    for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < A * wv; t += gridDim.x * blockDim.x) {
+      const int a2 = t / wv;
+      const int X = a2 * w + (t - a2 * wv) * VEC;
+      const int mode = md.m[a1 * A + a2];
+      if (VEC == 4) {
+        float4 v = __ldg(reinterpret_cast<const float4*>(src + X));
+        float4* o = reinterpret_cast<float4*>(dst + X);
+        if (mode != 0) {
+          const float4 a = *o;
+          v = make_float4(win_merge(a.x, v.x, mode), win_merge(a.y, v.y, mode), win_merge(a.z, v.z, mode),
+                          win_merge(a.w, v.w, mode));
+        }
+        *o = v;
+      } else {
+        const float v = __ldg(src + X);
+        dst[X] = mode == 0 ? v : win_merge(dst[X], v, mode);
+      }
+    }
+  }
+}
+}  // namespace lfsr
+
+extern "C" int lfsr_window_accumulate(const float* win, float* grid, int ang, int n, int h, int w, int o_u, int o_v,
+                                      const int32_t* host_modes, void* stream) {
+  using lfsr::WIN_MAX_ANG;
+  LFSR_REQUIRE(win && grid && host_modes, "lfsr_window_accumulate: null pointer");
+  LFSR_REQUIRE(ang > 0 && ang <= WIN_MAX_ANG && h > 0 && w > 0, "lfsr_window_accumulate: bad geometry A=%d h=%d w=%d "
+               "(1 <= A <= %d)", ang, h, w, WIN_MAX_ANG);
+  LFSR_REQUIRE(n >= ang, "lfsr_window_accumulate: a %dx%d grid is smaller than the %dx%d window", n, n, ang, ang);
+  LFSR_REQUIRE((long long)n * h < (1LL << 31) && (long long)n * w < (1LL << 31),
+               "lfsr_window_accumulate: mosaic %lldx%lld too large", (long long)n * h, (long long)n * w);
+  LFSR_REQUIRE(0 <= o_u && o_u <= n - ang && 0 <= o_v && o_v <= n - ang,
+               "lfsr_window_accumulate: window at (%d, %d) lies outside the %dx%d grid (A=%d)", o_u, o_v, n, n, ang);
+  const long long win_n = (long long)ang * h * ang * w, grid_n = (long long)n * h * n * w;
+  LFSR_REQUIRE(win + win_n <= grid || grid + grid_n <= win, "lfsr_window_accumulate: window and grid mosaics overlap");
+  // a view lies in at most A windows per angular axis (distinct origins in (u - A, u]) and in at most N - A + 1
+  const int per_axis = ang < n - ang + 1 ? ang : n - ang + 1;
+  lfsr::WinModes md;
+  for (int i = 0; i < ang * ang; ++i) {
+    LFSR_REQUIRE(host_modes[i] >= 0 && host_modes[i] <= per_axis * per_axis,
+                 "lfsr_window_accumulate: bad mode %d for view %d (0 store, 1 add, 2..%d add then divide)", host_modes[i],
+                 i, per_axis * per_axis);
+    md.m[i] = host_modes[i];
+  }
+  const int rows = ang * h;
+  const bool vec = w % 4 == 0 && (uintptr_t)win % 16 == 0 && (uintptr_t)grid % 16 == 0;
+  const int per_row = vec ? ang * (w / 4) : ang * w;
+  dim3 g(ceil_div(per_row, 256), rows < 32768 ? rows : 32768);
+  if (vec)
+    lfsr::window_accumulate_kernel<4><<<g, 256, 0, (cudaStream_t)stream>>>(win, grid, ang, n, h, w, o_u, o_v, md);
+  else
+    lfsr::window_accumulate_kernel<1><<<g, 256, 0, (cudaStream_t)stream>>>(win, grid, ang, n, h, w, o_u, o_v, md);
+  return lfsr::check_launch("window_accumulate_kernel");
+}

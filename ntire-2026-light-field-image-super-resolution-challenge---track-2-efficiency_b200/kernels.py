@@ -171,6 +171,18 @@ class CudaOps:
         N.check(self.lib.lfsr_integrate_rows_d8(patches8.data_ptr(), out.data_ptr(), ang, pz, stride, h, w, num_u, num_v,
                                                 u0, u1, self._stream(out)), "lfsr_integrate_rows_d8")
 
+    def window_accumulate(self, win, grid, ang, n, h, w, o_u, o_v, modes):
+        """merge the SR window mosaic win [(ang h), (ang w)] into the N x N mosaic grid [(n h), (n w)] at view offset
+        (o_u, o_v); modes: ang * ang ints, per window view 0 = store, 1 = add, c >= 2 = add then divide by c
+        (include/lfsr.h, "Angular window tiling")"""
+        if not (win.is_contiguous() and grid.is_contiguous() and win.dtype == grid.dtype == torch.float32):
+            raise N.LfsrError("window_accumulate: dense fp32 mosaics required")
+        if len(modes) != ang * ang:
+            raise N.LfsrError(f"window_accumulate: {len(modes)} modes for {ang * ang} window views")
+        m = (C.c_int32 * (ang * ang))(*[int(x) for x in modes])
+        N.check(self.lib.lfsr_window_accumulate(win.data_ptr(), grid.data_ptr(), ang, n, h, w, o_u, o_v, m,
+                                                self._stream(grid)), "lfsr_window_accumulate")
+
     def interp(self, x, out, n, h, w, scale, mode, block_h, block_w):
         N.check(self.lib.lfsr_interp(x.data_ptr(), out.data_ptr(), n, h, w, scale, mode, block_h, block_w,
                                      self._stream(x)), "lfsr_interp")

@@ -264,17 +264,22 @@ class SceneRunner:
         return psnr, ssim, (s["host_sr"] if s["readback"] else s["mosaic"])
 
     def metrics_from_sums(self, acc):
-        A = self.ang
-        a = np.asarray(acc, dtype=np.float64).reshape(A, A, 2)
-        mse = a[..., 0] / float(self.hs * self.ws)
-        with np.errstate(divide="ignore"):
-            P = (10.0 * np.log10(1.0 / mse)).astype(np.float32)
-        S = (a[..., 1] / float((self.hs - 10) * (self.ws - 10))).astype(np.float32)
-        vp, vs = np.sum(P > 0), np.sum(S > 0)
-        return (P.sum() / vp if vp > 0 else 0.0), (S.sum() / vs if vs > 0 else 0.0)
+        return metrics_from_sums(acc, self.ang, self.hs, self.ws)
 
     def device_slot(self, k: int = 0):
         return self.slots[k % self.depth]
+
+
+def metrics_from_sums(acc, ang: int, hs: int, ws: int):
+    """(psnr, ssim) from the per-view sums of lfsr_metric_sums over an ang x ang mosaic of hs x ws views: means over views
+    with value > 0, as utils/utils.py:121-134."""
+    a = np.asarray(acc, dtype=np.float64).reshape(ang, ang, 2)
+    mse = a[..., 0] / float(hs * ws)
+    with np.errstate(divide="ignore"):
+        P = (10.0 * np.log10(1.0 / mse)).astype(np.float32)
+    S = (a[..., 1] / float((hs - 10) * (ws - 10))).astype(np.float32)
+    vp, vs = np.sum(P > 0), np.sum(S > 0)
+    return (P.sum() / vp if vp > 0 else 0.0), (S.sum() / vs if vs > 0 else 0.0)
 
 
 class _NullCtx:
@@ -377,4 +382,109 @@ def test_scene(net, lr_sai, hr_sai, ang: int, scale: int, patch: int = 32, strid
     r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops, world=world, rank=rank,
                    self_ensemble=self_ensemble)
     psnr, ssim, sr = r.result(r.submit(lr_sai, hr_sai, readback=False))
+    return psnr, ssim, sr
+
+
+# -- angular window tiling (include/lfsr.h, "Angular window tiling"; DESIGN.md row f-8) ---------------------------------------
+def window_origins(n: int, ang: int, stride: Optional[int] = None):
+    """origins of the A x A windows along one angular axis of an N-view grid: 0, t, 2t, ... while < N - A, then N - A.
+    stride t in [1, A - 1] (None or 0: A - 1, the fewest windows that cover the grid); N = A gives the one origin 0."""
+    n, ang = int(n), int(ang)
+    if ang < 1 or n < ang:
+        raise ValueError(f"window_origins: a {n}-view axis has no {ang}-view window")
+    if n == ang:
+        return [0]
+    t = ang - 1 if not stride else int(stride)
+    if not 1 <= t <= ang - 1:
+        raise ValueError(f"window_origins: angular stride {t} outside [1, {ang - 1}] (neighbouring windows of {ang} views "
+                         f"share at least one view)")
+    return list(range(0, n - ang, t)) + [n - ang]
+
+
+def window_plan(n: int, ang: int, stride: Optional[int] = None):
+    """[(o_u, o_v, modes)] in window order (row-major in (o_u, o_v)); modes[a1 * ang + a2] is the lfsr_window_accumulate step
+    for window view (a1, a2): 0 = store (first window over the view), 1 = add, c >= 2 = add then divide by the view's
+    window count c (last window over it)."""
+    orig = window_origins(n, ang, stride)
+    cover = [[i for i, o in enumerate(orig) if o <= x < o + ang] for x in range(n)]
+    plan = []
+    for i, ou in enumerate(orig):
+        for j, ov in enumerate(orig):
+            modes = []
+            for a1 in range(ang):
+                cu = cover[ou + a1]
+                for a2 in range(ang):
+                    cv = cover[ov + a2]
+                    if (i, j) == (cu[0], cv[0]):
+                        modes.append(0)
+                    elif (i, j) == (cu[-1], cv[-1]):
+                        modes.append(len(cu) * len(cv))
+                    else:
+                        modes.append(1)
+            plan.append((ou, ov, modes))
+    return plan
+
+
+def _grid_run(net, lr_sai, n, ang, scale, patch, stride, minibatch, group, ops, ang_stride, self_ensemble, world, rank):
+    """(runner, N x N SR mosaic): every window through the scene pipeline of one runner, merged as it completes."""
+    lr = lr_sai.reshape(lr_sai.shape[-2:])
+    n, ang = int(n), int(ang)
+    H, W = lr.shape
+    if H % n or W % n:
+        raise ValueError(f"super_resolve_grid: LR mosaic {H}x{W} is not a {n}x{n} grid of views")
+    h0, w0 = H // n, W // n
+    plan = window_plan(n, ang, ang_stride)
+    dev = lr.device
+    if not lr.is_cuda:
+        try:
+            dev = next(net.parameters()).device
+        except StopIteration:
+            pass
+    r = runner_for(net, ang, scale, h0, w0, patch, stride, minibatch, dev, ops, group, world, rank,
+                   self_ensemble=self_ensemble)
+    # the windows go through one slot of the runner, taken in turn like a submitted scene (so a test_scene mosaic stays
+    # valid as long as documented there)
+    s = r.slots[r._n % r.depth]
+    if s["busy"]:
+        raise RuntimeError("super_resolve_grid: the runner's next slot is in flight - call result() first")
+    r._n += 1
+    out = torch.empty((n * r.hs, n * r.ws), dtype=torch.float32, device=dev)
+    ctx = torch.cuda.device(dev) if dev.type == "cuda" else _NullCtx()
+    with ctx:
+        views = lr.to(device=dev, dtype=torch.float32).contiguous().view(n, h0, n, w0)
+        win_lr = s["lr"].view(ang, h0, ang, w0)
+        for ou, ov, modes in plan:
+            win_lr.copy_(views[ou:ou + ang, :, ov:ov + ang, :])
+            r.run_resident(s["lr"], s["mosaic"])
+            r.ops.window_accumulate(s["mosaic"], out, ang, n, r.hs, r.ws, ou, ov, modes)
+    return r, out
+
+
+def super_resolve_grid(net, lr_sai: torch.Tensor, n: int, ang: int, scale: int, patch: int = 32, stride: int = 16,
+                       minibatch: int = 64, group=None, ops=None, ang_stride: Optional[int] = None,
+                       self_ensemble: bool = False, world: Optional[int] = None, rank: Optional[int] = None) -> torch.Tensor:
+    """Every view of an N x N light field with a network for A x A inputs (A = ang): lr_sai [(N h0), (N w0)] -> the device
+    SR mosaic [(N h0 s), (N w0 s)] owned by the caller. The A x A windows of window_plan(N, A, ang_stride) each run exactly
+    what super_resolve_scene runs (row-sharded and all-gathered like a scene under a process group, so the result is the
+    same on every rank); lfsr_window_accumulate averages the views several windows produce. N = A is super_resolve_scene."""
+    return _grid_run(net, lr_sai, n, ang, scale, patch, stride, minibatch, group, ops, ang_stride, self_ensemble, world,
+                     rank)[1]
+
+
+def test_grid(net, lr_sai, hr_sai, n: int, ang: int, scale: int, patch: int = 32, stride: int = 16, minibatch: int = 64,
+              ops=None, ang_stride: Optional[int] = None, self_ensemble: bool = False, world: Optional[int] = None,
+              rank: Optional[int] = None):
+    """(psnr, ssim, sr_mosaic) of super_resolve_grid against the N x N HR mosaic: means over all N^2 views with value > 0,
+    as test_scene's over A^2."""
+    r, sr = _grid_run(net, lr_sai, n, ang, scale, patch, stride, minibatch, None, ops, ang_stride, self_ensemble, world,
+                      rank)
+    hr = hr_sai.reshape(hr_sai.shape[-2:])
+    if tuple(hr.shape) != tuple(sr.shape):
+        raise ValueError(f"HR label {tuple(hr.shape)} does not match the SR mosaic {tuple(sr.shape)}")
+    n = int(n)
+    acc = torch.zeros(2 * n * n, dtype=torch.float64, device=sr.device)
+    ctx = torch.cuda.device(sr.device) if sr.is_cuda else _NullCtx()
+    with ctx:
+        r.ops.metric_sums(hr.to(device=sr.device, dtype=torch.float32).contiguous(), sr, n, r.hs, r.ws, acc)
+    psnr, ssim = metrics_from_sums(acc.cpu().numpy(), n, r.hs, r.ws)
     return psnr, ssim, sr

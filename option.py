@@ -2,7 +2,8 @@
 reference's option.py:4-34 (including its `type=bool` quirk: any non-empty string is True, so the
 random-init path needs --use_pre_ckpt ''), parsed at import time like the reference because
 utils/utils.py and the entry points do `from option import args`.
-Additive flags (not in the reference): --synthetic, --synthetic_size, --minibatch, --self_ensemble."""
+Additive flags (not in the reference): --synthetic, --synthetic_size, --minibatch, --self_ensemble, --full_grid,
+--ang_stride."""
 import argparse
 
 _FLAGS = [
@@ -33,6 +34,10 @@ _FLAGS = [
     ("--synthetic_size", dict(type=int, default=64, help="view height/width of the synthetic LR scenes")),
     ("--minibatch", dict(type=int, default=64, help="patches per forward on the device path")),
     ("--self_ensemble", dict(type=int, default=0, help="1: x8 flip/transpose self-ensemble per patch (8x the forwards)")),
+    ("--full_grid", dict(type=int, default=0, help="1: super-resolve every view of the central N x N (N = min(U, V)) of "
+                         "view-image light fields with overlapping angRes x angRes windows, averaged where they overlap")),
+    ("--ang_stride", dict(type=int, default=0, help="angular stride of the --full_grid windows, 1..angRes-1 "
+                          "(0: angRes - 1, the fewest windows)")),
 ]
 
 parser = argparse.ArgumentParser()

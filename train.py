@@ -7,7 +7,10 @@ a host round trip per patch) -> LFintegrate -> PSNR/SSIM -> YCbCr->RGB uint8 vie
 kernels; one D2H copy of the uint8 views per scene feeds the BMP writer.
 
 With torch.distributed initialised (test.py / inference.py under torchrun), a dataset is split across the ranks by
-`scene.assign_scenes`: full rounds of scenes run one per rank, the remaining scenes are row-sharded over all ranks."""
+`scene.assign_scenes`: full rounds of scenes run one per rank, the remaining scenes are row-sharded over all ranks.
+
+With --full_grid 1 every scene is the central N x N of a larger light field (data_info [A, A, N]); it runs through
+`scene.test_grid`: overlapping A x A windows (A = args.angRes_in), averaged where they overlap, N^2 views written."""
 import torch
 
 from lfsr_b200 import scene as _scene
@@ -73,9 +76,18 @@ def gather_in_order(rows, world):
     return sorted((r for p in parts for r in p), key=lambda r: r[0])
 
 
+def grid_size(data_info):
+    """N of a full-grid scene: the third data_info entry (utils_datasets.ViewsTestSet with full_grid)."""
+    if len(data_info) < 3:
+        raise ValueError("--full_grid 1: the loader did not report the grid size of the scene")
+    n = data_info[2]
+    return int(n[0].item()) if torch.is_tensor(n) else int(n)
+
+
 def test(test_loader, device, net, args, save_dir=None):
     net.eval()
     world, rank = dist_world()
+    full_grid = bool(getattr(args, "full_grid", 0))
     rows = []
     for i, solo, owner, (Lr_SAI_y, Hr_SAI_y, Sr_SAI_cbcr, data_info, LF_name) in rank_scenes(test_loader, world, rank):
         ang = int(data_info[0][0].item()) if torch.is_tensor(data_info[0]) else int(data_info[0])
@@ -83,12 +95,21 @@ def test(test_loader, device, net, args, save_dir=None):
         lr, hr = Lr_SAI_y.squeeze(), Hr_SAI_y.squeeze()
         shard = dict(world=1, rank=0) if solo else {}
         with torch.no_grad():
-            psnr, ssim, sr = _scene.test_scene(net, lr, hr, ang, args.scale_factor, args.patch_size_for_test,
-                                               args.stride_for_test, getattr(args, "minibatch", 64),
-                                               self_ensemble=bool(getattr(args, "self_ensemble", 0)), **shard)
+            if full_grid:
+                views = grid_size(data_info)
+                psnr, ssim, sr = _scene.test_grid(net, lr, hr, views, args.angRes_in, args.scale_factor,
+                                                  args.patch_size_for_test, args.stride_for_test,
+                                                  getattr(args, "minibatch", 64),
+                                                  ang_stride=getattr(args, "ang_stride", 0) or None,
+                                                  self_ensemble=bool(getattr(args, "self_ensemble", 0)), **shard)
+            else:
+                views = args.angRes_out
+                psnr, ssim, sr = _scene.test_scene(net, lr, hr, ang, args.scale_factor, args.patch_size_for_test,
+                                                   args.stride_for_test, getattr(args, "minibatch", 64),
+                                                   self_ensemble=bool(getattr(args, "self_ensemble", 0)), **shard)
         if owner:
             rows.append((i, psnr, ssim, LF_name[0]))
             if save_dir is not None:
-                _write_views(save_dir, LF_name[0], sr, Sr_SAI_cbcr, args.angRes_out)
+                _write_views(save_dir, LF_name[0], sr, Sr_SAI_cbcr, views)
     rows = gather_in_order(rows, world)
     return [r[1] for r in rows], [r[2] for r in rows], [r[3] for r in rows]

@@ -15,8 +15,10 @@ import numpy as np
 import torch
 
 
-def _batch1(lr, hr, cbcr, ang_in, ang_out, name):
-    return (lr[None], hr[None], cbcr[None], [torch.tensor([ang_in]), torch.tensor([ang_out])], [name])
+def _batch1(lr, hr, cbcr, ang_in, ang_out, name, grid=None):
+    """grid: the N of a full-grid scene (--full_grid 1), carried as a third data_info entry next to the window size"""
+    info = [torch.tensor([ang_in]), torch.tensor([ang_out])] + ([] if grid is None else [torch.tensor([grid])])
+    return (lr[None], hr[None], cbcr[None], info, [name])
 
 
 class SyntheticTestSet:
@@ -106,10 +108,11 @@ def _check_rgb8(im, fn):
             raise ValueError(f"{fn}: 16-bit samples are not supported (8-bit RGB views only)")
 
 
-def read_views(scene_dir, ang):
-    """the central ang x ang views of one scene folder of View_u_v.{png,bmp} images -> uint8 [ang, ang, H, W, 3].
-    Every view of the grid must be present, 8-bit RGB and of one size (headers only are read for the views outside
-    the centre); only the central views are decoded. Raises ValueError naming the file and the problem."""
+def read_views(scene_dir, ang, full_grid=False):
+    """the central ang x ang views of one scene folder of View_u_v.{png,bmp} images -> uint8 [ang, ang, H, W, 3]; with
+    full_grid, the central N x N views with N = min(U, V) of the U x V grid -> uint8 [N, N, H, W, 3] (angular window
+    tiling, include/lfsr.h). Every view of the grid must be present, 8-bit RGB and of one size (headers only are read for
+    the views outside the centre); only the central views are decoded. Raises ValueError naming the file and the problem."""
     from PIL import Image
     files = {}
     for f in sorted(os.listdir(scene_dir)):
@@ -139,10 +142,11 @@ def read_views(scene_dir, ang):
                 size, first = im.size, fn
             elif im.size != size:
                 raise ValueError(f"{fn}: view is {im.size[0]}x{im.size[1]} (WxH) but {first} is {size[0]}x{size[1]}")
-    u0, v0 = (U - ang) // 2, (V - ang) // 2
-    out = np.empty((ang, ang, size[1], size[0], 3), dtype=np.uint8)
-    for i in range(ang):
-        for j in range(ang):
+    n = min(U, V) if full_grid else ang
+    u0, v0 = (U - n) // 2, (V - n) // 2
+    out = np.empty((n, n, size[1], size[0], 3), dtype=np.uint8)
+    for i in range(n):
+        for j in range(n):
             with Image.open(files[(u0 + i, v0 + j)]) as im:
                 out[i, j] = np.asarray(im)
     return out
@@ -158,12 +162,14 @@ class ViewsTestSet:
     """one dataset directory <path_for_test>/<data_name>/ of scene folders of View_u_v.{png,bmp} images. kind="hr":
     the views are ground truth (test.py: LR input = their bicubic x1/s); kind="lr": the views are the LR input
     (inference.py; Hr_SAI_y is an empty tensor). Yields the batch-1 5-tuple with the tensors on the current CUDA device;
-    __getitem__ decodes only the scene asked for."""
+    __getitem__ decodes only the scene asked for. full_grid: every view of the central N x N (N = min(U, V)) instead of
+    the central A x A, for angular window tiling (scene.test_grid / super_resolve_grid); data_info is then
+    [A, A, N]."""
 
-    def __init__(self, args, data_name, kind):
+    def __init__(self, args, data_name, kind, full_grid=False):
         if kind not in ("hr", "lr"):
             raise ValueError(f"kind must be 'hr' or 'lr', got {kind!r}")
-        self.args, self.kind = args, kind
+        self.args, self.kind, self.full_grid = args, kind, bool(full_grid)
         self.root = os.path.join(args.path_for_test, data_name)
         self.scenes = _scene_dirs(self.root)
 
@@ -174,11 +180,17 @@ class ViewsTestSet:
         if not 0 <= i < len(self.scenes):
             raise IndexError(i)
         A, s = self.args.angRes_in, self.args.scale_factor
-        rgb8 = read_views(os.path.join(self.root, self.scenes[i]), A)
-        lr, hr, cbcr = prepare_views(rgb8, A, s, self.kind)
+        if self.full_grid:
+            rgb8 = read_views(os.path.join(self.root, self.scenes[i]), A, full_grid=True)
+            n = rgb8.shape[0]
+        else:
+            rgb8 = read_views(os.path.join(self.root, self.scenes[i]), A)
+            n = A
+        lr, hr, cbcr = prepare_views(rgb8, n, s, self.kind)
         if hr is None:
             hr = lr.new_empty((0, 0))
-        return _batch1(lr[None], hr[None], cbcr, A, self.args.angRes_out, self.scenes[i])
+        return _batch1(lr[None], hr[None], cbcr, A, self.args.angRes_out, self.scenes[i],
+                       n if self.full_grid else None)
 
     def __iter__(self):
         for i in range(len(self)):
@@ -189,12 +201,20 @@ def MultiTestSetDataLoader(args, views=None):
     """(dataset names, loaders, total scenes). --synthetic N wins; then BasicLFSR's h5 layout
     <path_for_test>/SR_AxA_sx/<data_name>/*.h5 if that directory exists (or `views` is None); otherwise light fields
     stored as view images, <path_for_test>/<data_name>/<scene>/View_u_v.{png,bmp}, read as `views` = "hr" (ground
-    truth, test.py) or "lr" (LR input, inference.py)."""
+    truth, test.py) or "lr" (LR input, inference.py). --full_grid 1 (every view, angular window tiling) needs the view
+    layout: synthetic scenes and h5 files hold only A x A views, so it raises ValueError with them."""
+    full_grid = bool(getattr(args, "full_grid", 0))
+    if full_grid and getattr(args, "synthetic", 0) > 0:
+        raise ValueError("--full_grid 1 needs light fields stored as view images: --synthetic scenes have only "
+                         f"{args.angRes_in}x{args.angRes_in} views")
     if getattr(args, "synthetic", 0) > 0:
         ds = SyntheticTestSet(args, args.synthetic, args.synthetic_size)
         return ["Synthetic"], [ds], len(ds)
     base = os.path.join(args.path_for_test, "SR_%dx%d_%dx" % (args.angRes_in, args.angRes_in, args.scale_factor))
     if views is None or os.path.isdir(base):
+        if full_grid:
+            raise ValueError(f"--full_grid 1 needs light fields stored as view images: the h5 test sets in {base} hold "
+                             f"only {args.angRes_in}x{args.angRes_in} views")
         names = sorted(os.listdir(base)) if args.data_name == "ALL" else [args.data_name]
         loaders = [H5TestSet(args, n) for n in names]
         return names, loaders, sum(len(d) for d in loaders)
@@ -203,7 +223,7 @@ def MultiTestSetDataLoader(args, views=None):
         names = [d for d in sorted(os.listdir(root)) if _scene_dirs(os.path.join(root, d))] if os.path.isdir(root) else []
     else:
         names = [args.data_name]
-    loaders = [ViewsTestSet(args, n, views) for n in names]
+    loaders = [ViewsTestSet(args, n, views, full_grid) for n in names]
     n_scenes = sum(len(d) for d in loaders)
     if n_scenes == 0:
         raise FileNotFoundError(
