@@ -155,6 +155,10 @@ int lfsr_interp(const float* in, float* out, int n, int h, int w, int scale, int
  * mat_inv255 = inv(M_BT601) * 255 (row-major 3x3) and offset = inv(M) @ [16,128,128] come from the host (host pointers). */
 int lfsr_ycbcr_to_rgb8(const float* y, const float* cb, const float* cr, unsigned char* rgb, int ang, int h, int w,
                        const double* mat_inv255, const double* offset, void* stream);
+/* the same for an ang_u x ang_v grid of views: mosaics [(ang_u h)][(ang_v w)] -> uint8 views [ang_u][ang_v][h][w][3].
+ * lfsr_ycbcr_to_rgb8 is this with ang_u = ang_v = ang. */
+int lfsr_ycbcr_to_rgb8_uv(const float* y, const float* cb, const float* cr, unsigned char* rgb, int ang_u, int ang_v, int h,
+                          int w, const double* mat_inv255, const double* offset, void* stream);
 
 /* ---- View preparation (input side; BasicLFSR's Generate_Data_for_Test.py / _for_inference.py as recorded in DESIGN.md
  * row f-7: the generator scripts are not in this tree, so parity with them is unpinned). Per scene of U x V RGB views
@@ -175,6 +179,10 @@ int lfsr_ycbcr_to_rgb8(const float* y, const float* cb, const float* cr, unsigne
  * to skip that output; at least one is written. Bit-exact to the numpy statement. */
 int lfsr_rgb_to_ycbcr_mosaic(const void* views, int is_u8, float* y, float* cb, float* cr, int ang, int h, int w,
                              void* stream);
+/* the same for an ang_u x ang_v grid: views [ang_u][ang_v][h][w][3] -> mosaics [(ang_u h)][(ang_v w)].
+ * lfsr_rgb_to_ycbcr_mosaic is this with ang_u = ang_v = ang. */
+int lfsr_rgb_to_ycbcr_mosaic_uv(const void* views, int is_u8, float* y, float* cb, float* cr, int ang_u, int ang_v, int h,
+                                int w, void* stream);
 
 /* One separable pass of the reference's MATLAB-style imresize (utils/imresize.py:57-102 `resizeAlongDim`), fp64:
  * out[a][i][b] = sum_p weights[i][p] * in[a][indices[i][p]][b] over a tensor viewed as [outer][in_len][inner]
@@ -184,16 +192,19 @@ int lfsr_resample_f64(const double* in, double* out, const double* weights, cons
 
 /* ---- Angular window tiling (no counterpart in the reference; DESIGN.md row f-8): every view of a light field larger than
  * the A x A a network was trained for (A = angRes), off by default (--full_grid 1).
- *   grid     N = min(U, V) of a U x V grid of views; the central N x N by the rule of "View preparation" (u0 = (U - N) // 2,
- *            v0 = (V - N) // 2); N >= A. Square only: the metric and colour kernels take one angular size.
- *   origins  along each angular axis, for a stride t with 1 <= t <= A - 1 when N > A (default t = A - 1, the fewest windows
- *            that cover the grid): 0, t, 2t, ... while < N - A, then N - A. N = A: the single origin 0. E.g. N = 9, A = 5:
- *            {0, 4}; N = 14, A = 5: {0, 4, 8, 9}.
- *   windows  the pairs (o_u, o_v) in row-major order of (o_u, o_v); that order is the summation order.
+ *   grid     N_u x N_v views of a U x V grid of views, the central ones by the rule of "View preparation"
+ *            (u0 = (U - N_u) // 2, v0 = (V - N_v) // 2); A <= N_u <= U and A <= N_v <= V. By default (--grid_views '')
+ *            N_u = N_v = N = min(U, V); --grid_views all takes the whole U x V, --grid_views RxC the central R x C.
+ *   origins  along each angular axis independently, window_origins(N_u, A, t) and window_origins(N_v, A, t), one stride t
+ *            for both, 1 <= t <= A - 1 when the axis is longer than A (default t = A - 1, the fewest windows that cover the
+ *            axis): 0, t, 2t, ... while < N - A, then N - A for an axis of N views. N = A: the single origin 0. E.g.
+ *            N = 9, A = 5: {0, 4}; N = 13, A = 5: {0, 4, 8}; N = 14, A = 5: {0, 4, 8, 9}.
+ *   windows  the pairs (o_u, o_v) in row-major order of (o_u, o_v); that order is the summation order. N_u = N_v gives
+ *            exactly the square plan.
  *   window   the LR Y mosaic of views [o_u, o_u + A) x [o_v, o_v + A) through the scene pipeline unchanged (LFdivide ->
  *            forward -> LFintegrate, with the x8 self-ensemble when it is on) -> an SR window mosaic [(A hs), (A ws)].
- *   merge    SR view (u, v) of the N x N mosaic = (((W_k1 + W_k2) + ...) + W_kc) / c over the windows k1 < k2 < ... that
- *            contain it, c their count: fp32 sums with __fadd_rn, one __fdiv_rn by (float)c; c = 1 is a plain copy. This is
+ *   merge    SR view (u, v) of the N_u x N_v mosaic = (((W_k1 + W_k2) + ...) + W_kc) / c over the windows k1 < k2 < ...
+ *            that contain it, c = c_u * c_v their count (c_u origins along u cover u, c_v along v cover v): fp32 sums with __fadd_rn, one __fdiv_rn by (float)c; c = 1 is a plain copy. This is
  *            what torch's fp32 `a + b` then `/ c` (c as a tensor: a Python scalar divisor may become a reciprocal multiply)
  *            computes, bit for bit.
  *
@@ -204,6 +215,11 @@ int lfsr_resample_f64(const double* in, double* out, const double* weights, cons
  * ang > 16, a window outside the grid, overlapping mosaics or a mode outside [0, min(ang, n - ang + 1)^2]. */
 int lfsr_window_accumulate(const float* win, float* grid, int ang, int n, int h, int w, int o_u, int o_v,
                            const int32_t* host_modes, void* stream);
+/* the same into an n_u x n_v mosaic `grid` [(n_u h)][(n_v w)]: n_u, n_v >= ang, 0 <= o_u <= n_u - ang,
+ * 0 <= o_v <= n_v - ang, modes in [0, min(ang, n_u - ang + 1) * min(ang, n_v - ang + 1)]. lfsr_window_accumulate is this
+ * with n_u = n_v = n. */
+int lfsr_window_accumulate_uv(const float* win, float* grid, int ang, int n_u, int n_v, int h, int w, int o_u, int o_v,
+                              const int32_t* host_modes, void* stream);
 
 /* ---- convolutions --------------------------------------------------------------------- */
 /* fp32 CUDA-core implicit GEMM; weights packed [kh*kw][cin][cout]. */
@@ -402,6 +418,11 @@ int lfsr_metric_sums(const float* label, const float* out, int ang, int h, int w
  * by the caller. */
 int lfsr_metric_sums_batched(const float* label, const float* out, int n, int ang, int h, int w, double* acc,
                              void* stream);
+/* the same for an ang_u x ang_v mosaic [(ang_u h)][(ang_v w)] (row stride ang_v * w): acc[a1 * ang_v + a2] = {sum sq. err,
+ * sum SSIM}, 2 * ang_u * ang_v doubles, zeroed by the caller. lfsr_metric_sums is this with ang_u = ang_v = ang, and
+ * lfsr_metric_sums_batched with ang_u = n * ang, ang_v = ang. */
+int lfsr_metric_sums_uv(const float* label, const float* out, int ang_u, int ang_v, int h, int w, double* acc,
+                        void* stream);
 
 #ifdef __cplusplus
 }

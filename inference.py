@@ -5,8 +5,8 @@ there (wrapped in try/except) and is not reproduced.
 
 Under torchrun (WORLD_SIZE > 1) each dataset is split across the ranks like test.py's (train.rank_scenes); every
 View_i_j.bmp is written once, by the rank that owns its scene, and only rank 0 prints. With --full_grid 1 every view of
-the central N x N of each light field is super-resolved with overlapping angRes x angRes windows
-(scene.super_resolve_grid) and N^2 View_i_j.bmp are written."""
+the central N x N of each light field (with --grid_views: the whole U x V grid, or its central R x C) is super-resolved
+with overlapping angRes x angRes windows (scene.super_resolve_grid) and N_u * N_v View_i_j.bmp are written."""
 import importlib
 
 import torch

@@ -92,9 +92,12 @@ SIGNATURES = {
     "lfsr_integrate_rows_d8": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
     "lfsr_interp": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "lfsr_ycbcr_to_rgb8": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
+    "lfsr_ycbcr_to_rgb8_uv": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P]),
     "lfsr_resample_f64": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "lfsr_rgb_to_ycbcr_mosaic": (_I, [_P, _I, _P, _P, _P, _I, _I, _I, _P]),
+    "lfsr_rgb_to_ycbcr_mosaic_uv": (_I, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _P]),
     "lfsr_window_accumulate": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _P, _P]),
+    "lfsr_window_accumulate_uv": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P]),
     "lfsr_conv2d_f32": (_I, [_TP, _P, _TP, C.POINTER(ConvDesc), _P]),
     "lfsr_dwconv_f32": (_I, [_TP, _P, _P, _P, _TP, _I, _I, _I, _I, _I, C.c_float, _P]),
     "lfsr_dwconv_multi": (_I, [_TP, _TP, C.POINTER(DwBranch), _I, _P]),
@@ -138,6 +141,7 @@ SIGNATURES = {
     "lfsr_epit_basictrans": (_I, [_TP, _P, _TP, C.POINTER(BasicTransDesc), _P]),
     "lfsr_metric_sums": (_I, [_P, _P, _I, _I, _I, _P, _P]),
     "lfsr_metric_sums_batched": (_I, [_P, _P, _I, _I, _I, _I, _P, _P]),
+    "lfsr_metric_sums_uv": (_I, [_P, _P, _I, _I, _I, _I, _P, _P]),
 }
 
 _lib = None

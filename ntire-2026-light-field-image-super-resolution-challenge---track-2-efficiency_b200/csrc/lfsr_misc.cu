@@ -538,7 +538,7 @@ constexpr int MT_W = 32, MT_H = 16, MT_R = 5;
 struct Gauss11 { float g[11]; };
 
 __global__ void __launch_bounds__(256)
-metric_kernel(const float* __restrict__ la, const float* __restrict__ ou, int A, int h, int w, double* acc,
+metric_kernel(const float* __restrict__ la, const float* __restrict__ ou, int Av, int h, int w, double* acc,
               int tiles_x, int tiles_y, const Gauss11 gw) {
   __shared__ float sa[MT_H + 2 * MT_R][MT_W + 2 * MT_R];
   __shared__ float sb[MT_H + 2 * MT_R][MT_W + 2 * MT_R];
@@ -548,8 +548,8 @@ metric_kernel(const float* __restrict__ la, const float* __restrict__ ou, int A,
   const int tx = blk % tiles_x; blk /= tiles_x;
   const int ty = blk % tiles_y;
   const int view = blk / tiles_y;
-  const int va = view / A, vb = view % A;
-  const size_t rs = (size_t)A * w;
+  const int va = view / Av, vb = view % Av;
+  const size_t rs = (size_t)Av * w;
   const float* pa = la + (size_t)va * h * rs + (size_t)vb * w;
   const float* pb = ou + (size_t)va * h * rs + (size_t)vb * w;
   // tile origin in view coordinates; tiles cover the full view, SSIM is only taken on the interior
@@ -979,14 +979,22 @@ extern "C" int lfsr_to_f16(const lfsr_tensor* in, const lfsr_tensor* out16, void
 
 extern "C" int lfsr_metric_sums(const float* label, const float* out, int ang, int h, int w, double* acc,
                                 void* stream) {
-  return lfsr_metric_sums_batched(label, out, 1, ang, h, w, acc, stream);
+  return lfsr_metric_sums_uv(label, out, ang, ang, h, w, acc, stream);
 }
 
 extern "C" int lfsr_metric_sums_batched(const float* label, const float* out, int n, int ang, int h, int w, double* acc,
                                         void* stream) {
-  LFSR_REQUIRE(label && out && acc, "lfsr_metric_sums: null pointer");
-  LFSR_REQUIRE(ang > 0 && h >= 11 && w >= 11, "lfsr_metric_sums: views must be at least 11x11 (skimage win_size)");
   LFSR_REQUIRE(n > 0, "lfsr_metric_sums: empty batch");
+  LFSR_REQUIRE((long long)n * ang < (1LL << 31), "lfsr_metric_sums: too many tiles");
+  // n mosaics stacked along y are one mosaic with n * ang view rows: view index = (img * ang + a1) * ang + a2
+  return lfsr_metric_sums_uv(label, out, n * ang, ang, h, w, acc, stream);
+}
+
+extern "C" int lfsr_metric_sums_uv(const float* label, const float* out, int ang_u, int ang_v, int h, int w, double* acc,
+                                   void* stream) {
+  LFSR_REQUIRE(label && out && acc, "lfsr_metric_sums: null pointer");
+  LFSR_REQUIRE(ang_u > 0 && ang_v > 0 && h >= 11 && w >= 11,
+               "lfsr_metric_sums: views must be at least 11x11 (skimage win_size)");
   // scipy.ndimage._gaussian_kernel1d(sigma=1.5, order=0, radius=5): float64 weights, cast to fp32
   Gauss11 gw;
   {
@@ -995,9 +1003,9 @@ extern "C" int lfsr_metric_sums_batched(const float* label, const float* out, in
     for (int i = 0; i < 11; ++i) gw.g[i] = (float)(g[i] / s);
   }
   const int tiles_x = ceil_div(w, MT_W), tiles_y = ceil_div(h, MT_H);
-  // n mosaics stacked along y are one mosaic with n * ang view rows: view index = (img * ang + a1) * ang + a2
-  const long long blocks = (long long)n * ang * ang * tiles_x * tiles_y;
+  // view index = a1 * ang_v + a2, the row-major order of the views in the [(ang_u h), (ang_v w)] mosaic
+  const long long blocks = (long long)ang_u * ang_v * tiles_x * tiles_y;
   LFSR_REQUIRE(blocks < 0x7fffffffLL, "lfsr_metric_sums: too many tiles");
-  metric_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(label, out, ang, h, w, acc, tiles_x, tiles_y, gw);
+  metric_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(label, out, ang_v, h, w, acc, tiles_x, tiles_y, gw);
   return check_launch("metric_kernel");
 }

@@ -387,14 +387,14 @@ namespace lfsr {
 struct ColourMat { double m[9]; double off[3]; };
 __global__ void __launch_bounds__(256)
 ycbcr_rgb8_kernel(const float* __restrict__ y, const float* __restrict__ cb, const float* __restrict__ cr,
-                  unsigned char* __restrict__ rgb, int ang, int h, int w, ColourMat cm) {
-  const int W = ang * w;
-  const long long total = (long long)ang * h * W;
+                  unsigned char* __restrict__ rgb, int ang_u, int ang_v, int h, int w, ColourMat cm) {
+  const int W = ang_v * w;
+  const long long total = (long long)ang_u * h * W;
   for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
     const int X = (int)(t % W), Y = (int)(t / W);
     const int u = Y / h, yy = Y - u * h, v = X / w, xx = X - v * w;
     const double a = (double)y[t], b = (double)cb[t], c = (double)cr[t];
-    unsigned char* dst = rgb + ((((long long)u * ang + v) * h + yy) * w + xx) * 3;
+    unsigned char* dst = rgb + ((((long long)u * ang_v + v) * h + yy) * w + xx) * 3;
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
       double r = __dadd_rn(__dadd_rn(__dmul_rn(cm.m[3 * k], a), __dmul_rn(cm.m[3 * k + 1], b)), __dmul_rn(cm.m[3 * k + 2], c));
@@ -408,15 +408,20 @@ ycbcr_rgb8_kernel(const float* __restrict__ y, const float* __restrict__ cb, con
 
 extern "C" int lfsr_ycbcr_to_rgb8(const float* y, const float* cb, const float* cr, unsigned char* rgb, int ang, int h, int w,
                                   const double* mat_inv255, const double* offset, void* stream) {
+  return lfsr_ycbcr_to_rgb8_uv(y, cb, cr, rgb, ang, ang, h, w, mat_inv255, offset, stream);
+}
+
+extern "C" int lfsr_ycbcr_to_rgb8_uv(const float* y, const float* cb, const float* cr, unsigned char* rgb, int ang_u,
+                                     int ang_v, int h, int w, const double* mat_inv255, const double* offset, void* stream) {
   LFSR_REQUIRE(y && cb && cr && rgb && mat_inv255 && offset, "lfsr_ycbcr_to_rgb8: null pointer");
-  LFSR_REQUIRE(ang > 0 && h > 0 && w > 0, "lfsr_ycbcr_to_rgb8: bad geometry");
+  LFSR_REQUIRE(ang_u > 0 && ang_v > 0 && h > 0 && w > 0, "lfsr_ycbcr_to_rgb8: bad geometry");
   lfsr::ColourMat cm;
   for (int i = 0; i < 9; ++i) cm.m[i] = mat_inv255[i];
   for (int i = 0; i < 3; ++i) cm.off[i] = offset[i];
-  const long long total = (long long)ang * h * ang * w;
+  const long long total = (long long)ang_u * h * ang_v * w;
   long long blocks = (total + 255) / 256;
   if (blocks > 148LL * 32) blocks = 148LL * 32;
-  lfsr::ycbcr_rgb8_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(y, cb, cr, rgb, ang, h, w, cm);
+  lfsr::ycbcr_rgb8_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(y, cb, cr, rgb, ang_u, ang_v, h, w, cm);
   return lfsr::check_launch("ycbcr_rgb8_kernel");
 }
 
@@ -438,13 +443,13 @@ __device__ __forceinline__ float ycbcr_term(double r, double g, double b, double
 template <class T>
 __global__ void __launch_bounds__(256)
 rgb_ycbcr_mosaic_kernel(const T* __restrict__ views, float* __restrict__ y, float* __restrict__ cb, float* __restrict__ cr,
-                        int ang, int h, int w) {
-  const int W = ang * w;
-  const long long total = (long long)ang * h * W;
+                        int ang_u, int ang_v, int h, int w) {
+  const int W = ang_v * w;
+  const long long total = (long long)ang_u * h * W;
   for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
     const int X = (int)(t % W), Y = (int)(t / W);
     const int u = Y / h, yy = Y - u * h, v = X / w, xx = X - v * w;
-    const T* src = views + ((((long long)u * ang + v) * h + yy) * w + xx) * 3;
+    const T* src = views + ((((long long)u * ang_v + v) * h + yy) * w + xx) * 3;
     const double r = view_value(src), g = view_value(src + 1), b = view_value(src + 2);
     if (y) y[t] = ycbcr_term(r, g, b, 65.481, 128.553, 24.966, 16.0);
     if (cb) {
@@ -457,28 +462,34 @@ rgb_ycbcr_mosaic_kernel(const T* __restrict__ views, float* __restrict__ y, floa
 
 extern "C" int lfsr_rgb_to_ycbcr_mosaic(const void* views, int is_u8, float* y, float* cb, float* cr, int ang, int h, int w,
                                         void* stream) {
+  return lfsr_rgb_to_ycbcr_mosaic_uv(views, is_u8, y, cb, cr, ang, ang, h, w, stream);
+}
+
+extern "C" int lfsr_rgb_to_ycbcr_mosaic_uv(const void* views, int is_u8, float* y, float* cb, float* cr, int ang_u,
+                                           int ang_v, int h, int w, void* stream) {
   LFSR_REQUIRE(views, "lfsr_rgb_to_ycbcr_mosaic: null views");
   LFSR_REQUIRE(y || cb, "lfsr_rgb_to_ycbcr_mosaic: no output (need Y, CbCr or both)");
   LFSR_REQUIRE((cb == nullptr) == (cr == nullptr), "lfsr_rgb_to_ycbcr_mosaic: cb and cr go together");
-  LFSR_REQUIRE(ang > 0 && h > 0 && w > 0, "lfsr_rgb_to_ycbcr_mosaic: bad geometry ang=%d h=%d w=%d", ang, h, w);
-  LFSR_REQUIRE((long long)ang * h < (1LL << 31) && (long long)ang * w < (1LL << 31),
-               "lfsr_rgb_to_ycbcr_mosaic: mosaic %lldx%lld too large", (long long)ang * h, (long long)ang * w);
-  const long long total = (long long)ang * h * ang * w;
+  LFSR_REQUIRE(ang_u > 0 && ang_v > 0 && h > 0 && w > 0, "lfsr_rgb_to_ycbcr_mosaic: bad geometry ang=%dx%d h=%d w=%d",
+               ang_u, ang_v, h, w);
+  LFSR_REQUIRE((long long)ang_u * h < (1LL << 31) && (long long)ang_v * w < (1LL << 31),
+               "lfsr_rgb_to_ycbcr_mosaic: mosaic %lldx%lld too large", (long long)ang_u * h, (long long)ang_v * w);
+  const long long total = (long long)ang_u * h * ang_v * w;
   long long blocks = (total + 255) / 256;
   if (blocks > 148LL * 32) blocks = 148LL * 32;
   if (is_u8) {
     lfsr::rgb_ycbcr_mosaic_kernel<unsigned char><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(
-        (const unsigned char*)views, y, cb, cr, ang, h, w);
+        (const unsigned char*)views, y, cb, cr, ang_u, ang_v, h, w);
   } else {
     lfsr::rgb_ycbcr_mosaic_kernel<double><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>((const double*)views, y, cb, cr,
-                                                                                          ang, h, w);
+                                                                                          ang_u, ang_v, h, w);
   }
   return lfsr::check_launch("rgb_ycbcr_mosaic_kernel");
 }
 
 
 // ---- angular window tiling (include/lfsr.h, "Angular window tiling"): one SR window mosaic [(A h), (A w)] merged into the
-// N x N SR mosaic [(N h), (N w)] at view offset (o_u, o_v). Per view of the window a mode: 0 = store, 1 = add, c >= 2 = add,
+// N_u x N_v SR mosaic [(N_u h), (N_v w)] at view offset (o_u, o_v). Per view of the window a mode: 0 = store, 1 = add, c >= 2 = add,
 // then divide by c (the last window over that view). Sums with __fadd_rn, the mean with one __fdiv_rn: fp32 `a + b` and
 // `a / c` in torch give the same bits. One thread = VEC consecutive x of one view row, in window-mosaic order, so the window
 // reads are dense; a window row lands as one contiguous run of the grid row (views o_v .. o_v + A - 1 are adjacent there).
@@ -493,13 +504,13 @@ __device__ __forceinline__ float win_merge(float acc, float v, int mode) {
 
 template <int VEC>
 __global__ void __launch_bounds__(256)
-window_accumulate_kernel(const float* __restrict__ win, float* __restrict__ grid, int A, int N, int h, int w, int o_u,
+window_accumulate_kernel(const float* __restrict__ win, float* __restrict__ grid, int A, int Nv, int h, int w, int o_u,
                          int o_v, WinModes md) {
   const int wv = w / VEC;
   for (int Y = blockIdx.y; Y < A * h; Y += gridDim.y) {
     const int a1 = Y / h, y = Y - a1 * h;
     const float* src = win + (size_t)Y * A * w;
-    float* dst = grid + ((size_t)(o_u + a1) * h + y) * ((size_t)N * w) + (size_t)o_v * w;
+    float* dst = grid + ((size_t)(o_u + a1) * h + y) * ((size_t)Nv * w) + (size_t)o_v * w;
     for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < A * wv; t += gridDim.x * blockDim.x) {
       const int a2 = t / wv;
       const int X = a2 * w + (t - a2 * wv) * VEC;
@@ -524,24 +535,30 @@ window_accumulate_kernel(const float* __restrict__ win, float* __restrict__ grid
 
 extern "C" int lfsr_window_accumulate(const float* win, float* grid, int ang, int n, int h, int w, int o_u, int o_v,
                                       const int32_t* host_modes, void* stream) {
+  return lfsr_window_accumulate_uv(win, grid, ang, n, n, h, w, o_u, o_v, host_modes, stream);
+}
+
+extern "C" int lfsr_window_accumulate_uv(const float* win, float* grid, int ang, int n_u, int n_v, int h, int w, int o_u,
+                                         int o_v, const int32_t* host_modes, void* stream) {
   using lfsr::WIN_MAX_ANG;
   LFSR_REQUIRE(win && grid && host_modes, "lfsr_window_accumulate: null pointer");
   LFSR_REQUIRE(ang > 0 && ang <= WIN_MAX_ANG && h > 0 && w > 0, "lfsr_window_accumulate: bad geometry A=%d h=%d w=%d "
                "(1 <= A <= %d)", ang, h, w, WIN_MAX_ANG);
-  LFSR_REQUIRE(n >= ang, "lfsr_window_accumulate: a %dx%d grid is smaller than the %dx%d window", n, n, ang, ang);
-  LFSR_REQUIRE((long long)n * h < (1LL << 31) && (long long)n * w < (1LL << 31),
-               "lfsr_window_accumulate: mosaic %lldx%lld too large", (long long)n * h, (long long)n * w);
-  LFSR_REQUIRE(0 <= o_u && o_u <= n - ang && 0 <= o_v && o_v <= n - ang,
-               "lfsr_window_accumulate: window at (%d, %d) lies outside the %dx%d grid (A=%d)", o_u, o_v, n, n, ang);
-  const long long win_n = (long long)ang * h * ang * w, grid_n = (long long)n * h * n * w;
+  LFSR_REQUIRE(n_u >= ang && n_v >= ang, "lfsr_window_accumulate: a %dx%d grid is smaller than the %dx%d window", n_u, n_v,
+               ang, ang);
+  LFSR_REQUIRE((long long)n_u * h < (1LL << 31) && (long long)n_v * w < (1LL << 31),
+               "lfsr_window_accumulate: mosaic %lldx%lld too large", (long long)n_u * h, (long long)n_v * w);
+  LFSR_REQUIRE(0 <= o_u && o_u <= n_u - ang && 0 <= o_v && o_v <= n_v - ang,
+               "lfsr_window_accumulate: window at (%d, %d) lies outside the %dx%d grid (A=%d)", o_u, o_v, n_u, n_v, ang);
+  const long long win_n = (long long)ang * h * ang * w, grid_n = (long long)n_u * h * n_v * w;
   LFSR_REQUIRE(win + win_n <= grid || grid + grid_n <= win, "lfsr_window_accumulate: window and grid mosaics overlap");
   // a view lies in at most A windows per angular axis (distinct origins in (u - A, u]) and in at most N - A + 1
-  const int per_axis = ang < n - ang + 1 ? ang : n - ang + 1;
+  const int per_u = ang < n_u - ang + 1 ? ang : n_u - ang + 1, per_v = ang < n_v - ang + 1 ? ang : n_v - ang + 1;
   lfsr::WinModes md;
   for (int i = 0; i < ang * ang; ++i) {
-    LFSR_REQUIRE(host_modes[i] >= 0 && host_modes[i] <= per_axis * per_axis,
+    LFSR_REQUIRE(host_modes[i] >= 0 && host_modes[i] <= per_u * per_v,
                  "lfsr_window_accumulate: bad mode %d for view %d (0 store, 1 add, 2..%d add then divide)", host_modes[i],
-                 i, per_axis * per_axis);
+                 i, per_u * per_v);
     md.m[i] = host_modes[i];
   }
   const int rows = ang * h;
@@ -549,8 +566,8 @@ extern "C" int lfsr_window_accumulate(const float* win, float* grid, int ang, in
   const int per_row = vec ? ang * (w / 4) : ang * w;
   dim3 g(ceil_div(per_row, 256), rows < 32768 ? rows : 32768);
   if (vec)
-    lfsr::window_accumulate_kernel<4><<<g, 256, 0, (cudaStream_t)stream>>>(win, grid, ang, n, h, w, o_u, o_v, md);
+    lfsr::window_accumulate_kernel<4><<<g, 256, 0, (cudaStream_t)stream>>>(win, grid, ang, n_v, h, w, o_u, o_v, md);
   else
-    lfsr::window_accumulate_kernel<1><<<g, 256, 0, (cudaStream_t)stream>>>(win, grid, ang, n, h, w, o_u, o_v, md);
+    lfsr::window_accumulate_kernel<1><<<g, 256, 0, (cudaStream_t)stream>>>(win, grid, ang, n_v, h, w, o_u, o_v, md);
   return lfsr::check_launch("window_accumulate_kernel");
 }

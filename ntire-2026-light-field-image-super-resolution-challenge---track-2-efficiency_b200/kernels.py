@@ -175,13 +175,17 @@ class CudaOps:
         """merge the SR window mosaic win [(ang h), (ang w)] into the N x N mosaic grid [(n h), (n w)] at view offset
         (o_u, o_v); modes: ang * ang ints, per window view 0 = store, 1 = add, c >= 2 = add then divide by c
         (include/lfsr.h, "Angular window tiling")"""
+        self.window_accumulate_uv(win, grid, ang, n, n, h, w, o_u, o_v, modes)
+
+    def window_accumulate_uv(self, win, grid, ang, n_u, n_v, h, w, o_u, o_v, modes):
+        """window_accumulate into an n_u x n_v mosaic grid [(n_u h), (n_v w)]"""
         if not (win.is_contiguous() and grid.is_contiguous() and win.dtype == grid.dtype == torch.float32):
             raise N.LfsrError("window_accumulate: dense fp32 mosaics required")
         if len(modes) != ang * ang:
             raise N.LfsrError(f"window_accumulate: {len(modes)} modes for {ang * ang} window views")
         m = (C.c_int32 * (ang * ang))(*[int(x) for x in modes])
-        N.check(self.lib.lfsr_window_accumulate(win.data_ptr(), grid.data_ptr(), ang, n, h, w, o_u, o_v, m,
-                                                self._stream(grid)), "lfsr_window_accumulate")
+        N.check(self.lib.lfsr_window_accumulate_uv(win.data_ptr(), grid.data_ptr(), ang, n_u, n_v, h, w, o_u, o_v, m,
+                                                   self._stream(grid)), "lfsr_window_accumulate_uv")
 
     def interp(self, x, out, n, h, w, scale, mode, block_h, block_w):
         N.check(self.lib.lfsr_interp(x.data_ptr(), out.data_ptr(), n, h, w, scale, mode, block_h, block_w,
@@ -490,6 +494,11 @@ class CudaOps:
     def metric_sums(self, label, out, ang, h, w, acc):
         N.check(self.lib.lfsr_metric_sums(label.data_ptr(), out.data_ptr(), ang, h, w, acc.data_ptr(),
                                           self._stream(label)), "lfsr_metric_sums")
+
+    def metric_sums_uv(self, label, out, ang_u, ang_v, h, w, acc):
+        """metric_sums over an ang_u x ang_v mosaic [(ang_u h), (ang_v w)]: 2 * ang_u * ang_v sums"""
+        N.check(self.lib.lfsr_metric_sums_uv(label.data_ptr(), out.data_ptr(), ang_u, ang_v, h, w, acc.data_ptr(),
+                                             self._stream(label)), "lfsr_metric_sums_uv")
 
     def metric_sums_batched(self, label, out, n, ang, h, w, acc):
         """label/out [n,1,A*h,A*w] contiguous; acc [n*A*A*2] float64, zeroed by the caller"""

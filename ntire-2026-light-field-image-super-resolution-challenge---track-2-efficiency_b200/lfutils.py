@@ -250,9 +250,19 @@ def imresize_views(views: torch.Tensor, scalar_scale: float, method: str = "bicu
 _BT601 = np.array([[65.481, 128.553, 24.966], [-37.797, -74.203, 112.0], [112.0, -93.786, -18.214]])
 
 
-def sai_to_rgb8_views(sr_y: torch.Tensor, sr_cbcr: torch.Tensor, angRes: int) -> torch.Tensor:
+def ang_pair(angRes):
+    """(a1, a2) of an angular size given as an int (a square grid) or as a (U, V) pair"""
+    if isinstance(angRes, (tuple, list)):
+        if len(angRes) != 2:
+            raise ValueError(f"an angular size is an int or a (U, V) pair, got {angRes!r}")
+        return int(angRes[0]), int(angRes[1])
+    return int(angRes), int(angRes)
+
+
+def sai_to_rgb8_views(sr_y: torch.Tensor, sr_cbcr: torch.Tensor, angRes) -> torch.Tensor:
     """Sr_SAI_y [.., (a1 h), (a2 w)] + Sr_SAI_cbcr [.., 2, (a1 h), (a2 w)] -> uint8 [a1, a2, h, w, 3] on the device:
-    torch.cat + ycbcr2rgb (fp64) + clip(0,1)*255 + astype(uint8) + the view rearrange of train.py:332-335 in one kernel."""
+    torch.cat + ycbcr2rgb (fp64) + clip(0,1)*255 + astype(uint8) + the view rearrange of train.py:332-335 in one kernel.
+    angRes: a1 = a2 as an int, or the pair (a1, a2) of a rectangular grid."""
     y = sr_y.reshape(sr_y.shape[-2:])
     cbcr = sr_cbcr.reshape(2, *sr_cbcr.shape[-2:])
     if cbcr.shape[-2:] != y.shape:
@@ -261,60 +271,72 @@ def sai_to_rgb8_views(sr_y: torch.Tensor, sr_cbcr: torch.Tensor, angRes: int) ->
     if dev.type != "cuda":
         raise N.LfsrError("lfsr_b200 needs a CUDA device (sm_100a); there is no CPU fallback for this path")
     H, W = y.shape
-    if H % angRes or W % angRes:
+    au, av = ang_pair(angRes)
+    if H % au or W % av:
         raise ValueError(f"mosaic {H}x{W} is not divisible by angRes={angRes}")
     y = y.to(dev, torch.float32).contiguous()
     cbcr = cbcr.to(dev, torch.float32).contiguous()
     inv = np.linalg.inv(_BT601)                                   # exactly the reference's constants (utils/utils.py:192-198)
     offset = np.ascontiguousarray(np.matmul(inv, np.array([16, 128, 128])))
     inv255 = np.ascontiguousarray(inv * 255)
-    out = torch.empty((angRes, angRes, H // angRes, W // angRes, 3), dtype=torch.uint8, device=dev)
-    N.check(N.load().lfsr_ycbcr_to_rgb8(y.data_ptr(), cbcr[0].data_ptr(), cbcr[1].data_ptr(), out.data_ptr(), angRes, H // angRes,
-                                        W // angRes, inv255.ctypes.data, offset.ctypes.data,
-                                        torch.cuda.current_stream(dev).cuda_stream), "lfsr_ycbcr_to_rgb8")
+    out = torch.empty((au, av, H // au, W // av, 3), dtype=torch.uint8, device=dev)
+    lib, stream = N.load(), torch.cuda.current_stream(dev).cuda_stream
+    if not isinstance(angRes, (tuple, list)):
+        N.check(lib.lfsr_ycbcr_to_rgb8(y.data_ptr(), cbcr[0].data_ptr(), cbcr[1].data_ptr(), out.data_ptr(), angRes,
+                                       H // angRes, W // angRes, inv255.ctypes.data, offset.ctypes.data, stream),
+                "lfsr_ycbcr_to_rgb8")
+    else:
+        N.check(lib.lfsr_ycbcr_to_rgb8_uv(y.data_ptr(), cbcr[0].data_ptr(), cbcr[1].data_ptr(), out.data_ptr(), au, av,
+                                          H // au, W // av, inv255.ctypes.data, offset.ctypes.data, stream),
+                "lfsr_ycbcr_to_rgb8_uv")
     return out
 
 
 # ---- input side: RGB views -> the Lr_SAI_y / Hr_SAI_y / Sr_SAI_cbcr tensors of a test set (include/lfsr.h) ------------------
-def rgb_to_ycbcr_mosaic(views: torch.Tensor, angRes: int, y: bool = True, cbcr: bool = True):
+def rgb_to_ycbcr_mosaic(views: torch.Tensor, angRes, y: bool = True, cbcr: bool = True):
     """views [a1, a2, h, w, 3] (or [a1*a2, h, w, 3]) on the device, uint8 or fp64 in [0, 1] -> (Y mosaic [(a1 h), (a2 w)],
     CbCr mosaics [2, (a1 h), (a2 w)]) in fp32, BasicLFSR's term-by-term rgb2ycbcr in one kernel; an output that is not
-    asked for is None."""
+    asked for is None. angRes: a1 = a2 as an int, or the pair (a1, a2)."""
     if not views.is_cuda:
         raise N.LfsrError("lfsr_b200 needs a CUDA device (sm_100a); there is no CPU fallback for this path")
     if views.dtype not in (torch.uint8, torch.float64):
         raise ValueError(f"views must be uint8 or float64, got {views.dtype}")
     h, w, c = views.shape[-3:]
-    if c != 3 or views.numel() != angRes * angRes * h * w * 3:
-        raise ValueError(f"expected {angRes}x{angRes} RGB views, got {tuple(views.shape)}")
+    au, av = ang_pair(angRes)
+    if c != 3 or views.numel() != au * av * h * w * 3:
+        raise ValueError(f"expected {au}x{av} RGB views, got {tuple(views.shape)}")
     if not (y or cbcr):
         raise ValueError("rgb_to_ycbcr_mosaic: ask for Y, CbCr or both")
     src = views.contiguous()
     dev = src.device
-    oy = torch.empty((angRes * h, angRes * w), dtype=torch.float32, device=dev) if y else None
-    oc = torch.empty((2, angRes * h, angRes * w), dtype=torch.float32, device=dev) if cbcr else None
+    oy = torch.empty((au * h, av * w), dtype=torch.float32, device=dev) if y else None
+    oc = torch.empty((2, au * h, av * w), dtype=torch.float32, device=dev) if cbcr else None
     ptr = lambda t: None if t is None else t.data_ptr()
-    N.check(N.load().lfsr_rgb_to_ycbcr_mosaic(src.data_ptr(), int(src.dtype == torch.uint8), ptr(oy),
-                                              None if oc is None else oc[0].data_ptr(), None if oc is None else oc[1].data_ptr(),
-                                              angRes, h, w, torch.cuda.current_stream(dev).cuda_stream),
-            "lfsr_rgb_to_ycbcr_mosaic")
+    outs = (src.data_ptr(), int(src.dtype == torch.uint8), ptr(oy), None if oc is None else oc[0].data_ptr(),
+            None if oc is None else oc[1].data_ptr())
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    if not isinstance(angRes, (tuple, list)):
+        N.check(N.load().lfsr_rgb_to_ycbcr_mosaic(*outs, angRes, h, w, stream), "lfsr_rgb_to_ycbcr_mosaic")
+    else:
+        N.check(N.load().lfsr_rgb_to_ycbcr_mosaic_uv(*outs, au, av, h, w, stream), "lfsr_rgb_to_ycbcr_mosaic_uv")
     return oy, oc
 
 
-def central_views(rgb8: np.ndarray, angRes: int, scale: int) -> np.ndarray:
-    """the views the preparation uses, as a host view (no copy): the central angRes x angRes of a [U, V, H, W, 3] grid,
-    each cropped top-left to a multiple of `scale` in height and width."""
+def central_views(rgb8: np.ndarray, angRes, scale: int) -> np.ndarray:
+    """the views the preparation uses, as a host view (no copy): the central angRes x angRes of a [U, V, H, W, 3] grid
+    (or the central a1 x a2 for angRes = (a1, a2)), each cropped top-left to a multiple of `scale` in height and width."""
     a = np.asarray(rgb8)
     if a.ndim != 5 or a.shape[-1] != 3:
         raise ValueError(f"expected RGB views [U, V, H, W, 3], got {a.shape}")
     U, V, H, W, _ = a.shape
-    if U < angRes or V < angRes:
-        raise ValueError(f"a {U}x{V} grid of views has no central {angRes}x{angRes}")
+    au, av = ang_pair(angRes)
+    if U < au or V < av:
+        raise ValueError(f"a {U}x{V} grid of views has no central {au}x{av}")
     hc, wc = H - H % scale, W - W % scale
     if hc == 0 or wc == 0:
         raise ValueError(f"views of {H}x{W} are smaller than the scale factor {scale}")
-    u0, v0 = (U - angRes) // 2, (V - angRes) // 2
-    return a[u0:u0 + angRes, v0:v0 + angRes, :hc, :wc]
+    u0, v0 = (U - au) // 2, (V - av) // 2
+    return a[u0:u0 + au, v0:v0 + av, :hc, :wc]
 
 
 _U8_TO_UNIT = {}
@@ -329,9 +351,10 @@ def _unit(x8: torch.Tensor) -> torch.Tensor:
     return lut.index_select(0, x8.reshape(-1).to(torch.int32)).view(x8.shape)
 
 
-def prepare_views(rgb8, angRes: int, scale: int, kind: str = "hr"):
+def prepare_views(rgb8, angRes, scale: int, kind: str = "hr"):
     """RGB views of one scene -> (Lr_SAI_y, Hr_SAI_y or None, Sr_SAI_cbcr) as fp32 mosaics on the current CUDA device,
-    by the recipe of include/lfsr.h. rgb8: host uint8 [U, V, H, W, 3]. kind="hr": the views are ground truth (test.py),
+    by the recipe of include/lfsr.h. rgb8: host uint8 [U, V, H, W, 3]; angRes: the central angRes x angRes views, or the
+    central a1 x a2 for a pair (a1, a2). kind="hr": the views are ground truth (test.py),
     the LR input is their bicubic x1/scale; kind="lr": the views are the LR input (inference.py) and there is no HR.
     The cropped central views cross PCIe once (3 bytes per pixel, from pinned memory); the rest runs on the device."""
     if kind not in ("hr", "lr"):

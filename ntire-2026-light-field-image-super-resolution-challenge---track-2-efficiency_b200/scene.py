@@ -270,10 +270,10 @@ class SceneRunner:
         return self.slots[k % self.depth]
 
 
-def metrics_from_sums(acc, ang: int, hs: int, ws: int):
-    """(psnr, ssim) from the per-view sums of lfsr_metric_sums over an ang x ang mosaic of hs x ws views: means over views
-    with value > 0, as utils/utils.py:121-134."""
-    a = np.asarray(acc, dtype=np.float64).reshape(ang, ang, 2)
+def metrics_from_sums(acc, ang, hs: int, ws: int):
+    """(psnr, ssim) from the per-view sums of lfsr_metric_sums over an ang x ang mosaic of hs x ws views (an
+    ang_u x ang_v one for ang = (ang_u, ang_v)): means over views with value > 0, as utils/utils.py:121-134."""
+    a = np.asarray(acc, dtype=np.float64).reshape(*U.ang_pair(ang), 2)
     mse = a[..., 0] / float(hs * ws)
     with np.errstate(divide="ignore"):
         P = (10.0 * np.log10(1.0 / mse)).astype(np.float32)
@@ -401,20 +401,23 @@ def window_origins(n: int, ang: int, stride: Optional[int] = None):
     return list(range(0, n - ang, t)) + [n - ang]
 
 
-def window_plan(n: int, ang: int, stride: Optional[int] = None):
-    """[(o_u, o_v, modes)] in window order (row-major in (o_u, o_v)); modes[a1 * ang + a2] is the lfsr_window_accumulate step
-    for window view (a1, a2): 0 = store (first window over the view), 1 = add, c >= 2 = add then divide by the view's
-    window count c (last window over it)."""
-    orig = window_origins(n, ang, stride)
-    cover = [[i for i, o in enumerate(orig) if o <= x < o + ang] for x in range(n)]
+def window_plan(n, ang: int, stride: Optional[int] = None):
+    """[(o_u, o_v, modes)] in window order (row-major in (o_u, o_v)) for an N x N grid, or an N_u x N_v one for
+    n = (N_u, N_v) (origins per axis, one stride); modes[a1 * ang + a2] is the lfsr_window_accumulate step for window view
+    (a1, a2): 0 = store (first window over the view), 1 = add, c >= 2 = add then divide by the view's window count
+    c = c_u * c_v (last window over it)."""
+    n_u, n_v = U.ang_pair(n)
+    orig_u, orig_v = window_origins(n_u, ang, stride), window_origins(n_v, ang, stride)
+    cover_u = [[i for i, o in enumerate(orig_u) if o <= x < o + ang] for x in range(n_u)]
+    cover_v = [[j for j, o in enumerate(orig_v) if o <= x < o + ang] for x in range(n_v)]
     plan = []
-    for i, ou in enumerate(orig):
-        for j, ov in enumerate(orig):
+    for i, ou in enumerate(orig_u):
+        for j, ov in enumerate(orig_v):
             modes = []
             for a1 in range(ang):
-                cu = cover[ou + a1]
+                cu = cover_u[ou + a1]
                 for a2 in range(ang):
-                    cv = cover[ov + a2]
+                    cv = cover_v[ov + a2]
                     if (i, j) == (cu[0], cv[0]):
                         modes.append(0)
                     elif (i, j) == (cu[-1], cv[-1]):
@@ -426,14 +429,15 @@ def window_plan(n: int, ang: int, stride: Optional[int] = None):
 
 
 def _grid_run(net, lr_sai, n, ang, scale, patch, stride, minibatch, group, ops, ang_stride, self_ensemble, world, rank):
-    """(runner, N x N SR mosaic): every window through the scene pipeline of one runner, merged as it completes."""
+    """(runner, N_u x N_v SR mosaic): every window through the scene pipeline of one runner, merged as it completes."""
     lr = lr_sai.reshape(lr_sai.shape[-2:])
-    n, ang = int(n), int(ang)
+    n_u, n_v = U.ang_pair(n)
+    ang = int(ang)
     H, W = lr.shape
-    if H % n or W % n:
-        raise ValueError(f"super_resolve_grid: LR mosaic {H}x{W} is not a {n}x{n} grid of views")
-    h0, w0 = H // n, W // n
-    plan = window_plan(n, ang, ang_stride)
+    if H % n_u or W % n_v:
+        raise ValueError(f"super_resolve_grid: LR mosaic {H}x{W} is not a {n_u}x{n_v} grid of views")
+    h0, w0 = H // n_u, W // n_v
+    plan = window_plan((n_u, n_v), ang, ang_stride)
     dev = lr.device
     if not lr.is_cuda:
         try:
@@ -448,43 +452,51 @@ def _grid_run(net, lr_sai, n, ang, scale, patch, stride, minibatch, group, ops, 
     if s["busy"]:
         raise RuntimeError("super_resolve_grid: the runner's next slot is in flight - call result() first")
     r._n += 1
-    out = torch.empty((n * r.hs, n * r.ws), dtype=torch.float32, device=dev)
+    out = torch.empty((n_u * r.hs, n_v * r.ws), dtype=torch.float32, device=dev)
     ctx = torch.cuda.device(dev) if dev.type == "cuda" else _NullCtx()
     with ctx:
-        views = lr.to(device=dev, dtype=torch.float32).contiguous().view(n, h0, n, w0)
+        views = lr.to(device=dev, dtype=torch.float32).contiguous().view(n_u, h0, n_v, w0)
         win_lr = s["lr"].view(ang, h0, ang, w0)
         for ou, ov, modes in plan:
             win_lr.copy_(views[ou:ou + ang, :, ov:ov + ang, :])
             r.run_resident(s["lr"], s["mosaic"])
-            r.ops.window_accumulate(s["mosaic"], out, ang, n, r.hs, r.ws, ou, ov, modes)
+            if n_u == n_v:                    # square grids keep the square entry points (and backends with only those)
+                r.ops.window_accumulate(s["mosaic"], out, ang, n_u, r.hs, r.ws, ou, ov, modes)
+            else:
+                r.ops.window_accumulate_uv(s["mosaic"], out, ang, n_u, n_v, r.hs, r.ws, ou, ov, modes)
     return r, out
 
 
-def super_resolve_grid(net, lr_sai: torch.Tensor, n: int, ang: int, scale: int, patch: int = 32, stride: int = 16,
+def super_resolve_grid(net, lr_sai: torch.Tensor, n, ang: int, scale: int, patch: int = 32, stride: int = 16,
                        minibatch: int = 64, group=None, ops=None, ang_stride: Optional[int] = None,
                        self_ensemble: bool = False, world: Optional[int] = None, rank: Optional[int] = None) -> torch.Tensor:
     """Every view of an N x N light field with a network for A x A inputs (A = ang): lr_sai [(N h0), (N w0)] -> the device
-    SR mosaic [(N h0 s), (N w0 s)] owned by the caller. The A x A windows of window_plan(N, A, ang_stride) each run exactly
+    SR mosaic [(N h0 s), (N w0 s)] owned by the caller; n = (N_u, N_v) for an N_u x N_v light field
+    [(N_u h0), (N_v w0)]. The A x A windows of window_plan(n, A, ang_stride) each run exactly
     what super_resolve_scene runs (row-sharded and all-gathered like a scene under a process group, so the result is the
     same on every rank); lfsr_window_accumulate averages the views several windows produce. N = A is super_resolve_scene."""
     return _grid_run(net, lr_sai, n, ang, scale, patch, stride, minibatch, group, ops, ang_stride, self_ensemble, world,
                      rank)[1]
 
 
-def test_grid(net, lr_sai, hr_sai, n: int, ang: int, scale: int, patch: int = 32, stride: int = 16, minibatch: int = 64,
+def test_grid(net, lr_sai, hr_sai, n, ang: int, scale: int, patch: int = 32, stride: int = 16, minibatch: int = 64,
               ops=None, ang_stride: Optional[int] = None, self_ensemble: bool = False, world: Optional[int] = None,
               rank: Optional[int] = None):
-    """(psnr, ssim, sr_mosaic) of super_resolve_grid against the N x N HR mosaic: means over all N^2 views with value > 0,
-    as test_scene's over A^2."""
+    """(psnr, ssim, sr_mosaic) of super_resolve_grid against the N x N (or N_u x N_v) HR mosaic: means over all the
+    grid's views with value > 0, as test_scene's over A^2."""
     r, sr = _grid_run(net, lr_sai, n, ang, scale, patch, stride, minibatch, None, ops, ang_stride, self_ensemble, world,
                       rank)
     hr = hr_sai.reshape(hr_sai.shape[-2:])
     if tuple(hr.shape) != tuple(sr.shape):
         raise ValueError(f"HR label {tuple(hr.shape)} does not match the SR mosaic {tuple(sr.shape)}")
-    n = int(n)
-    acc = torch.zeros(2 * n * n, dtype=torch.float64, device=sr.device)
+    n_u, n_v = U.ang_pair(n)
+    acc = torch.zeros(2 * n_u * n_v, dtype=torch.float64, device=sr.device)
     ctx = torch.cuda.device(sr.device) if sr.is_cuda else _NullCtx()
     with ctx:
-        r.ops.metric_sums(hr.to(device=sr.device, dtype=torch.float32).contiguous(), sr, n, r.hs, r.ws, acc)
-    psnr, ssim = metrics_from_sums(acc.cpu().numpy(), n, r.hs, r.ws)
+        label = hr.to(device=sr.device, dtype=torch.float32).contiguous()
+        if n_u == n_v:
+            r.ops.metric_sums(label, sr, n_u, r.hs, r.ws, acc)
+        else:
+            r.ops.metric_sums_uv(label, sr, n_u, n_v, r.hs, r.ws, acc)
+    psnr, ssim = metrics_from_sums(acc.cpu().numpy(), (n_u, n_v), r.hs, r.ws)
     return psnr, ssim, sr

@@ -3,7 +3,7 @@ reference's option.py:4-34 (including its `type=bool` quirk: any non-empty strin
 random-init path needs --use_pre_ckpt ''), parsed at import time like the reference because
 utils/utils.py and the entry points do `from option import args`.
 Additive flags (not in the reference): --synthetic, --synthetic_size, --minibatch, --self_ensemble, --full_grid,
---ang_stride."""
+--ang_stride, --grid_views."""
 import argparse
 
 _FLAGS = [
@@ -38,6 +38,8 @@ _FLAGS = [
                          "view-image light fields with overlapping angRes x angRes windows, averaged where they overlap")),
     ("--ang_stride", dict(type=int, default=0, help="angular stride of the --full_grid windows, 1..angRes-1 "
                           "(0: angRes - 1, the fewest windows)")),
+    ("--grid_views", dict(type=str, default="", help="with --full_grid 1: which views to super-resolve; '' the central "
+                          "N x N (N = min(U, V)), 'all' the whole U x V grid, RxC (e.g. 9x13) the central R x C")),
 ]
 
 parser = argparse.ArgumentParser()

@@ -9,8 +9,9 @@ kernels; one D2H copy of the uint8 views per scene feeds the BMP writer.
 With torch.distributed initialised (test.py / inference.py under torchrun), a dataset is split across the ranks by
 `scene.assign_scenes`: full rounds of scenes run one per rank, the remaining scenes are row-sharded over all ranks.
 
-With --full_grid 1 every scene is the central N x N of a larger light field (data_info [A, A, N]); it runs through
-`scene.test_grid`: overlapping A x A windows (A = args.angRes_in), averaged where they overlap, N^2 views written."""
+With --full_grid 1 every scene is the central N x N of a larger light field (data_info [A, A, N]), or with --grid_views
+its whole U x V grid or central R x C (data_info [A, A, N_u, N_v]); it runs through `scene.test_grid`: overlapping A x A
+windows (A = args.angRes_in), averaged where they overlap, N_u * N_v views written."""
 import torch
 
 from lfsr_b200 import scene as _scene
@@ -20,12 +21,13 @@ from lfsr_b200 import lfutils as _lfutils
 def _write_views(save_dir, name, sr_sai_y, cbcr, ang):
     """Colour tail of the reference's test() (train.py:329-341): cat(Y, CbCr) -> ycbcr2rgb -> clip*255 -> uint8 -> one
     View_i_j.bmp per view. The conversion runs on the device (lfsr_ycbcr_to_rgb8, bit-exact to the reference's fp64 numpy
-    arithmetic) so only 1 byte per channel crosses PCIe; the BMP files are byte-identical to imageio.imwrite's."""
+    arithmetic) so only 1 byte per channel crosses PCIe; the BMP files are byte-identical to imageio.imwrite's.
+    ang: an ang x ang grid of views, or (N_u, N_v) for N_u x N_v (i < N_u, j < N_v)."""
     d = save_dir.joinpath(name)
     d.mkdir(exist_ok=True)
     views = _lfutils.sai_to_rgb8_views(sr_sai_y, cbcr, ang).cpu().numpy()
-    for i in range(ang):
-        for j in range(ang):
+    for i in range(views.shape[0]):
+        for j in range(views.shape[1]):
             _lfutils.write_bmp(str(d) + "/View_%d_%d.bmp" % (i, j), views[i, j])
 
 
@@ -77,11 +79,12 @@ def gather_in_order(rows, world):
 
 
 def grid_size(data_info):
-    """N of a full-grid scene: the third data_info entry (utils_datasets.ViewsTestSet with full_grid)."""
+    """(N_u, N_v) of a full-grid scene: data_info [A, A, N] (utils_datasets.ViewsTestSet with full_grid: N_u = N_v = N)
+    or [A, A, N_u, N_v] (with --grid_views)."""
     if len(data_info) < 3:
         raise ValueError("--full_grid 1: the loader did not report the grid size of the scene")
-    n = data_info[2]
-    return int(n[0].item()) if torch.is_tensor(n) else int(n)
+    n = [int(x[0].item()) if torch.is_tensor(x) else int(x) for x in data_info[2:4]]
+    return (n[0], n[0]) if len(n) == 1 else (n[0], n[1])
 
 
 def test(test_loader, device, net, args, save_dir=None):

@@ -16,8 +16,10 @@ import torch
 
 
 def _batch1(lr, hr, cbcr, ang_in, ang_out, name, grid=None):
-    """grid: the N of a full-grid scene (--full_grid 1), carried as a third data_info entry next to the window size"""
-    info = [torch.tensor([ang_in]), torch.tensor([ang_out])] + ([] if grid is None else [torch.tensor([grid])])
+    """grid: the N of a full-grid scene (--full_grid 1), carried as a third data_info entry next to the window size, or
+    its (N_u, N_v) (--grid_views), carried as a third and a fourth"""
+    grid = [] if grid is None else list(grid) if isinstance(grid, (tuple, list)) else [grid]
+    info = [torch.tensor([ang_in]), torch.tensor([ang_out])] + [torch.tensor([g]) for g in grid]
     return (lr[None], hr[None], cbcr[None], info, [name])
 
 
@@ -108,11 +110,29 @@ def _check_rgb8(im, fn):
             raise ValueError(f"{fn}: 16-bit samples are not supported (8-bit RGB views only)")
 
 
-def read_views(scene_dir, ang, full_grid=False):
+def parse_grid_views(value, full_grid):
+    """--grid_views -> None ('' : the central N x N, N = min(U, V)), "all" (the whole U x V grid) or (R, C) (the central
+    R x C views, from "RxC"). Valid only with --full_grid 1. Raises ValueError naming the flag."""
+    value = (value or "").strip()
+    if not value:
+        return None
+    if not full_grid:
+        raise ValueError(f"--grid_views {value!r} needs --full_grid 1")
+    if value == "all":
+        return "all"
+    m = re.fullmatch(r"(\d+)x(\d+)", value)
+    if not m or int(m.group(1)) < 1 or int(m.group(2)) < 1:
+        raise ValueError(f"--grid_views {value!r}: expected '', 'all' or RxC with positive integers R and C (e.g. 9x13)")
+    return int(m.group(1)), int(m.group(2))
+
+
+def read_views(scene_dir, ang, full_grid=False, grid=None):
     """the central ang x ang views of one scene folder of View_u_v.{png,bmp} images -> uint8 [ang, ang, H, W, 3]; with
     full_grid, the central N x N views with N = min(U, V) of the U x V grid -> uint8 [N, N, H, W, 3] (angular window
-    tiling, include/lfsr.h). Every view of the grid must be present, 8-bit RGB and of one size (headers only are read for
-    the views outside the centre); only the central views are decoded. Raises ValueError naming the file and the problem."""
+    tiling, include/lfsr.h), or with grid = "all" the whole grid [U, V, H, W, 3] and with grid = (R, C) the central R x C
+    views [R, C, H, W, 3] (--grid_views; A <= R <= U and A <= C <= V). Every view of the grid must be present, 8-bit RGB
+    and of one size (headers only are read for the views outside the centre); only the chosen views are decoded. Raises
+    ValueError naming the file and the problem."""
     from PIL import Image
     files = {}
     for f in sorted(os.listdir(scene_dir)):
@@ -134,6 +154,17 @@ def read_views(scene_dir, ang, full_grid=False):
                                  f"from the {U}x{V} grid")
     if U < ang or V < ang:
         raise ValueError(f"{scene_dir}: a {U}x{V} grid of views is smaller than angRes {ang}x{ang}")
+    if grid is not None and not full_grid:
+        raise ValueError("--grid_views needs --full_grid 1")
+    if grid is None:
+        nu = nv = min(U, V) if full_grid else ang
+    elif grid == "all":
+        nu, nv = U, V
+    else:
+        nu, nv = (int(g) for g in grid)
+        if not (ang <= nu <= U and ang <= nv <= V):
+            raise ValueError(f"{scene_dir}: --grid_views {nu}x{nv} is not a sub-grid of the {U}x{V} grid of views of at "
+                             f"least angRes {ang}x{ang}")
     size = None
     for (u, v), fn in sorted(files.items()):
         with Image.open(fn) as im:
@@ -142,11 +173,10 @@ def read_views(scene_dir, ang, full_grid=False):
                 size, first = im.size, fn
             elif im.size != size:
                 raise ValueError(f"{fn}: view is {im.size[0]}x{im.size[1]} (WxH) but {first} is {size[0]}x{size[1]}")
-    n = min(U, V) if full_grid else ang
-    u0, v0 = (U - n) // 2, (V - n) // 2
-    out = np.empty((n, n, size[1], size[0], 3), dtype=np.uint8)
-    for i in range(n):
-        for j in range(n):
+    u0, v0 = (U - nu) // 2, (V - nv) // 2
+    out = np.empty((nu, nv, size[1], size[0], 3), dtype=np.uint8)
+    for i in range(nu):
+        for j in range(nv):
             with Image.open(files[(u0 + i, v0 + j)]) as im:
                 out[i, j] = np.asarray(im)
     return out
@@ -164,12 +194,15 @@ class ViewsTestSet:
     (inference.py; Hr_SAI_y is an empty tensor). Yields the batch-1 5-tuple with the tensors on the current CUDA device;
     __getitem__ decodes only the scene asked for. full_grid: every view of the central N x N (N = min(U, V)) instead of
     the central A x A, for angular window tiling (scene.test_grid / super_resolve_grid); data_info is then
-    [A, A, N]."""
+    [A, A, N]. grid ("all" or (R, C), parse_grid_views; full_grid only): the whole grid or its central R x C views
+    instead, and data_info [A, A, N_u, N_v]."""
 
-    def __init__(self, args, data_name, kind, full_grid=False):
+    def __init__(self, args, data_name, kind, full_grid=False, grid=None):
         if kind not in ("hr", "lr"):
             raise ValueError(f"kind must be 'hr' or 'lr', got {kind!r}")
-        self.args, self.kind, self.full_grid = args, kind, bool(full_grid)
+        if grid is not None and not full_grid:
+            raise ValueError("--grid_views needs --full_grid 1")
+        self.args, self.kind, self.full_grid, self.grid = args, kind, bool(full_grid), grid
         self.root = os.path.join(args.path_for_test, data_name)
         self.scenes = _scene_dirs(self.root)
 
@@ -180,7 +213,10 @@ class ViewsTestSet:
         if not 0 <= i < len(self.scenes):
             raise IndexError(i)
         A, s = self.args.angRes_in, self.args.scale_factor
-        if self.full_grid:
+        if self.grid is not None:
+            rgb8 = read_views(os.path.join(self.root, self.scenes[i]), A, full_grid=True, grid=self.grid)
+            n = tuple(rgb8.shape[:2])
+        elif self.full_grid:
             rgb8 = read_views(os.path.join(self.root, self.scenes[i]), A, full_grid=True)
             n = rgb8.shape[0]
         else:
@@ -202,8 +238,10 @@ def MultiTestSetDataLoader(args, views=None):
     <path_for_test>/SR_AxA_sx/<data_name>/*.h5 if that directory exists (or `views` is None); otherwise light fields
     stored as view images, <path_for_test>/<data_name>/<scene>/View_u_v.{png,bmp}, read as `views` = "hr" (ground
     truth, test.py) or "lr" (LR input, inference.py). --full_grid 1 (every view, angular window tiling) needs the view
-    layout: synthetic scenes and h5 files hold only A x A views, so it raises ValueError with them."""
+    layout: synthetic scenes and h5 files hold only A x A views, so it raises ValueError with them. --grid_views (the
+    whole grid or a central R x C of it, parse_grid_views) raises ValueError without --full_grid 1 or when malformed."""
     full_grid = bool(getattr(args, "full_grid", 0))
+    grid = parse_grid_views(getattr(args, "grid_views", ""), full_grid)
     if full_grid and getattr(args, "synthetic", 0) > 0:
         raise ValueError("--full_grid 1 needs light fields stored as view images: --synthetic scenes have only "
                          f"{args.angRes_in}x{args.angRes_in} views")
@@ -223,7 +261,7 @@ def MultiTestSetDataLoader(args, views=None):
         names = [d for d in sorted(os.listdir(root)) if _scene_dirs(os.path.join(root, d))] if os.path.isdir(root) else []
     else:
         names = [args.data_name]
-    loaders = [ViewsTestSet(args, n, views, full_grid) for n in names]
+    loaders = [ViewsTestSet(args, n, views, full_grid, grid) for n in names]
     n_scenes = sum(len(d) for d in loaders)
     if n_scenes == 0:
         raise FileNotFoundError(
