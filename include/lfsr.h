@@ -159,6 +159,12 @@ int lfsr_ycbcr_to_rgb8(const float* y, const float* cb, const float* cr, unsigne
  * lfsr_ycbcr_to_rgb8 is this with ang_u = ang_v = ang. */
 int lfsr_ycbcr_to_rgb8_uv(const float* y, const float* cb, const float* cr, unsigned char* rgb, int ang_u, int ang_v, int h,
                           int w, const double* mat_inv255, const double* offset, void* stream);
+/* the same with the output in one of the layouts of "Image light fields" below: LFSR_LAYOUT_VIEWS [ang_u][ang_v][h][w][3]
+ * (lfsr_ycbcr_to_rgb8_uv is this with layout 0), LFSR_LAYOUT_MOSAIC [(ang_u h)][(ang_v w)][3] or LFSR_LAYOUT_LENSLET
+ * [(h ang_u)][(w ang_v)][3]. Only the store address differs between the layouts. LFSR_ERR_INVALID for an unknown layout or
+ * a mosaic side of 2^31 or more. */
+int lfsr_ycbcr_to_rgb8_layout(const float* y, const float* cb, const float* cr, unsigned char* rgb, int ang_u, int ang_v,
+                              int h, int w, int layout, const double* mat_inv255, const double* offset, void* stream);
 
 /* ---- View preparation (input side; BasicLFSR's Generate_Data_for_Test.py / _for_inference.py as recorded in DESIGN.md
  * row f-7: the generator scripts are not in this tree, so parity with them is unpinned). Per scene of U x V RGB views
@@ -183,6 +189,21 @@ int lfsr_rgb_to_ycbcr_mosaic(const void* views, int is_u8, float* y, float* cb, 
  * lfsr_rgb_to_ycbcr_mosaic is this with ang_u = ang_v = ang. */
 int lfsr_rgb_to_ycbcr_mosaic_uv(const void* views, int is_u8, float* y, float* cb, float* cr, int ang_u, int ang_v, int h,
                                 int w, void* stream);
+
+/* Image light fields: a U x V grid of H x W RGB views stored as ONE 8-bit RGB image instead of U*V view files.
+ *   mosaic   (sub-aperture image array) image [(U H)][(V W)][3]: image pixel (u*H + h, v*W + w) is view (u, v) at (h, w);
+ *   lenslet  (macro-pixel image, BasicLFSR's MacPI) image [(H U)][(W V)][3]: image pixel (h*U + u, w*V + v) is view (u, v) at
+ *            (h, w). For U = V = A this is SAI2MacPI (DistgSSR.py:145-155, oracle/nets.py `sai2macpi`) on each channel.
+ * Which views are taken, the crop and the colour / resampling recipe above are exactly those of the same light field
+ * stored as View_u_v files, so both give the same Lr_SAI_y / Hr_SAI_y / Sr_SAI_cbcr bit for bit.
+ *
+ * lfsr_image_to_views_u8: img (uint8, device) in `layout` (LFSR_LAYOUT_MOSAIC or LFSR_LAYOUT_LENSLET) -> the views
+ * [u0, u0 + n_u) x [v0, v0 + n_v), each cropped top-left to hc x wc, as view-major uint8 [n_u][n_v][hc][wc][3] (the input
+ * of lfsr_rgb_to_ycbcr_mosaic). A pure gather, bit-exact. LFSR_ERR_INVALID for an unknown layout, a selection outside the
+ * grid, hc > H or wc > W, or an image side U*H or V*W of 2^31 or more. */
+enum { LFSR_LAYOUT_VIEWS = 0, LFSR_LAYOUT_MOSAIC = 1, LFSR_LAYOUT_LENSLET = 2 };
+int lfsr_image_to_views_u8(const unsigned char* img, int layout, int U, int V, int H, int W, int u0, int v0, int n_u,
+                           int n_v, int hc, int wc, unsigned char* views, void* stream);
 
 /* One separable pass of the reference's MATLAB-style imresize (utils/imresize.py:57-102 `resizeAlongDim`), fp64:
  * out[a][i][b] = sum_p weights[i][p] * in[a][indices[i][p]][b] over a tensor viewed as [outer][in_len][inner]

@@ -6,7 +6,9 @@ there (wrapped in try/except) and is not reproduced.
 Under torchrun (WORLD_SIZE > 1) each dataset is split across the ranks like test.py's (train.rank_scenes); every
 View_i_j.bmp is written once, by the rank that owns its scene, and only rank 0 prints. With --full_grid 1 every view of
 the central N x N of each light field (with --grid_views: the whole U x V grid, or its central R x C) is super-resolved
-with overlapping angRes x angRes windows (scene.super_resolve_grid) and N_u * N_v View_i_j.bmp are written."""
+with overlapping angRes x angRes windows (scene.super_resolve_grid) and N_u * N_v View_i_j.bmp are written. Light
+fields stored as one mosaic or lenslet image each are read with --input_layout mosaic|lenslet --input_grid UxV; with
+--save_layout mosaic|lenslet each scene's SR grid is written as one <scene>.bmp in that layout."""
 import importlib
 
 import torch
@@ -63,7 +65,7 @@ def run(args, device, rank):
                                                     args.patch_size_for_test, args.stride_for_test, args.minibatch,
                                                     self_ensemble=bool(getattr(args, "self_ensemble", 0)), **shard)
                 if owner:
-                    _write_views(save_dir, lf_name[0], sr, cbcr, views)
+                    _write_views(save_dir, lf_name[0], sr, cbcr, views, getattr(args, "save_layout", "views"))
                     written.append((i, lf_name[0]))
                     if world == 1:
                         print("scene %s -> %s" % (lf_name[0], save_dir))

@@ -22,6 +22,7 @@ PERM_NONE, PERM_MACPI_OVER_SAI = 0, 1
 SHUF_CHANNEL_MAJOR, SHUF_FACTOR_MAJOR = 0, 1
 INTERP_BICUBIC, INTERP_BILINEAR = 0, 1
 OUT_F32, OUT_BOTH, OUT_F16 = 0, 1, 2       # lfsr_conv_desc.out_mode
+LAYOUT_VIEWS, LAYOUT_MOSAIC, LAYOUT_LENSLET = 0, 1, 2
 
 
 class LfsrError(RuntimeError):
@@ -93,6 +94,8 @@ SIGNATURES = {
     "lfsr_interp": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "lfsr_ycbcr_to_rgb8": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
     "lfsr_ycbcr_to_rgb8_uv": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P]),
+    "lfsr_ycbcr_to_rgb8_layout": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "lfsr_image_to_views_u8": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P]),
     "lfsr_resample_f64": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "lfsr_rgb_to_ycbcr_mosaic": (_I, [_P, _I, _P, _P, _P, _I, _I, _I, _P]),
     "lfsr_rgb_to_ycbcr_mosaic_uv": (_I, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _P]),

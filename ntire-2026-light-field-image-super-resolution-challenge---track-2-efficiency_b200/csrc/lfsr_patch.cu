@@ -382,19 +382,24 @@ extern "C" int lfsr_integrate_rows_d8(const float* patches8, float* out, int ang
 // ---- colour tail of test() (train.py:329-341, utils/utils.py:191-204): Y mosaic + CbCr mosaic -> uint8 RGB views -------
 // rgb8[u][v][y][x][c] = uint8(clip(M[c][0]*Y + M[c][1]*Cb + M[c][2]*Cr - off[c], 0, 1) * 255), fp64 with separate multiplies and
 // adds in the reference's left-to-right order (no FMA contraction) and truncation like numpy's astype('uint8'); the
-// (a1 h)(a2 w) -> a1 a2 h w view split is folded into the store address. 1 byte per channel leaves the GPU, not 4.
+// (a1 h)(a2 w) -> a1 a2 h w view split (or the mosaic / lenslet image address of the output layout) is folded into the
+// store address. 1 byte per channel leaves the GPU, not 4.
 namespace lfsr {
 struct ColourMat { double m[9]; double off[3]; };
 __global__ void __launch_bounds__(256)
 ycbcr_rgb8_kernel(const float* __restrict__ y, const float* __restrict__ cb, const float* __restrict__ cr,
-                  unsigned char* __restrict__ rgb, int ang_u, int ang_v, int h, int w, ColourMat cm) {
+                  unsigned char* __restrict__ rgb, int ang_u, int ang_v, int h, int w, int layout, ColourMat cm) {
   const int W = ang_v * w;
   const long long total = (long long)ang_u * h * W;
   for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
     const int X = (int)(t % W), Y = (int)(t / W);
     const int u = Y / h, yy = Y - u * h, v = X / w, xx = X - v * w;
     const double a = (double)y[t], b = (double)cb[t], c = (double)cr[t];
-    unsigned char* dst = rgb + ((((long long)u * ang_v + v) * h + yy) * w + xx) * 3;
+    long long px;                                       // output pixel index in the chosen layout
+    if (layout == LFSR_LAYOUT_MOSAIC) px = t;
+    else if (layout == LFSR_LAYOUT_LENSLET) px = ((long long)yy * ang_u + u) * W + (long long)xx * ang_v + v;
+    else px = (((long long)u * ang_v + v) * h + yy) * w + xx;
+    unsigned char* dst = rgb + px * 3;
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
       double r = __dadd_rn(__dadd_rn(__dmul_rn(cm.m[3 * k], a), __dmul_rn(cm.m[3 * k + 1], b)), __dmul_rn(cm.m[3 * k + 2], c));
@@ -413,15 +418,25 @@ extern "C" int lfsr_ycbcr_to_rgb8(const float* y, const float* cb, const float* 
 
 extern "C" int lfsr_ycbcr_to_rgb8_uv(const float* y, const float* cb, const float* cr, unsigned char* rgb, int ang_u,
                                      int ang_v, int h, int w, const double* mat_inv255, const double* offset, void* stream) {
+  return lfsr_ycbcr_to_rgb8_layout(y, cb, cr, rgb, ang_u, ang_v, h, w, LFSR_LAYOUT_VIEWS, mat_inv255, offset, stream);
+}
+
+extern "C" int lfsr_ycbcr_to_rgb8_layout(const float* y, const float* cb, const float* cr, unsigned char* rgb, int ang_u,
+                                         int ang_v, int h, int w, int layout, const double* mat_inv255, const double* offset,
+                                         void* stream) {
   LFSR_REQUIRE(y && cb && cr && rgb && mat_inv255 && offset, "lfsr_ycbcr_to_rgb8: null pointer");
   LFSR_REQUIRE(ang_u > 0 && ang_v > 0 && h > 0 && w > 0, "lfsr_ycbcr_to_rgb8: bad geometry");
+  LFSR_REQUIRE(layout == LFSR_LAYOUT_VIEWS || layout == LFSR_LAYOUT_MOSAIC || layout == LFSR_LAYOUT_LENSLET,
+               "lfsr_ycbcr_to_rgb8: unknown output layout %d", layout);
+  LFSR_REQUIRE((long long)ang_u * h < (1LL << 31) && (long long)ang_v * w < (1LL << 31),
+               "lfsr_ycbcr_to_rgb8: mosaic %lldx%lld too large", (long long)ang_u * h, (long long)ang_v * w);
   lfsr::ColourMat cm;
   for (int i = 0; i < 9; ++i) cm.m[i] = mat_inv255[i];
   for (int i = 0; i < 3; ++i) cm.off[i] = offset[i];
   const long long total = (long long)ang_u * h * ang_v * w;
   long long blocks = (total + 255) / 256;
   if (blocks > 148LL * 32) blocks = 148LL * 32;
-  lfsr::ycbcr_rgb8_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(y, cb, cr, rgb, ang_u, ang_v, h, w, cm);
+  lfsr::ycbcr_rgb8_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(y, cb, cr, rgb, ang_u, ang_v, h, w, layout, cm);
   return lfsr::check_launch("ycbcr_rgb8_kernel");
 }
 
@@ -485,6 +500,53 @@ extern "C" int lfsr_rgb_to_ycbcr_mosaic_uv(const void* views, int is_u8, float* 
                                                                                           ang_u, ang_v, h, w);
   }
   return lfsr::check_launch("rgb_ycbcr_mosaic_kernel");
+}
+
+// Image light fields (include/lfsr.h, "View preparation"): the views [u0, u0 + n_u) x [v0, v0 + n_v) of a U x V grid stored
+// as one mosaic or lenslet image, each cropped to hc x wc, gathered into view-major uint8 [n_u][n_v][hc][wc][3]. One thread
+// per output pixel in output order, so the stores are dense; the layout is folded into the load address.
+namespace lfsr {
+__global__ void __launch_bounds__(256)
+image_to_views_kernel(const unsigned char* __restrict__ img, unsigned char* __restrict__ views, int layout, int U, int V,
+                      int H, int W, int u0, int v0, int n_v, int hc, int wc, long long total) {
+  const long long row_px = (long long)V * W;            // image pixels per row, both layouts
+  for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
+    const int x = (int)(t % wc);
+    const long long r = t / wc;
+    const int y = (int)(r % hc);
+    const int view = (int)(r / hc);
+    const int u = u0 + view / n_v, v = v0 + view % n_v;
+    const long long px = layout == LFSR_LAYOUT_MOSAIC ? ((long long)u * H + y) * row_px + (long long)v * W + x
+                                                      : ((long long)y * U + u) * row_px + (long long)x * V + v;
+    const unsigned char* src = img + px * 3;
+    unsigned char* dst = views + t * 3;
+    dst[0] = __ldg(src);
+    dst[1] = __ldg(src + 1);
+    dst[2] = __ldg(src + 2);
+  }
+}
+}  // namespace lfsr
+
+extern "C" int lfsr_image_to_views_u8(const unsigned char* img, int layout, int U, int V, int H, int W, int u0, int v0,
+                                      int n_u, int n_v, int hc, int wc, unsigned char* views, void* stream) {
+  LFSR_REQUIRE(img && views, "lfsr_image_to_views_u8: null pointer");
+  LFSR_REQUIRE(layout == LFSR_LAYOUT_MOSAIC || layout == LFSR_LAYOUT_LENSLET,
+               "lfsr_image_to_views_u8: unknown image layout %d (1 mosaic, 2 lenslet)", layout);
+  LFSR_REQUIRE(U > 0 && V > 0 && H > 0 && W > 0 && n_u > 0 && n_v > 0 && hc > 0 && wc > 0,
+               "lfsr_image_to_views_u8: bad geometry grid=%dx%d view=%dx%d sel=%dx%d crop=%dx%d", U, V, H, W, n_u, n_v,
+               hc, wc);
+  LFSR_REQUIRE(u0 >= 0 && v0 >= 0 && (long long)u0 + n_u <= U && (long long)v0 + n_v <= V,
+               "lfsr_image_to_views_u8: views [%d, %d) x [%d, %d) lie outside the %dx%d grid", u0, u0 + n_u, v0, v0 + n_v,
+               U, V);
+  LFSR_REQUIRE(hc <= H && wc <= W, "lfsr_image_to_views_u8: crop %dx%d larger than the %dx%d views", hc, wc, H, W);
+  LFSR_REQUIRE((long long)U * H < (1LL << 31) && (long long)V * W < (1LL << 31),
+               "lfsr_image_to_views_u8: image %lldx%lld too large", (long long)U * H, (long long)V * W);
+  const long long total = (long long)n_u * n_v * hc * wc;
+  long long blocks = (total + 255) / 256;
+  if (blocks > 148LL * 32) blocks = 148LL * 32;
+  lfsr::image_to_views_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(img, views, layout, U, V, H, W, u0, v0, n_v,
+                                                                              hc, wc, total);
+  return lfsr::check_launch("image_to_views_kernel");
 }
 
 

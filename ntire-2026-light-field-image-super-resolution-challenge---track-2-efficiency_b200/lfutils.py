@@ -259,10 +259,8 @@ def ang_pair(angRes):
     return int(angRes), int(angRes)
 
 
-def sai_to_rgb8_views(sr_y: torch.Tensor, sr_cbcr: torch.Tensor, angRes) -> torch.Tensor:
-    """Sr_SAI_y [.., (a1 h), (a2 w)] + Sr_SAI_cbcr [.., 2, (a1 h), (a2 w)] -> uint8 [a1, a2, h, w, 3] on the device:
-    torch.cat + ycbcr2rgb (fp64) + clip(0,1)*255 + astype(uint8) + the view rearrange of train.py:332-335 in one kernel.
-    angRes: a1 = a2 as an int, or the pair (a1, a2) of a rectangular grid."""
+def _colour_inputs(sr_y: torch.Tensor, sr_cbcr: torch.Tensor, angRes):
+    """the arguments of the colour-tail kernels: (Y, CbCr mosaics on the device, a1, a2, H, W, inv(M) * 255, offset)"""
     y = sr_y.reshape(sr_y.shape[-2:])
     cbcr = sr_cbcr.reshape(2, *sr_cbcr.shape[-2:])
     if cbcr.shape[-2:] != y.shape:
@@ -279,8 +277,16 @@ def sai_to_rgb8_views(sr_y: torch.Tensor, sr_cbcr: torch.Tensor, angRes) -> torc
     inv = np.linalg.inv(_BT601)                                   # exactly the reference's constants (utils/utils.py:192-198)
     offset = np.ascontiguousarray(np.matmul(inv, np.array([16, 128, 128])))
     inv255 = np.ascontiguousarray(inv * 255)
-    out = torch.empty((au, av, H // au, W // av, 3), dtype=torch.uint8, device=dev)
-    lib, stream = N.load(), torch.cuda.current_stream(dev).cuda_stream
+    return y, cbcr, au, av, H, W, inv255, offset
+
+
+def sai_to_rgb8_views(sr_y: torch.Tensor, sr_cbcr: torch.Tensor, angRes) -> torch.Tensor:
+    """Sr_SAI_y [.., (a1 h), (a2 w)] + Sr_SAI_cbcr [.., 2, (a1 h), (a2 w)] -> uint8 [a1, a2, h, w, 3] on the device:
+    torch.cat + ycbcr2rgb (fp64) + clip(0,1)*255 + astype(uint8) + the view rearrange of train.py:332-335 in one kernel.
+    angRes: a1 = a2 as an int, or the pair (a1, a2) of a rectangular grid."""
+    y, cbcr, au, av, H, W, inv255, offset = _colour_inputs(sr_y, sr_cbcr, angRes)
+    out = torch.empty((au, av, H // au, W // av, 3), dtype=torch.uint8, device=y.device)
+    lib, stream = N.load(), torch.cuda.current_stream(y.device).cuda_stream
     if not isinstance(angRes, (tuple, list)):
         N.check(lib.lfsr_ycbcr_to_rgb8(y.data_ptr(), cbcr[0].data_ptr(), cbcr[1].data_ptr(), out.data_ptr(), angRes,
                                        H // angRes, W // angRes, inv255.ctypes.data, offset.ctypes.data, stream),
@@ -289,6 +295,32 @@ def sai_to_rgb8_views(sr_y: torch.Tensor, sr_cbcr: torch.Tensor, angRes) -> torc
         N.check(lib.lfsr_ycbcr_to_rgb8_uv(y.data_ptr(), cbcr[0].data_ptr(), cbcr[1].data_ptr(), out.data_ptr(), au, av,
                                           H // au, W // av, inv255.ctypes.data, offset.ctypes.data, stream),
                 "lfsr_ycbcr_to_rgb8_uv")
+    return out
+
+
+#: the layouts of a light field's views (include/lfsr.h, "Image light fields"): View_u_v files, or one image
+LAYOUTS = {"views": N.LAYOUT_VIEWS, "mosaic": N.LAYOUT_MOSAIC, "lenslet": N.LAYOUT_LENSLET}
+
+
+def _layout_code(layout: str, image_only: bool = False) -> int:
+    names = ("mosaic", "lenslet") if image_only else tuple(LAYOUTS)
+    if layout not in names:
+        raise ValueError(f"layout must be one of {', '.join(names)}; got {layout!r}")
+    return LAYOUTS[layout]
+
+
+def sai_to_rgb8(sr_y: torch.Tensor, sr_cbcr: torch.Tensor, angRes, layout: str = "views") -> torch.Tensor:
+    """sai_to_rgb8_views with the output in `layout`: "views" uint8 [a1, a2, h, w, 3] (sai_to_rgb8_views' result),
+    "mosaic" the sub-aperture image array [(a1 h), (a2 w), 3] or "lenslet" the macro-pixel image [(h a1), (w a2), 3], written
+    by the same kernel (lfsr_ycbcr_to_rgb8_layout; only the store address depends on the layout)."""
+    code = _layout_code(layout)
+    y, cbcr, au, av, H, W, inv255, offset = _colour_inputs(sr_y, sr_cbcr, angRes)
+    shape = (au, av, H // au, W // av, 3) if code == N.LAYOUT_VIEWS else (H, W, 3)
+    out = torch.empty(shape, dtype=torch.uint8, device=y.device)
+    N.check(N.load().lfsr_ycbcr_to_rgb8_layout(y.data_ptr(), cbcr[0].data_ptr(), cbcr[1].data_ptr(), out.data_ptr(), au, av,
+                                               H // au, W // av, code, inv255.ctypes.data, offset.ctypes.data,
+                                               torch.cuda.current_stream(y.device).cuda_stream),
+            "lfsr_ycbcr_to_rgb8_layout")
     return out
 
 
@@ -351,24 +383,43 @@ def _unit(x8: torch.Tensor) -> torch.Tensor:
     return lut.index_select(0, x8.reshape(-1).to(torch.int32)).view(x8.shape)
 
 
+def _current_cuda_device() -> torch.device:
+    if not torch.cuda.is_available():
+        raise N.LfsrError("lfsr_b200 needs a CUDA device (sm_100a); there is no CPU fallback for this path")
+    return torch.device("cuda", torch.cuda.current_device())
+
+
+def _to_device_pinned(a: np.ndarray, dev: torch.device) -> torch.Tensor:
+    """one H2D copy of a host uint8 array through a pinned staging buffer"""
+    host = torch.empty(a.shape, dtype=torch.uint8, pin_memory=True)
+    host.numpy()[...] = a
+    return host.to(dev, non_blocking=True)
+
+
+def _check_kind(kind: str) -> None:
+    if kind not in ("hr", "lr"):
+        raise ValueError(f"kind must be 'hr' or 'lr', got {kind!r}")
+
+
 def prepare_views(rgb8, angRes, scale: int, kind: str = "hr"):
     """RGB views of one scene -> (Lr_SAI_y, Hr_SAI_y or None, Sr_SAI_cbcr) as fp32 mosaics on the current CUDA device,
     by the recipe of include/lfsr.h. rgb8: host uint8 [U, V, H, W, 3]; angRes: the central angRes x angRes views, or the
     central a1 x a2 for a pair (a1, a2). kind="hr": the views are ground truth (test.py),
     the LR input is their bicubic x1/scale; kind="lr": the views are the LR input (inference.py) and there is no HR.
     The cropped central views cross PCIe once (3 bytes per pixel, from pinned memory); the rest runs on the device."""
-    if kind not in ("hr", "lr"):
-        raise ValueError(f"kind must be 'hr' or 'lr', got {kind!r}")
+    _check_kind(kind)
     a = np.asarray(rgb8)
     if a.dtype != np.uint8:
         raise ValueError(f"prepare_views takes uint8 views, got {a.dtype}")
-    if not torch.cuda.is_available():
-        raise N.LfsrError("lfsr_b200 needs a CUDA device (sm_100a); there is no CPU fallback for this path")
-    dev = torch.device("cuda", torch.cuda.current_device())
-    crop = central_views(a, angRes, scale)
-    host = torch.empty(crop.shape, dtype=torch.uint8, pin_memory=True)
-    host.numpy()[...] = crop
-    x8 = host.to(dev, non_blocking=True)
+    dev = _current_cuda_device()
+    x8 = _to_device_pinned(central_views(a, angRes, scale), dev)
+    return prepare_device_views(x8, angRes, scale, kind)
+
+
+def prepare_device_views(x8: torch.Tensor, angRes, scale: int, kind: str = "hr"):
+    """the device half of prepare_views: the chosen views, already cropped, as uint8 [a1, a2, h, w, 3] on the device ->
+    (Lr_SAI_y, Hr_SAI_y or None, Sr_SAI_cbcr)."""
+    _check_kind(kind)
     A = angRes
     if kind == "hr":
         hr_y, _ = rgb_to_ycbcr_mosaic(x8, A, cbcr=False)
@@ -379,6 +430,57 @@ def prepare_views(rgb8, angRes, scale: int, kind: str = "hr"):
         lr_y, _ = rgb_to_ycbcr_mosaic(x8, A, cbcr=False)
     _, sr_cbcr = rgb_to_ycbcr_mosaic(imresize_views(lr_rgb, float(scale)), A, y=False)
     return lr_y, hr_y, sr_cbcr
+
+
+def image_geometry(shape, grid):
+    """(U, V, H, W) of an image light field of `grid` = (U, V) views stored as an image of `shape` [rows, cols, 3] (either
+    layout: rows = U * H, cols = V * W). Raises ValueError when the image cannot hold such a grid."""
+    U, V = (int(g) for g in grid)
+    if len(shape) != 3 or shape[2] != 3:
+        raise ValueError(f"expected an RGB image [rows, cols, 3], got {tuple(shape)}")
+    rows, cols = int(shape[0]), int(shape[1])
+    if U < 1 or V < 1 or rows % U or cols % V or rows == 0 or cols == 0:
+        raise ValueError(f"a {cols}x{rows} (WxH) image does not hold a {U}x{V} grid of views: its height must be a "
+                         f"multiple of {U} and its width a multiple of {V}")
+    return U, V, rows // U, cols // V
+
+
+def image_to_views(img8_host, layout: str, grid, sel, scale: int) -> torch.Tensor:
+    """An image light field (include/lfsr.h, "Image light fields") -> the views the preparation uses, as uint8
+    [a1, a2, h, w, 3] on the current CUDA device: the central sel x sel views (or a1 x a2 for sel = (a1, a2)) of the
+    grid = (U, V) views stored in `layout` ("mosaic" or "lenslet"), each cropped top-left to a multiple of `scale`, the
+    same as central_views on the views of the grid. The decoded image crosses PCIe once (from pinned memory); the
+    gather runs on the device (lfsr_image_to_views_u8)."""
+    code = _layout_code(layout, image_only=True)
+    img = np.asarray(img8_host)
+    if img.dtype != np.uint8:
+        raise ValueError(f"image_to_views takes a uint8 image, got {img.dtype}")
+    U, V, H, W = image_geometry(img.shape, grid)
+    au, av = ang_pair(sel)
+    if U < au or V < av:
+        raise ValueError(f"a {U}x{V} grid of views has no central {au}x{av}")
+    hc, wc = H - H % scale, W - W % scale
+    if hc == 0 or wc == 0:
+        raise ValueError(f"views of {H}x{W} are smaller than the scale factor {scale}")
+    dev = _current_cuda_device()
+    src = _to_device_pinned(img, dev)
+    views = torch.empty((au, av, hc, wc, 3), dtype=torch.uint8, device=dev)
+    N.check(N.load().lfsr_image_to_views_u8(src.data_ptr(), code, U, V, H, W, (U - au) // 2, (V - av) // 2, au, av, hc, wc,
+                                            views.data_ptr(), torch.cuda.current_stream(dev).cuda_stream),
+            "lfsr_image_to_views_u8")
+    return views
+
+
+def prepare_image(img8, layout: str, grid, angRes, scale: int, kind: str = "hr"):
+    """prepare_views for a light field stored as one image: img8 host uint8 [rows, cols, 3] holding grid = (U, V) views in
+    `layout` ("mosaic" or "lenslet"). Gives the same tensors, bit for bit, as prepare_views on those views."""
+    _check_kind(kind)
+    return prepare_device_views(image_to_views(img8, layout, grid, angRes, scale), angRes, scale, kind)
+
+
+def bmp_bytes(h: int, w: int) -> int:
+    """the size of the file write_bmp writes for an [h, w, 3] image; a BMP holds at most 2^32 - 1 bytes"""
+    return 14 + 40 + h * ((w * 3 + 3) & ~3)
 
 
 def write_bmp(path, img) -> None:

@@ -3,7 +3,7 @@ reference's option.py:4-34 (including its `type=bool` quirk: any non-empty strin
 random-init path needs --use_pre_ckpt ''), parsed at import time like the reference because
 utils/utils.py and the entry points do `from option import args`.
 Additive flags (not in the reference): --synthetic, --synthetic_size, --minibatch, --self_ensemble, --full_grid,
---ang_stride, --grid_views."""
+--ang_stride, --grid_views, --input_layout, --input_grid, --save_layout."""
 import argparse
 
 _FLAGS = [
@@ -40,6 +40,14 @@ _FLAGS = [
                           "(0: angRes - 1, the fewest windows)")),
     ("--grid_views", dict(type=str, default="", help="with --full_grid 1: which views to super-resolve; '' the central "
                           "N x N (N = min(U, V)), 'all' the whole U x V grid, RxC (e.g. 9x13) the central R x C")),
+    ("--input_layout", dict(type=str, default="views", choices=["views", "mosaic", "lenslet"],
+                            help="how the test light fields are stored: views = <scene>/View_u_v.png|bmp folders, "
+                            "mosaic = one sub-aperture image array <scene>.png|bmp, lenslet = one macro-pixel image")),
+    ("--input_grid", dict(type=str, default="", help="UxV views of each mosaic / lenslet image (e.g. 14x14); "
+                          "required with --input_layout mosaic|lenslet")),
+    ("--save_layout", dict(type=str, default="views", choices=["views", "mosaic", "lenslet"],
+                           help="how SR results are written: views = <scene>/View_u_v.bmp, mosaic / lenslet = one "
+                           "<scene>.bmp of the whole SR grid")),
 ]
 
 parser = argparse.ArgumentParser()

@@ -11,18 +11,28 @@ With torch.distributed initialised (test.py / inference.py under torchrun), a da
 
 With --full_grid 1 every scene is the central N x N of a larger light field (data_info [A, A, N]), or with --grid_views
 its whole U x V grid or central R x C (data_info [A, A, N_u, N_v]); it runs through `scene.test_grid`: overlapping A x A
-windows (A = args.angRes_in), averaged where they overlap, N_u * N_v views written."""
+windows (A = args.angRes_in), averaged where they overlap, N_u * N_v views written. With --save_layout mosaic|lenslet
+each scene is written as one <scene>.bmp of its whole SR grid instead of View_i_j.bmp files."""
 import torch
 
 from lfsr_b200 import scene as _scene
 from lfsr_b200 import lfutils as _lfutils
 
 
-def _write_views(save_dir, name, sr_sai_y, cbcr, ang):
+def _write_views(save_dir, name, sr_sai_y, cbcr, ang, layout="views"):
     """Colour tail of the reference's test() (train.py:329-341): cat(Y, CbCr) -> ycbcr2rgb -> clip*255 -> uint8 -> one
     View_i_j.bmp per view. The conversion runs on the device (lfsr_ycbcr_to_rgb8, bit-exact to the reference's fp64 numpy
     arithmetic) so only 1 byte per channel crosses PCIe; the BMP files are byte-identical to imageio.imwrite's.
-    ang: an ang x ang grid of views, or (N_u, N_v) for N_u x N_v (i < N_u, j < N_v)."""
+    ang: an ang x ang grid of views, or (N_u, N_v) for N_u x N_v (i < N_u, j < N_v). layout (--save_layout) "mosaic" or
+    "lenslet": one <save_dir>/<name>.bmp of the whole grid in that layout instead (include/lfsr.h, "Image light fields")."""
+    if layout != "views":
+        rows, cols = sr_sai_y.shape[-2:]
+        if _lfutils.bmp_bytes(rows, cols) >= 1 << 32:
+            raise ValueError(f"--save_layout {layout}: the {cols}x{rows} (WxH) image of scene {name} does not fit a BMP "
+                             "file (4 GiB at most); use --save_layout views")
+        _lfutils.write_bmp(str(save_dir.joinpath(name + ".bmp")),
+                           _lfutils.sai_to_rgb8(sr_sai_y, cbcr, ang, layout).cpu().numpy())
+        return
     d = save_dir.joinpath(name)
     d.mkdir(exist_ok=True)
     views = _lfutils.sai_to_rgb8_views(sr_sai_y, cbcr, ang).cpu().numpy()
@@ -113,6 +123,6 @@ def test(test_loader, device, net, args, save_dir=None):
         if owner:
             rows.append((i, psnr, ssim, LF_name[0]))
             if save_dir is not None:
-                _write_views(save_dir, LF_name[0], sr, Sr_SAI_cbcr, views)
+                _write_views(save_dir, LF_name[0], sr, Sr_SAI_cbcr, views, getattr(args, "save_layout", "views"))
     rows = gather_in_order(rows, world)
     return [r[1] for r in rows], [r[2] for r in rows], [r[3] for r in rows]
