@@ -94,6 +94,7 @@ typedef struct {
    *              geometry, its pointer is not written). Copies need channel counts that are multiples of 8. */
   int32_t in_f16, out_mode;
   lfsr_tensor out16;     /* fp16 view with out's geometry (ld in 2-byte elements) */
+  const float* tail_w_host;   /* host copy of tail_w (required with tail_w): read at launch, passed to the kernel by value */
 } lfsr_conv_desc;
 
 const char* lfsr_last_error(void);
@@ -104,6 +105,11 @@ int lfsr_built_for_sm100a(void);
 uint64_t lfsr_launch_count(void);
 /* how many lfsr_conv2d_tc calls took the two-CTAs-per-SM kernel for narrow fp16 layers (tests assert the path taken) */
 uint64_t lfsr_conv_tc_lean_count(void);
+/* how many lfsr_conv2d_tc calls took the halo-block CTA-pair kernel (fp16 3x3 convs with 128 < N <= 256: the upsampler) */
+uint64_t lfsr_conv_tc_halo_count(void);
+/* that kernel's block plan for an h x w image and cout packed output channels: geom[0..7] = output block width, output block rows, padded block width, MMA tiles per block, blocks per image row, block rows
+ * per image, bytes of one input buffer, dynamic shared memory bytes. Returns 1 if the kernel can run that geometry, else 0. */
+int lfsr_conv_tc_halo_plan(int h, int w, int cout, int* geom);
 
 /* ---- patch pipeline ------------------------------------------------------------------ */
 /* LFdivide + ImageExtend (utils/utils.py:137-166): scene [A*h0, A*w0] -> [numU*numV, A*P, A*P],

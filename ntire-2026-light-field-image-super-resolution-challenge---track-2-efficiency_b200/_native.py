@@ -46,6 +46,7 @@ class ConvDesc(C.Structure):
         ("mul", Tensor), ("res", Tensor),
         ("tail_w", C.c_void_p), ("tail_taps", C.c_int32), ("tail_c", C.c_int32),
         ("in_f16", C.c_int32), ("out_mode", C.c_int32), ("out16", Tensor),
+        ("tail_w_host", C.c_void_p),
     ]
 
 
@@ -86,6 +87,8 @@ SIGNATURES = {
     "lfsr_built_for_sm100a": (_I, []),
     "lfsr_launch_count": (C.c_uint64, []),
     "lfsr_conv_tc_lean_count": (C.c_uint64, []),
+    "lfsr_conv_tc_halo_count": (C.c_uint64, []),
+    "lfsr_conv_tc_halo_plan": (_I, [_I, _I, _I, _P]),
     "lfsr_divide": (_I, [_P, _P, _I, _I, _I, _I, _I, _P]),
     "lfsr_divide_rows": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "lfsr_integrate_rows": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),

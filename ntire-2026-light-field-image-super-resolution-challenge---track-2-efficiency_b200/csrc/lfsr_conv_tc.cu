@@ -20,6 +20,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <mutex>
+#include <type_traits>
 #include <cuda_fp16.h>
 #include "lfsr_common.cuh"
 
@@ -27,6 +28,7 @@ namespace lfsr {
 namespace tc {
 
 static std::atomic<uint64_t> g_lean_launches{0};   // launches that took conv_tc_lean_kernel (tests assert the path)
+static std::atomic<uint64_t> g_halo_launches{0};   // launches that took conv_tc_halo_kernel
 constexpr int kThreads = 320;          // warp 0 TMA, warp 1 MMA, warps 2..9 epilogue (two warps per TMEM lane quarter)
 constexpr int kEpiWarps = 8;
 constexpr int kTmaWarp = 8, kMmaWarp = 9;
@@ -49,6 +51,14 @@ inline FastDiv make_fastdiv(int d) {
 }
 __device__ __forceinline__ int fdiv(int n, FastDiv f) { return (int)((__umulhi((uint32_t)n, f.mul) + (uint32_t)n) >> f.shift); }
 
+// Tail-projection table (lfsr_conv_desc.tail_w_host, zero rows beyond cq) passed BY VALUE as a __grid_constant__ kernel
+// parameter: the projection's FFMA2s then take each weight from the constant bank at a compile-time offset instead of a
+// broadcast LDS - those LDS were about as many shared-memory wavefronts per tile as the MMAs' operand reads.
+constexpr int kTailMaxC = 64;
+struct TailW { float w[kTailMaxC * 12]; };
+struct NoTailW {};
+template <bool T> using TailArg = typename std::conditional<T, TailW, NoTailW>::type;
+
 struct Params {
   FastDiv fd_tiles_x, fd_nbx, fd_tiles_y, fd_nby, fd_nchunks, fd_cq, fd_rx;
   int out_mode;                        // 0: fp32 output, 1: fp32 + fp16 copy, 2: fp16 only (lane-per-pixel epilogue only)
@@ -68,8 +78,6 @@ struct Params {
   int act, mul_act;
   float slope, alpha;
   int ry, rx, shuf_mode, cq, vec;      // vec: floats per lane in the coalesced write-out (4, 2 or 1)
-  // halo-block mode (conv_tc_halo_kernel): the input block with halo is staged ONCE per 32-channel group as
-  // [Rin][P] padded pixels and every tap's A operand is a row-shifted view of it
   // A-operand addressing: TMA coordinate d (1..4) of tap t = base_d(tile) + tap_off[t][d-1]; `amode` picks which tile
   // variable feeds which tensor-map dimension (0: same-size conv, dims (c, x, view-x, y, image*view-y);
   // 1: stride along x, dims (c, x%s, x/s, y, image); 2: stride along y, dims (c, x, y%s, y/s, image);
@@ -84,7 +92,11 @@ struct Params {
   short tap_off[25][4];
   long long* dbg;                      // optional per-CTA cycle counters (profiles/ experiments), else null
   int dbg_skip_a;                      // experiment (wrong results): only tap 0 loads its activation tile
-  int halo, TWo, Rout, P, Rin, ntiles, strips_x, blocks_y, total_blocks, a_cg_bytes, bstages, acc_stages, pdiv_mul;
+  // halo-block CTA pairs (conv_tc_halo_kernel): blocks of Rout x TWo output pixels; a CTA stages its block's (Rout + 2) x P
+  // input pixels (P = TWo + 2) once and each tap's A operand is that buffer read from a row-shifted descriptor, so MMA row m of
+  // tile j is the flattened padded position g = 128 j + m = ty * P + tx (tx >= TWo: halo columns, never stored)
+  int TWo, Rout, P, Rin, ntiles, strips_x, blocks_y, total_blocks, a_buf_bytes, pdiv_mul;
+  FastDiv fd_strips, fd_blocks_y;
 };
 
 // ---- PTX wrappers ----------------------------------------------------------------------------
@@ -403,7 +415,7 @@ __device__ __forceinline__ float act_t(float v, float slope) {
 
 template <int V, bool HAS_MUL, bool HAS_RES>
 __device__ __forceinline__ void epi_writeout(const Params& p, const float* stg, int lane, int q, const TileCoord& tc_, int pc0,
-                                             int ncols, int tile_j) {
+                                             int ncols) {
   constexpr int LPR = 32 / V;   // lanes per pixel row
   // rows handled together. The loop is written in phases (coordinates, global loads, shared loads, math, stores), each
   // over all NB rows, so that NB independent memory operations are in flight: with two epilogue warps per scheduler
@@ -429,9 +441,9 @@ __device__ __forceinline__ void epi_writeout(const Params& p, const float* stg, 
   const int m_py = p.mul.w * p.mul.ld, m_px = p.mul.ld;
   const int o_py = p.ry * p.out.w * p.out.ld, o_px = p.rx * p.out.ld;         // float pitch per tile row / column
   const int r_py = p.ry * p.res.w * p.res.ld, r_px = p.rx * p.res.ld;
-  const bool full = !p.halo && tc_.y0 + p.TH <= p.bh && tc_.x0 + p.TW <= p.bw;
+  const bool full = tc_.y0 + p.TH <= p.bh && tc_.x0 + p.TW <= p.bw;
   const int tw_mask = p.TW - 1;
-  const int rows_valid = min(p.halo ? p.Rout : p.TH, p.bh - tc_.y0), cols_valid = min(p.halo ? p.TWo : p.TW, p.bw - tc_.x0);
+  const int rows_valid = min(p.TH, p.bh - tc_.y0), cols_valid = min(p.TW, p.bw - tc_.x0);
   const float slope = p.slope, alpha = p.alpha;
   const bool mul_silu = p.mul_act == LFSR_ACT_SILU;   // the one multiplier activation the networks use (checked on the host)
   const int swz_hi = col >> 2, swz_lo = col & 3;
@@ -442,14 +454,7 @@ __device__ __forceinline__ void epi_writeout(const Params& p, const float* stg, 
 #pragma unroll
     for (int j = 0; j < NB; ++j) {
       const int m = q * 32 + (it0 + j) * V + lrow;
-      int ty, tx;
-      if (p.halo) {                    // flattened padded position g = ty*P + tx (tx >= TWo are halo garbage)
-        const int g = tile_j * 128 + m;
-        ty = (g * p.pdiv_mul) >> 16;
-        tx = g - ty * p.P;
-      } else {
-        ty = m >> p.tw_shift; tx = m & tw_mask;
-      }
+      const int ty = m >> p.tw_shift, tx = m & tw_mask;
       tyx[j] = (full || (ty < rows_valid && tx < cols_valid)) ? ((ty << 16) | tx) : -1;
     }
     // residual / multiplier operands first (longest latency). The stores below may alias `res` (in-place residuals),
@@ -536,17 +541,17 @@ __device__ __forceinline__ void epi_writeout(const Params& p, const float* stg, 
 
 template <int V>
 __device__ __forceinline__ void epi_writeout_act(const Params& p, const float* stg, int lane, int q, const TileCoord& tc_,
-                                                 int pc0, int ncols, int tile_j) {
+                                                 int pc0, int ncols) {
   const bool m = p.mul.p != nullptr, r = p.res.p != nullptr;
-  if (m && r) epi_writeout<V, true, true>(p, stg, lane, q, tc_, pc0, ncols, tile_j);
-  else if (m) epi_writeout<V, true, false>(p, stg, lane, q, tc_, pc0, ncols, tile_j);
-  else if (r) epi_writeout<V, false, true>(p, stg, lane, q, tc_, pc0, ncols, tile_j);
-  else epi_writeout<V, false, false>(p, stg, lane, q, tc_, pc0, ncols, tile_j);
+  if (m && r) epi_writeout<V, true, true>(p, stg, lane, q, tc_, pc0, ncols);
+  else if (m) epi_writeout<V, true, false>(p, stg, lane, q, tc_, pc0, ncols);
+  else if (r) epi_writeout<V, false, true>(p, stg, lane, q, tc_, pc0, ncols);
+  else epi_writeout<V, false, false>(p, stg, lane, q, tc_, pc0, ncols);
 }
 
 // TMEM accumulator (32 lanes x NC columns of this warp) -> staged transpose -> coalesced global stores
 __device__ __forceinline__ void epilogue_tile(const Params& p, float* stg, uint32_t taddr, int lane, int q, const TileCoord& tc_,
-                                              int tile_j, int g_first = 0, int g_step = 1, long long* dbg_ld = nullptr) {
+                                              int g_first = 0, int g_step = 1, long long* dbg_ld = nullptr) {
   for (int g = g_first; g * 32 < p.NC; g += g_step) {
     const int ncols = p.NC - g * 32 < 32 ? p.NC - g * 32 : 32;
     float v[32];
@@ -562,9 +567,9 @@ __device__ __forceinline__ void epilogue_tile(const Params& p, float* stg, uint3
     __syncwarp();
     if (dbg_ld) *dbg_ld += clock64() - t0;
     const int pc0 = tc_.chunk * p.NC + g * 32;
-    if (p.vec == 4) epi_writeout_act<4>(p, stg, lane, q, tc_, pc0, ncols, tile_j);
-    else if (p.vec == 2) epi_writeout_act<2>(p, stg, lane, q, tc_, pc0, ncols, tile_j);
-    else epi_writeout_act<1>(p, stg, lane, q, tc_, pc0, ncols, tile_j);
+    if (p.vec == 4) epi_writeout_act<4>(p, stg, lane, q, tc_, pc0, ncols);
+    else if (p.vec == 2) epi_writeout_act<2>(p, stg, lane, q, tc_, pc0, ncols);
+    else epi_writeout_act<1>(p, stg, lane, q, tc_, pc0, ncols);
     __syncwarp();
   }
 }
@@ -728,9 +733,9 @@ __device__ __forceinline__ void epilogue_tile_tma(const Params& p, const CUtenso
       }
     } else {
       __syncwarp();
-      if (p.vec == 4) epi_writeout_act<4>(p, stg, lane, q, tc_, pc0, ncols, 0);
-      else if (p.vec == 2) epi_writeout_act<2>(p, stg, lane, q, tc_, pc0, ncols, 0);
-      else epi_writeout_act<1>(p, stg, lane, q, tc_, pc0, ncols, 0);
+      if (p.vec == 4) epi_writeout_act<4>(p, stg, lane, q, tc_, pc0, ncols);
+      else if (p.vec == 2) epi_writeout_act<2>(p, stg, lane, q, tc_, pc0, ncols);
+      else epi_writeout_act<1>(p, stg, lane, q, tc_, pc0, ncols);
       __syncwarp();
     }
     LFSR_EPI_TICK(6)
@@ -741,30 +746,28 @@ __device__ __forceinline__ void epilogue_tile_tma(const Params& p, const CUtenso
 
 // Epilogue of one tile for one warp when the layer ends in a tail projection (Params::tail_w): the warp owns whole
 // PixelShuffle sub-pixels (alternating with its partner warp), a lane owns one pixel, and instead of storing the cq
-// activated channels of that output pixel it accumulates their dot products with the <= 12 tail vectors (weights
-// broadcast from shared memory) and stores those 12 floats - 48 bytes instead of 4*cq per output pixel.
-__device__ __forceinline__ void epilogue_tile_tail(const Params& p, const float* sTail, uint32_t taddr, int lane, int q,
-                                                   const TileCoord& tc_, int g_first, int g_step, uint64_t* tfull_bar,
-                                                   uint32_t tfull_parity) {
-  const int m = q * 32 + lane;
-  const int ty = m >> p.tw_shift, tx = m & (p.TW - 1);
-  const bool pix_ok = tc_.y0 + ty < p.bh && tc_.x0 + tx < p.bw;
-  const int img = fdiv(tc_.nb, p.fd_nby);
-  const int Y = (tc_.nb - img * p.nby) * p.bh + tc_.y0 + ty, X = tc_.vx * p.bw + tc_.x0 + tx;
+// activated channels of that output pixel it accumulates their dot products with the <= 12 tail vectors (weights from the
+// constant bank in the 16-warp kernels, else broadcast from shared memory) and stores those 12 floats - 48 bytes instead
+// of 4*cq per output pixel.
+// The projection of one pixel per lane (conv-output pixel (Y, X) of image img) for sub-pixels sub0 + g_first, + g_step, ...
+// below sub1; taddr addresses accumulator column sub0 * cq. Shared by the per-tap and the halo-block kernels.
+// CW: `tw` is the __grid_constant__ table (cq <= kTailMaxC; both 32-channel blocks unrolled so that every weight offset is
+// a compile-time constant), else the zero-padded copy in shared memory.
+template <bool CW>
+__device__ __forceinline__ void tail_project(const Params& p, const float* tw, uint32_t taddr, int lane, int img, int Y, int X,
+                                             bool pix_ok, int sub0, int sub1, int g_first, int g_step) {
   const int r2 = p.ry * p.rx;
   const bool chan_major = p.shuf_mode == LFSR_SHUF_CHANNEL_MAJOR;
   const float slope = p.slope;
-  mbar_wait(tfull_bar, tfull_parity);
-  tc_fence_after();
-  // sub-pixels of this cout-chunk: all of them with one chunk, else NC / cq whole sub-pixels per chunk (host-checked)
-  const int sub0 = p.nchunks == 1 ? 0 : tc_.chunk * (p.NC / p.cq);
-  const int sub1 = p.nchunks == 1 ? r2 : min(r2, sub0 + p.NC / p.cq);
   taddr -= sub0 * p.cq;                            // accumulator column of global output column pc0 is pc0 - sub0 * cq
   for (int sub = sub0 + g_first; sub < sub1; sub += g_step) {
     f32x2 rp[6];                      // 12 tap responses as 6 packed pairs: the projection is FFMA2 throughout
 #pragma unroll
     for (int t = 0; t < 6; ++t) rp[t] = pack2(0.f, 0.f);
-    for (int c0 = 0; c0 < p.cq; c0 += 32) {
+#pragma unroll
+    for (int cb = 0; cb < (CW ? kTailMaxC / 32 : 1 << 20); ++cb) {
+      const int c0 = cb * 32;
+      if (c0 >= p.cq) break;
       const int pc0 = sub * p.cq + c0;
       float bcol = 0.f;
       if (p.bias && c0 + lane < p.cq) bcol = __ldg(p.bias + (chan_major ? (c0 + lane) * r2 + sub : pc0 + lane));
@@ -793,15 +796,13 @@ __device__ __forceinline__ void epilogue_tile_tail(const Params& p, const float*
         for (int k = 0; k < 32; ++k)
           if (c0 + k >= p.cq) v[k] = 0.f;
       }
-      const float4* wt = reinterpret_cast<const float4*>(sTail + c0 * 12);
+      const float* wt = tw + c0 * 12;
 #pragma unroll
       for (int k = 0; k < 32; ++k) {
-        const float4 w0 = wt[3 * k], w1 = wt[3 * k + 1], w2 = wt[3 * k + 2];
         const float a = v[k] * p.alpha;
         const f32x2 aa = pack2(a, a);
-        rp[0] = fma2(aa, pack2(w0.x, w0.y), rp[0]); rp[1] = fma2(aa, pack2(w0.z, w0.w), rp[1]);
-        rp[2] = fma2(aa, pack2(w1.x, w1.y), rp[2]); rp[3] = fma2(aa, pack2(w1.z, w1.w), rp[3]);
-        rp[4] = fma2(aa, pack2(w2.x, w2.y), rp[4]); rp[5] = fma2(aa, pack2(w2.z, w2.w), rp[5]);
+#pragma unroll
+        for (int t = 0; t < 6; ++t) rp[t] = fma2(aa, pack2(wt[12 * k + 2 * t], wt[12 * k + 2 * t + 1]), rp[t]);
       }
     }
     if (pix_ok) {
@@ -817,6 +818,27 @@ __device__ __forceinline__ void epilogue_tile_tail(const Params& p, const float*
   }
 }
 
+template <bool CW>
+__device__ __forceinline__ void epilogue_tile_tail(const Params& p, const float* tw, uint32_t taddr, int lane, int q,
+                                                   const TileCoord& tc_, int g_first, int g_step, uint64_t* tfull_bar,
+                                                   uint32_t tfull_parity) {
+  const int m = q * 32 + lane;
+  const int ty = m >> p.tw_shift, tx = m & (p.TW - 1);
+  const bool pix_ok = tc_.y0 + ty < p.bh && tc_.x0 + tx < p.bw;
+  const int img = fdiv(tc_.nb, p.fd_nby);
+  const int Y = (tc_.nb - img * p.nby) * p.bh + tc_.y0 + ty, X = tc_.vx * p.bw + tc_.x0 + tx;
+  mbar_wait(tfull_bar, tfull_parity);
+  tc_fence_after();
+  // sub-pixels of this cout-chunk: all of them with one chunk, else NC / cq whole sub-pixels per chunk (host-checked)
+  const int r2 = p.ry * p.rx;
+  const int sub0 = p.nchunks == 1 ? 0 : tc_.chunk * (p.NC / p.cq);
+  const int sub1 = p.nchunks == 1 ? r2 : min(r2, sub0 + p.NC / p.cq);
+  tail_project<CW>(p, tw, taddr, lane, img, Y, X, pix_ok, sub0, sub1, g_first, g_step);
+}
+
+__device__ __forceinline__ const float* tail_w_of(const TailW& tw, const float*) { return tw.w; }
+__device__ __forceinline__ const float* tail_w_of(const NoTailW&, const float* sTail) { return sTail; }
+
 // (register files are allocated for 4-warp groups: 320 threads cost what 384 do, i.e. at most 168 registers each)
 // CTA2 = true is a separate instantiation: a kernel that contains cta_group::2 instructions can only be launched in
 // clusters of two, so the single-CTA paths must not see them
@@ -829,7 +851,8 @@ __device__ __forceinline__ void epilogue_tile_tail(const Params& p, const float*
 template <bool CTA2, bool DBG, bool F16, bool T16 = false>
 __global__ void __launch_bounds__(T16 ? 640 : kThreads, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-               const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmO, const Params p) {
+               const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmO, const Params p,
+               const __grid_constant__ TailArg<T16> tw) {
   constexpr int CG = F16 ? 64 : 32;            // channels per 128-byte row / channel group
   constexpr int kEpiW = T16 ? 16 : kEpiWarps;  // epilogue warps; the TMA producer and the MMA issuer are the two warps after them
   constexpr int kTmaWarp = kEpiW, kMmaWarp = kEpiW + 1;
@@ -853,7 +876,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
-  for (int i = threadIdx.x; i < p.tail_rows * 12; i += (int)blockDim.x) sTail[i] = i < p.cq * 12 ? __ldg(p.tail_w + i) : 0.f;
+  if (!T16)
+    for (int i = threadIdx.x; i < p.tail_rows * 12; i += (int)blockDim.x) sTail[i] = i < p.cq * 12 ? __ldg(p.tail_w + i) : 0.f;
   if (threadIdx.x == 0) {
     for (int s = 0; s < p.stages; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, p.pair ? 2 : 1); }
     for (int a = 0; a < 2; ++a) { mbar_init(tfull + a, 1); mbar_init(tempty + a, CTA2 ? 2 * kEpiW : kEpiW); }
@@ -1140,10 +1164,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + a * kAccStride;
       long long tw1 = 0;
       if (T16) {
-        if (m_ >= 0) epilogue_tile_tail(p, sTail, taddr, lane, q, tc_, half, 4, tfull + a, aph);
+        if (m_ >= 0) epilogue_tile_tail<T16>(p, tail_w_of(tw, sTail), taddr, lane, q, tc_, half, 4, tfull + a, aph);
         else { mbar_wait(tfull + a, aph); tc_fence_after(); }
       } else if (p.tail_w && m_ >= 0) {
-        epilogue_tile_tail(p, sTail, taddr, lane, q, tc_, half, 2, tfull + a, aph);
+        epilogue_tile_tail<false>(p, sTail, taddr, lane, q, tc_, half, 2, tfull + a, aph);
       } else if (p.tma_epi && m_ >= 0) {
         if ((DBG && p.dbg)) tw1 = clock64();
         epilogue_tile_tma(p, &tmO, stg, taddr, lane, q, tc_, half, 2, tfull + a, aph, (DBG && p.dbg) ? dbg_seg : nullptr);
@@ -1154,7 +1178,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         if ((DBG && p.dbg)) dbg_wait += clock64() - tw0;
         tc_fence_after();
         if ((DBG && p.dbg)) tw1 = clock64();
-        if (m_ >= 0) epilogue_tile(p, stg, taddr, lane, q, tc_, 0, half, 2, (DBG && p.dbg) ? &dbg_ld : nullptr);
+        if (m_ >= 0) epilogue_tile(p, stg, taddr, lane, q, tc_, half, 2, (DBG && p.dbg) ? &dbg_ld : nullptr);
         if ((DBG && p.dbg)) dbg_epi += clock64() - tw1;
       }
       tc_fence_before();
@@ -1413,162 +1437,238 @@ conv_tc_lean_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   }
 }
 
-// ======================= halo-block kernel =======================================================
-// 7 warps: 0 = A (activation block) producer, 1 = MMA issuer, 2..5 = epilogue, 6 = B (weights) producer.
-constexpr int kHaloThreads = 224;
+// ======================= halo-block CTA-pair kernel: fp16 3x3 "same" convs with 128 < N <= 256 ===========================
+// The per-tap kernel stages a 16 KB activation tile and a half weight slice per tap: ~270 KB written to shared memory per
+// 128-pixel tile, which (with the MMA operand reads) is what bounds the upsampler convs. Here each CTA of a pair
+//   * keeps ITS HALF of all 9 taps' weights resident (loaded once),
+//   * stages its block's haloed input ONCE per block: one TMA box of (Rout + 2) x P pixels x 64 fp16 channels, out-of-image
+//     pixels zero-filled (the conv padding); tap (ky, kx) of MMA tile j reads that buffer from the descriptor start row
+//     128 j + ky P + kx (SWIZZLE_128B is a function of the absolute address, so any 128-byte row works as a start),
+//   * runs tcgen05.mma.cta_group::2 (M = 256: 128 rows from each CTA's own block at the same offsets), taps and K-steps in
+//     the per-tap kernel's order, so every fp32 sum is the same,
+// with two input buffers and two TMEM accumulator stages, and 16 epilogue warps (four per TMEM lane quarter, each owning
+// whole PixelShuffle sub-pixels / column blocks). TAIL: the layer ends in the head-conv tap projection (epilogue of the
+// T16 kernel), else it writes its fp16 output only.
+constexpr int kHaloEpiW = 16;
+constexpr int kHaloThreads = (kHaloEpiW + 2) * 32;
 
-struct BlockCoord { int nb, y0, vx, x0; };
+struct BlockCoord { int img, y0, x0; };
+// cluster c walks block pairs c, c + clusters, ...; rank r of the pair owns block 2 * pair + r (an odd tail: a dummy block
+// that loads valid data and stores nothing, so both CTAs step through the same barrier phases)
+__device__ __forceinline__ bool next_block(const Params& p, int i, int& b) {
+  const int pr = (int)(blockIdx.x >> 1) + i * (int)(gridDim.x >> 1);
+  if (2 * pr >= p.total_blocks) return false;
+  b = 2 * pr + (int)(blockIdx.x & 1);
+  if (b >= p.total_blocks) b = -1;
+  return true;
+}
 __device__ __forceinline__ BlockCoord decode_block(const Params& p, int b) {
+  if (b < 0) b = p.total_blocks - 1;
   BlockCoord c;
-  c.x0 = (b % p.strips_x) * p.TWo; b /= p.strips_x;
-  c.vx = b % p.nbx; b /= p.nbx;
-  c.y0 = (b % p.blocks_y) * p.Rout;
-  c.nb = b / p.blocks_y;
+  const int u = fdiv(b, p.fd_strips);
+  c.x0 = (b - u * p.strips_x) * p.TWo;
+  c.img = fdiv(u, p.fd_blocks_y);
+  c.y0 = (u - c.img * p.blocks_y) * p.Rout;
   return c;
 }
 
-__global__ void __launch_bounds__(kHaloThreads, 1)
-conv_tc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const Params p) {
+// fp16-only write-out of one pixel per lane (what epilogue_tile_tma does with out_mode 2 and no residual / multiplier):
+// column blocks of <= 32 packed channels that never straddle a sub-pixel run, g_first, + g_step, ... of them
+__device__ __forceinline__ void halo_store_f16(const Params& p, uint32_t taddr, int lane, int img, int Y, int X, bool pix_ok,
+                                               int g_first, int g_step) {
+  const int r2 = p.ry * p.rx;
+  const bool chan_major = r2 > 1 && p.shuf_mode == LFSR_SHUF_CHANNEL_MAJOR;
+  const float slope = p.slope, alpha = p.alpha;
+  int bi = 0;
+  for (int pc0 = 0, ncols = 0; pc0 < p.cout; pc0 += ncols, ++bi) {
+    int sub = 0, c0 = pc0;
+    if (r2 > 1) { sub = fdiv(pc0, p.fd_cq); c0 = pc0 - sub * p.cq; }
+    ncols = p.cq - c0 < 32 ? p.cq - c0 : 32;
+    if (p.cout - pc0 < ncols) ncols = p.cout - pc0;
+    if (bi % g_step != g_first) continue;
+    float bcol = 0.f;
+    if (p.bias) {
+      const int pcl = pc0 + lane;
+      if (pcl < p.cout) {
+        int bidx = pcl;
+        if (chan_major) { const int s_ = fdiv(pcl, p.fd_cq); bidx = (pcl - s_ * p.cq) * r2 + s_; }
+        bcol = __ldg(p.bias + bidx);
+      }
+    }
+    float v[32];
+    tmem_ld16(taddr + pc0, v);
+    if (ncols > 16) tmem_ld16(taddr + pc0 + 16, v + 16);
+    else {
+#pragma unroll
+      for (int k = 16; k < 32; ++k) v[k] = 0.f;
+    }
+    if (p.bias) {
+#pragma unroll
+      for (int k = 0; k < 32; ++k) v[k] += __shfl_sync(0xffffffffu, bcol, k);
+    }
+#define LFSR_EPI_ACT32(A) _Pragma("unroll") for (int k = 0; k < 32; ++k) v[k] = act_t<A>(v[k], slope);
+    switch (p.act) {
+      case LFSR_ACT_RELU: LFSR_EPI_ACT32(LFSR_ACT_RELU) break;
+      case LFSR_ACT_LRELU: LFSR_EPI_ACT32(LFSR_ACT_LRELU) break;
+      case LFSR_ACT_SIGMOID: LFSR_EPI_ACT32(LFSR_ACT_SIGMOID) break;
+      case LFSR_ACT_GELU: LFSR_EPI_ACT32(LFSR_ACT_GELU) break;
+      case LFSR_ACT_SILU: LFSR_EPI_ACT32(LFSR_ACT_SILU) break;
+      default: break;
+    }
+#undef LFSR_EPI_ACT32
+#pragma unroll
+    for (int k = 0; k < 32; ++k) v[k] = fmaf(v[k], alpha, 0.f);      // (as the per-tap epilogue rounds it: alpha * v + 0)
+    if (pix_ok) {
+      int Yo = Y, Xo = X;
+      if (r2 > 1) { const int si = fdiv(sub, p.fd_rx), sj = sub - si * p.rx; Yo = Y * p.ry + si; Xo = X * p.rx + sj; }
+      __half* dst = p.out16 + ((size_t)((size_t)img * p.out16_h + Yo) * p.out16_w + Xo) * (size_t)p.out16_ld + c0;
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+        if (8 * j < ncols)
+          *reinterpret_cast<uint4*>(dst + 8 * j) =
+              make_uint4(pack_h2(v[8 * j], v[8 * j + 1]), pack_h2(v[8 * j + 2], v[8 * j + 3]), pack_h2(v[8 * j + 4], v[8 * j + 5]),
+                         pack_h2(v[8 * j + 6], v[8 * j + 7]));
+    }
+  }
+}
+
+// (register files are allocated per 4-warp group: the bound is stated for 20 warps so that ptxas budgets what 18 cost)
+template <bool TAIL>
+__global__ void __launch_bounds__(640, 1)
+conv_tc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmBh, const Params p,
+                    const __grid_constant__ TailArg<TAIL> tw) {
+  constexpr int kTmaW = kHaloEpiW, kMmaW = kHaloEpiW + 1;
+  constexpr int kTaps = 9;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
   uint8_t* smem = smem_raw + (((raw + 1023u) & ~1023u) - raw);
-  const int taps = p.kh * p.kw;
-  const int nks = taps * p.cgs;
-  uint8_t* sA = smem;                                   // cgs x a_cg_bytes
-  uint8_t* sB = sA + p.cgs * p.a_cg_bytes;              // resident: nks stages, else bstages
-  float* sEpi = reinterpret_cast<float*>(sB + (p.resident ? nks : p.bstages) * p.b_stage_bytes);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sEpi + 4 * 1024);
-  uint64_t* afull = bars;            // [2]
-  uint64_t* aempty = bars + 2;       // [2]
-  uint64_t* bfull = bars + 4;        // [kMaxStages]
-  uint64_t* bempty = bfull + kMaxStages;
-  uint64_t* tfull = bempty + kMaxStages;   // [2]
-  uint64_t* tempty = tfull + 2;            // [2]
-  uint64_t* bres = tempty + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bres + 1);
+  const uint32_t half_bytes = (uint32_t)(p.NC >> 1) * 128u;      // this CTA's rows of one tap's weight slice
+  uint8_t* sA = smem;                                              // 2 x a_buf_bytes
+  uint8_t* sB = sA + 2 * p.a_buf_bytes;                            // kTaps x half_bytes
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sB + kTaps * half_bytes);
+  uint64_t* afull = bars;
+  uint64_t* aempty = bars + 2;
+  uint64_t* tfull = bars + 4;
+  uint64_t* tempty = bars + 6;
+  uint64_t* bfull = bars + 8;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 9);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   if (threadIdx.x == 0) {
-    for (int c = 0; c < 2; ++c) { mbar_init(afull + c, 1); mbar_init(aempty + c, 1); }
-    for (int s_ = 0; s_ < kMaxStages; ++s_) { mbar_init(bfull + s_, 1); mbar_init(bempty + s_, 1); }
-    for (int a = 0; a < 2; ++a) { mbar_init(tfull + a, 1); mbar_init(tempty + a, 4); }
-    mbar_init(bres, 1);
+    for (int k = 0; k < 2; ++k) {
+      mbar_init(afull + k, 1); mbar_init(aempty + k, 1);
+      mbar_init(tfull + k, 1); mbar_init(tempty + k, 2 * kHaloEpiW);
+    }
+    mbar_init(bfull, 1);
     fence_barrier_init();
     tma_prefetch_desc(&tmA);
-    tma_prefetch_desc(&tmB);
+    tma_prefetch_desc(&tmBh);
   }
-  if (warp == 1) tmem_alloc(tmem_slot, kTmemCols);
+  cluster_sync_all();                           // both CTAs are resident before the paired allocation is requested
+  if (warp == kMmaW) tmem_alloc2(tmem_slot, kTmemCols);
   tc_fence_before();
   __syncthreads();
+  cluster_sync_all();                           // the partner's barriers are initialised before anything signals them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  const bool has_work = (int)blockIdx.x < p.total_blocks;
+  const uint32_t crank = cluster_ctarank();
 
-  if (warp == 0) {
-    // ---- A producer: one TMA box per (block, 32-channel group): [Rin][P] padded pixels
-    const uint32_t a_bytes = (uint32_t)p.Rin * p.P * 128;
-    int i = 0;
-    for (int b = blockIdx.x; b < p.total_blocks; b += gridDim.x, ++i) {
-      const BlockCoord bc = decode_block(p, b);
-      for (int cg = 0; cg < p.cgs; ++cg) {
-        mbar_wait(aempty + cg, (i & 1) ^ 1);
-        if (lane == 0) {
-          mbar_expect_tx(afull + cg, a_bytes);
-          tma_load_5d(sA + cg * p.a_cg_bytes, &tmA, afull + cg, cg * 32, bc.x0 - p.pad_w, bc.vx, bc.y0 - p.pad_h, bc.nb);
-        }
-        __syncwarp();
+  if (warp == kTmaW) {
+    // ---- TMA producer (both CTAs): the weight halves once, then one haloed input box per block; all transaction bytes
+    // land on the leader's barriers, whose MMAs read both CTAs' buffers
+    if (elect_one()) {
+      if (crank == 0) mbar_expect_tx(bfull, 2u * kTaps * half_bytes);
+      for (int t = 0; t < kTaps; ++t)
+        tma_load_2d_2sm(sB + t * half_bytes, &tmBh, bfull, 0, t * p.NC + (int)crank * (p.NC >> 1));
+      const uint32_t box_bytes = (uint32_t)(p.Rin * p.P * 128);
+      int b;
+      for (int i = 0; next_block(p, i, b); ++i) {
+        const int buf = i & 1;
+        mbar_wait(aempty + buf, ((i >> 1) & 1) ^ 1);      // own barrier: the leader's commit arrives in both CTAs
+        if (crank == 0) mbar_expect_tx(afull + buf, 2u * box_bytes);
+        const BlockCoord bc = decode_block(p, b);
+        tma_load_5d_2sm(sA + buf * p.a_buf_bytes, &tmA, afull + buf, 0, bc.x0 - 1, 0, bc.y0 - 1, bc.img);
       }
     }
-  } else if (warp == 6) {
-    // ---- B producer: weights of K-stage (cg, tap); resident mode loads all of them once
-    if (p.resident) {
-      if (lane == 0 && has_work) {
-        mbar_expect_tx(bres, (uint32_t)nks * p.b_stage_bytes);
-        for (int ks = 0; ks < nks; ++ks) tma_load_2d(sB + ks * p.b_stage_bytes, &tmB, bres, 0, ks * p.NC);
-      }
-    } else {
-      uint32_t it = 0;
-      for (int b = blockIdx.x; b < p.total_blocks; b += gridDim.x) {
-        for (int cg = 0; cg < p.cgs; ++cg)
-          for (int tap = 0; tap < taps; ++tap, ++it) {
-            const int s_ = it % p.bstages;
-            mbar_wait(bempty + s_, ((it / p.bstages) & 1) ^ 1);
-            if (lane == 0) {
-              mbar_expect_tx(bfull + s_, (uint32_t)p.b_stage_bytes);
-              tma_load_2d(sB + s_ * p.b_stage_bytes, &tmB, bfull + s_, 0, (tap * p.cgs + cg) * p.NC);
-            }
-            __syncwarp();
-          }
-      }
-    }
-  } else if (warp == 1) {
-    // ---- MMA issuer
-    const uint32_t idesc = make_idesc(p.NC);
-    if (p.resident && has_work) mbar_wait(bres, 0);
-    uint32_t it = 0;
-    int b_ring = 0;
-    uint32_t b_ph = 0;
-    const uint64_t b_desc0 = make_smem_desc(smem_u32(sB));
-    int i = 0;
-    for (int b = blockIdx.x; b < p.total_blocks; b += gridDim.x, ++i) {
-      const uint32_t a = p.acc_stages == 2 ? (i & 1) : 0;
-      const uint32_t aph = p.acc_stages == 2 ? ((i >> 1) & 1) : (i & 1);
-      mbar_wait(tempty + a, aph ^ 1);
-      tc_fence_after();
-      const uint32_t d_base = tmem_base + a * (p.ntiles * p.NC);
-      for (int cg = 0; cg < p.cgs; ++cg) {
-        mbar_wait(afull + cg, i & 1);
+    __syncwarp();
+  } else if (warp == kMmaW) {
+    // ---- MMA issuer: the leader's elected lane issues M = 256 for the pair; the partner's MMA warp idles
+    if (crank == 0) {
+      if (elect_one()) {
+        const uint32_t idesc2 = (make_idesc(p.NC, 0u) & ~(0x1fu << 24)) | ((uint32_t)(256 >> 4) << 24);
+        const uint64_t a_desc0 = make_smem_desc(smem_u32(sA)), b_desc0 = make_smem_desc(smem_u32(sB));
+        const uint32_t row_p = (uint32_t)p.P * 8u;                 // one padded input row (P pixels x 128 B), 16-byte units
+        const uint32_t b_tap = half_bytes >> 4;
+        const int ksteps = p.C >= 64 ? 4 : (p.C + 15) >> 4;
+        mbar_wait(bfull, 0);
         tc_fence_after();
-        const int rem = p.C - cg * 32;
-        const int ksteps = rem >= 32 ? 4 : (rem + 7) >> 3;
-        const uint64_t a_cg_desc = make_smem_desc(smem_u32(sA + cg * p.a_cg_bytes));
-        int ky = 0, kx = 0;
-        for (int tap = 0; tap < taps; ++tap, ++it) {
-          if (b_ring == p.bstages) { b_ring = 0; b_ph ^= 1; }
-          const int s_ = p.resident ? (tap * p.cgs + cg) : b_ring++;
-          if (!p.resident) { mbar_wait(bfull + s_, b_ph); tc_fence_after(); }
-          if (lane == 0) {
-            const uint64_t a_d = a_cg_desc + (uint64_t)((ky * p.dil_h * p.P + kx * p.dil_w) * 8);      // rows * 128 B >> 4
-            const uint64_t b_d = b_desc0 + (uint64_t)(s_ * (p.b_stage_bytes >> 4));
-            for (int j = 0; j < p.ntiles; ++j) {
-              if ((cg | tap) == 0) umma_stage<true>(d_base + j * p.NC, a_d + (uint64_t)(j * 1024), b_d, idesc, ksteps);
-              else umma_stage<false>(d_base + j * p.NC, a_d + (uint64_t)(j * 1024), b_d, idesc, ksteps);
+        uint32_t tcount = 0;
+        int b;
+        for (int i = 0; next_block(p, i, b); ++i) {
+          const int buf = i & 1;
+          mbar_wait(afull + buf, (i >> 1) & 1);
+          tc_fence_after();
+          const uint64_t a_blk = a_desc0 + (uint64_t)buf * (uint64_t)(p.a_buf_bytes >> 4);
+          for (int j = 0; j < p.ntiles; ++j, ++tcount) {
+            const uint32_t a = tcount & 1;
+            mbar_wait(tempty + a, ((tcount >> 1) & 1) ^ 1);          // both CTAs' epilogues have drained this stage
+            tc_fence_after();
+            const uint32_t d_tmem = tmem_base + a * kAccStride;
+            const uint64_t a_tile = a_blk + (uint64_t)(j * 1024);   // 128 rows x 128 B
+            uint64_t b_d = b_desc0;
+#pragma unroll
+            for (int ky = 0; ky < 3; ++ky) {
+#pragma unroll
+              for (int kx = 0; kx < 3; ++kx) {
+                const uint64_t a_d = a_tile + (uint64_t)(ky * row_p + kx * 8);
+                if (ky == 0 && kx == 0) umma2_tf32_c<0, true>(d_tmem, a_d, b_d, idesc2);
+                else umma2_tf32_c<1, true>(d_tmem, a_d, b_d, idesc2);
+                if (ksteps == 4) {
+                  umma2_tf32_c<1, true>(d_tmem, a_d + 2, b_d + 2, idesc2);
+                  umma2_tf32_c<1, true>(d_tmem, a_d + 4, b_d + 4, idesc2);
+                  umma2_tf32_c<1, true>(d_tmem, a_d + 6, b_d + 6, idesc2);
+                } else {
+                  for (int k = 1; k < ksteps; ++k) umma2_tf32_c<1, true>(d_tmem, a_d + 2 * k, b_d + 2 * k, idesc2);
+                }
+                b_d += b_tap;
+              }
             }
-            if (!p.resident) umma_commit(bempty + s_);
-            if (tap == taps - 1) umma_commit(aempty + cg);       // this group's block may be overwritten
-            if (tap == taps - 1 && cg == p.cgs - 1) umma_commit(tfull + a);
+            umma2_commit_mc(tfull + a);              // accumulator complete -> both CTAs' epilogues
           }
-          if (++kx == p.kw) { kx = 0; ++ky; }
-          __syncwarp();
+          umma2_commit_mc(aempty + buf);             // both CTAs' input buffers may be refilled
         }
       }
+      __syncwarp();
     }
   } else {
-    // ---- epilogue warps 2..5
-    const int q = warp & 3;
-    float* stg = sEpi + (warp - 2) * 1024;
-    int i = 0;
-    for (int b = blockIdx.x; b < p.total_blocks; b += gridDim.x, ++i) {
-      const uint32_t a = p.acc_stages == 2 ? (i & 1) : 0;
-      const uint32_t aph = p.acc_stages == 2 ? ((i >> 1) & 1) : (i & 1);
+    // ---- epilogue: warp w <-> TMEM lane quarter w & 3; the four warps of a quarter take alternate sub-pixels / blocks ----
+    const int q = warp & 3, grp = warp >> 2;
+    uint32_t tcount = 0;
+    int b;
+    for (int i = 0; next_block(p, i, b); ++i) {
       const BlockCoord bc = decode_block(p, b);
-      TileCoord tc_;
-      tc_.chunk = 0; tc_.nb = bc.nb; tc_.y0 = bc.y0; tc_.vx = bc.vx; tc_.x0 = bc.x0;
-      mbar_wait(tfull + a, aph);
-      tc_fence_after();
-      for (int j = 0; j < p.ntiles; ++j) {
-        const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + a * (p.ntiles * p.NC) + j * p.NC;
-        epilogue_tile(p, stg, taddr, lane, q, tc_, j);
+      for (int j = 0; j < p.ntiles; ++j, ++tcount) {
+        const uint32_t a = tcount & 1;
+        const int g = j * 128 + q * 32 + lane;                     // flattened padded position of the lane's MMA row
+        const int ty = (g * p.pdiv_mul) >> 16, tx = g - ty * p.P;
+        const int Y = bc.y0 + ty, X = bc.x0 + tx;
+        const bool pix_ok = b >= 0 && ty < p.Rout && tx < p.TWo && Y < p.bh && X < p.bw;
+        const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + a * kAccStride;
+        mbar_wait(tfull + a, (tcount >> 1) & 1);
+        tc_fence_after();
+        if (TAIL) tail_project<true>(p, tail_w_of(tw, nullptr), taddr, lane, bc.img, Y, X, pix_ok, 0, p.ry * p.rx, grp, 4);
+        else halo_store_f16(p, taddr, lane, bc.img, Y, X, pix_ok, grp, 4);
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive_leader(tempty + a);
       }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(tempty + a);
     }
   }
   __syncthreads();
-  if (warp == 1) {
+  cluster_sync_all();                           // no CTA may exit while its partner can still signal it
+  if (warp == kMmaW) {
     __syncwarp();
-    tmem_dealloc(tmem_base, kTmemCols);
+    tmem_dealloc2(tmem_base, kTmemCols);
   }
 }
 
@@ -1613,11 +1713,63 @@ static float round_tf32(float x) {
   return y;
 }
 
+// Block geometry of conv_tc_halo_kernel for an H x W image: output blocks of Rout x TWo pixels, flattened over padded rows of
+// P = TWo + 2 into ntiles MMA tiles of 128 rows. Chosen to maximise the share of MMA rows that are output pixels (halo
+// columns, the unused tail of the last tile and the blocks that overhang the image are the waste), then to minimise the
+// input rows staged per output pixel. Shared memory: two input buffers (each must also cover the rows the last tile's
+// bottom-right tap reads: 128 ntiles + 2 P + 2) and the resident weight halves of 9 taps.
+struct HaloGeom { int TWo, Rout, P, Rin, ntiles, strips_x, blocks_y, a_buf_bytes, smem, pdiv_mul; };
+constexpr int kHaloSmemMax = 227 * 1024;
+static int halo_smem_bytes(int a_buf_bytes, int NC) { return 1024 + 2 * a_buf_bytes + 9 * (NC / 2) * 128 + 9 * 8 + 16; }
+static bool plan_halo(int H, int W, int NC, HaloGeom& g) {
+  if (H < 1 || W < 1 || NC < 16 || NC > 256 || NC % 16) return false;
+  double best = 0.0, best_rows = 1e30;
+  bool found = false;
+  for (int nt = 1; nt <= 3; ++nt)
+    for (int two = W < 254 ? W : 254; two >= 1; --two) {
+      const int P = two + 2;
+      int rout = nt * 128 / P;
+      if (rout > H) rout = H;
+      if (rout > 254) rout = 254;
+      if (rout < 1 || rout * P <= (nt - 1) * 128) continue;       // a tile that holds no block position
+      const int rin = rout + 2;
+      const int rows = rin * P > nt * 128 + 2 * P + 2 ? rin * P : nt * 128 + 2 * P + 2;
+      const int a_buf = (rows * 128 + 1023) / 1024 * 1024;
+      if (halo_smem_bytes(a_buf, NC) > kHaloSmemMax) continue;
+      const int sx = (W + two - 1) / two, by = (H + rout - 1) / rout;
+      const double eff = (double)H * W / ((double)sx * by * nt * 128);
+      const double staged = (double)sx * by * rin * P / ((double)H * W);
+      if (eff > best + 1e-9 || (eff > best - 1e-9 && staged < best_rows - 1e-9)) {
+        best = eff; best_rows = staged; found = true;
+        g.TWo = two; g.Rout = rout; g.P = P; g.Rin = rin; g.ntiles = nt; g.strips_x = sx; g.blocks_y = by;
+        g.a_buf_bytes = a_buf; g.smem = halo_smem_bytes(a_buf, NC);
+      }
+    }
+  if (!found) return false;
+  g.pdiv_mul = (65536 + g.P - 1) / g.P;             // ty = (g * pdiv_mul) >> 16 == g / P for every position of a block
+  for (int k = 0; k < 128 * g.ntiles; ++k)
+    if (((k * g.pdiv_mul) >> 16) != k / g.P) return false;
+  return true;
+}
+
 }  // namespace tc
 }  // namespace lfsr
 
 using namespace lfsr;
 using namespace lfsr::tc;
+
+// Block plan of the halo-block kernel for an h x w fp16 image (lfsr.h): geom[0..7] = TWo, Rout, P, ntiles, strips_x,
+// blocks_y, input buffer bytes, dynamic shared memory bytes. Returns 1 when a plan exists.
+extern "C" int lfsr_conv_tc_halo_plan(int h, int w, int cout, int* geom) {
+  if (!geom || cout < 1) return 0;
+  const Plan pl = plan_for(64, cout, true);
+  if (pl.nchunks != 1) return 0;
+  HaloGeom g;
+  if (!plan_halo(h, w, pl.NC, g)) return 0;
+  const int v[8] = {g.TWo, g.Rout, g.P, g.ntiles, g.strips_x, g.blocks_y, g.a_buf_bytes, g.smem};
+  memcpy(geom, v, sizeof(v));
+  return 1;
+}
 
 extern "C" size_t lfsr_conv2d_tc_packed_floats(int kh, int kw, int cin, int cout) {
   if (kh <= 0 || kw <= 0 || cin <= 0 || cout <= 0) return 0;
@@ -1731,6 +1883,7 @@ static bool tc_geometry_ok(const lfsr_tensor* in, const lfsr_tensor* out, const 
   if (cout < 1) return false;
   if (d->tail_w) {      // tail projection: one cout-chunk whose sub-pixel blocks stay inside a 256-column accumulator stage
     if (ry * rx < 2 || d->tail_c < 4 || d->tail_c % 4 || d->tail_taps < 1 || d->tail_taps > 12 || out->c != d->tail_taps) return false;
+    if (!d->tail_w_host) return false;
     if ((cout > 256 && (d->tail_c % 32 || 256 % d->tail_c)) || (cout > 240 && d->tail_c % 32) || out->ld < 12 || out->ld % 4 || ((uintptr_t)out->ptr & 15) || ((uintptr_t)d->tail_w & 15)) return false;
     if (d->res.ptr || d->mul.ptr || sh > 1 || sw > 1 || d->block_h > 0 || d->block_w > 0) return false;
   }
@@ -1791,6 +1944,9 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
   p.bias = d->bias; p.act = d->act; p.slope = d->act_slope; p.alpha = d->alpha; p.mul_act = d->mul_act;
   p.ry = ry; p.rx = rx; p.shuf_mode = d->shuf_mode; p.cq = d->tail_w ? d->tail_c : out->c;
   p.tail_w = d->tail_w; p.tail_rows = d->tail_w ? (d->tail_c + 31) / 32 * 32 : 0;
+  TailW tt;                                        // the table by value (kernels with 16 epilogue warps read it from there)
+  memset(&tt, 0, sizeof(tt));
+  if (d->tail_w && p.cq <= kTailMaxC) memcpy(tt.w, d->tail_w_host, (size_t)p.cq * 12 * sizeof(float));
   // (a short last block of a sub-pixel run reads up to 31 accumulator columns past it: keep that inside the 256-column stage)
   if (d->tail_w)
     LFSR_REQUIRE((p.nchunks == 1 && (p.NC <= 240 || p.cq % 32 == 0)) ||
@@ -1825,83 +1981,9 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
         opt_in_smem(conv_tc_kernel<false, true, true>, 227 * 1024, w_) || opt_in_smem(conv_tc_kernel<true, true, true>, 227 * 1024, w_) ||
         opt_in_smem(conv_tc_kernel<true, true, true, true>, 227 * 1024, w_) ||
 #endif
-        opt_in_smem(conv_tc_halo_kernel, 227 * 1024, w_))
+        opt_in_smem(conv_tc_halo_kernel<true>, 227 * 1024, w_) || opt_in_smem(conv_tc_halo_kernel<false>, 227 * 1024, w_))
       return LFSR_ERR_CUDA;
     once.done();
-  }
-
-  // ---- halo-block plan: multi-tap kernels whose haloed input block fits in shared memory -------------
-  // Measured on B200 (profiles/r01_notes.md): correct, but not yet faster than the per-tap kernel below - the single
-  // accumulator stage at N = 224 serialises epilogue and MMAs - so it is opt-in (LFSR_TC_HALO=1) until that is fixed.
-  static const bool use_halo = dbg_env("LFSR_TC_HALO") != nullptr;
-  if (use_halo && !f16 && d->out_mode == 0 && !d->tail_w && d->w_batch_stride <= 0 && p.kh * p.kw > 1 && p.cgs <= 2 && p.nchunks == 1) {
-    const int taps = p.kh * p.kw, nks = taps * p.cgs;
-    const int kSmemAvail = 227 * 1024 - 1024 - 512 - 16 * 1024;
-    const int TWo = p.bw < 32 ? p.bw : 32;
-    const int P = TWo + 2 * p.pad_w;
-    double best = 0.0;
-    int bestR = 0;
-    for (int R = p.bh < 64 ? p.bh : 64; R >= 1; --R) {
-      const int Rin = R + 2 * p.pad_h;
-      if (Rin > 256 || P > 256) continue;
-      const int nt = ceil_div(R * P, 128);
-      if (nt * p.NC > 512) continue;
-      const long long a_bytes = ((long long)(128 * nt + 2 * p.pad_h * P + 2 * p.pad_w) * 128 + 1023) / 1024 * 1024;
-      const long long need = a_bytes * p.cgs + 2LL * p.b_stage_bytes;
-      if (need > kSmemAvail) continue;
-      // useful outputs per MMA row, times the fraction of loaded rows that are not halo, with a mild
-      // preference for blocks that tile the view height evenly
-      const int nblk = ceil_div(p.bh, R);
-      const double eff = ((double)p.bh * TWo / ((double)nblk * nt * 128)) * ((double)p.bh / ((double)nblk * Rin));
-      if (eff > best + 1e-9) { best = eff; bestR = R; }
-    }
-    if (bestR > 0 && best >= 0.35) {
-      p.halo = 1; p.TWo = TWo; p.P = P; p.Rout = bestR; p.Rin = bestR + 2 * p.pad_h;
-      p.ntiles = ceil_div(p.Rout * P, 128);
-      p.a_cg_bytes = (int)(((long long)(128 * p.ntiles + 2 * p.pad_h * P + 2 * p.pad_w) * 128 + 1023) / 1024 * 1024);
-      p.pdiv_mul = (65536 + P - 1) / P;
-      bool div_ok = true;
-      for (int g = 0; g < 128 * p.ntiles && div_ok; ++g) div_ok = ((g * p.pdiv_mul) >> 16) == g / P;
-      const long long b_all = (long long)nks * p.b_stage_bytes;
-      const long long left = kSmemAvail - (long long)p.a_cg_bytes * p.cgs;
-      p.resident = b_all <= left ? 1 : 0;
-      p.bstages = p.resident ? 0 : (int)(left / p.b_stage_bytes);
-      if (p.bstages > kMaxStages) p.bstages = kMaxStages;
-      p.acc_stages = 2 * p.ntiles * p.NC <= 512 ? 2 : 1;
-      p.strips_x = ceil_div(p.bw, TWo); p.blocks_y = ceil_div(p.bh, p.Rout);
-      const long long blocks = (long long)p.nb_total * p.blocks_y * p.nbx * p.strips_x;
-      if (div_ok && (p.resident || p.bstages >= 2) && blocks < 0x7fffffffLL) {
-        p.total_blocks = (int)blocks;
-        CUtensorMap tmA, tmB;
-        const cuuint64_t ld_b = (cuuint64_t)in->ld * 4;
-        {
-          cuuint64_t dims[5] = {(cuuint64_t)p.C, (cuuint64_t)p.bw, (cuuint64_t)p.nbx, (cuuint64_t)p.bh, (cuuint64_t)p.nb_total};
-          cuuint64_t strides[4] = {ld_b, ld_b * p.bw, ld_b * in->w, ld_b * in->w * p.bh};
-          cuuint32_t box[5] = {32, (cuuint32_t)p.P, 1, (cuuint32_t)p.Rin, 1};
-          cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-          CUresult r = encode(&tmA, CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, 5, in->ptr, dims, strides, box, estr,
-                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-          if (r != CUDA_SUCCESS) { set_error("lfsr_conv2d_tc: cuTensorMapEncodeTiled(A halo) failed with %d", (int)r); return LFSR_ERR_CUDA; }
-        }
-        {
-          cuuint64_t dims[2] = {32, (cuuint64_t)nks * p.NC};
-          cuuint64_t strides[1] = {128};
-          cuuint32_t box[2] = {32, (cuuint32_t)p.NC};
-          cuuint32_t estr[2] = {1, 1};
-          CUresult r = encode(&tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(w_packed_tc), dims, strides, box, estr,
-                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-          if (r != CUDA_SUCCESS) { set_error("lfsr_conv2d_tc: cuTensorMapEncodeTiled(B halo) failed with %d", (int)r); return LFSR_ERR_CUDA; }
-        }
-        const size_t smem = 1024 + (size_t)p.cgs * p.a_cg_bytes + (size_t)(p.resident ? nks : p.bstages) * p.b_stage_bytes +
-                            16 * 1024 + (4 + 2 * kMaxStages + 5) * 8 + 16;
-        const int grid = p.total_blocks < sm_count ? p.total_blocks : sm_count;
-        conv_tc_halo_kernel<<<grid, kHaloThreads, smem, (cudaStream_t)stream>>>(tmA, tmB, p);
-        return check_launch("conv_tc_halo_kernel");
-      }
-      p.halo = 0;
-    }
   }
 
   // tile shape TH x TW = 128 minimising padding waste inside a block (prefer wide tiles)
@@ -2119,6 +2201,65 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
                                        "multiples of 8, 16-byte aligned rows, no residual + multiplier pair)");
   }
   static const bool verbose = dbg_env("LFSR_TC_VERBOSE") != nullptr;
+  // ---- halo-block CTA pairs (conv_tc_halo_kernel): fp16 3x3 stride-1 dilation-1 "same" convs over whole images (the
+  // upsampler convs) with 128 < N <= 256 in one chunk, ending in the tail projection or writing fp16 only ----------------
+  {
+    static const bool no_halo = dbg_env("LFSR_TC_NO_HALO") != nullptr;     // A/B switch (profiles/ experiments)
+    const int r2 = ry * rx;
+    const bool tail_ok = p.tail_w && r2 >= 4 && r2 % 4 == 0 && p.cq <= kTailMaxC;
+    const bool f16out_ok = !p.tail_w && d->out_mode == 2 && p.tma_epi;      // (tma_epi: every column block is 8-aligned)
+    HaloGeom hg;
+    const bool halo = !no_halo && f16 && !per_image_w && p.kh == 3 && p.kw == 3 && !strided && p.dil_h == 1 && p.dil_w == 1 &&
+                      p.pad_h == 1 && p.pad_w == 1 && p.nby == 1 && p.nbx == 1 && p.cgs == 1 && p.nchunks == 1 && p.NC > 128 &&
+                      !d->res.ptr && !d->mul.ptr && (tail_ok || f16out_ok) && !p.dbg && sm_count >= 2 &&
+                      plan_halo(p.bh, p.bw, p.NC, hg) &&
+                      (long long)in->n * hg.blocks_y * hg.strips_x < 0x7fffffffLL;
+    if (halo) {
+      p.TWo = hg.TWo; p.Rout = hg.Rout; p.P = hg.P; p.Rin = hg.Rin; p.ntiles = hg.ntiles; p.strips_x = hg.strips_x;
+      p.blocks_y = hg.blocks_y; p.a_buf_bytes = hg.a_buf_bytes; p.pdiv_mul = hg.pdiv_mul;
+      p.total_blocks = in->n * hg.blocks_y * hg.strips_x;
+      p.fd_strips = make_fastdiv(hg.strips_x); p.fd_blocks_y = make_fastdiv(hg.blocks_y);
+      CUtensorMap tmH;
+      {
+        const cuuint64_t ld_b = (cuuint64_t)in->ld * 2;
+        cuuint64_t dims[5] = {(cuuint64_t)p.C, (cuuint64_t)in->w, 1, (cuuint64_t)in->h, (cuuint64_t)in->n};
+        cuuint64_t strides[4] = {ld_b, ld_b * in->w, ld_b * in->w, ld_b * in->w * in->h};
+        cuuint32_t box[5] = {64, (cuuint32_t)p.P, 1, (cuuint32_t)p.Rin, 1};
+        cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+        CUresult r = encode(&tmH, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, in->ptr, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) { set_error("lfsr_conv2d_tc: cuTensorMapEncodeTiled(A halo) failed with %d", (int)r); return LFSR_ERR_CUDA; }
+      }
+      CUtensorMap tmWh;
+      {
+        cuuint64_t dims[2] = {32, (cuuint64_t)9 * p.NC};
+        cuuint64_t strides[1] = {128};
+        cuuint32_t box[2] = {32, (cuuint32_t)(p.NC / 2)};
+        cuuint32_t estr[2] = {1, 1};
+        CUresult r = encode(&tmWh, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(w_packed_tc), dims, strides, box, estr,
+                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) { set_error("lfsr_conv2d_tc: cuTensorMapEncodeTiled(B halo) failed with %d", (int)r); return LFSR_ERR_CUDA; }
+      }
+      const int pairs = (p.total_blocks + 1) / 2;
+      const int hgrid = 2 * (pairs < sm_count / 2 ? pairs : sm_count / 2);
+      if (verbose)
+        fprintf(stderr, "[lfsr tc halo] C=%d cout=%d NC=%d %dx%d block %dx%d P=%d ntiles=%d blocks=%d grid=%d tail=%d smem=%d\n",
+                p.C, p.cout, p.NC, p.bh, p.bw, p.Rout, p.TWo, p.P, p.ntiles, p.total_blocks, hgrid, p.tail_w != nullptr, hg.smem);
+      cudaLaunchConfig_t cfg;
+      memset(&cfg, 0, sizeof(cfg));
+      cfg.gridDim = dim3(hgrid); cfg.blockDim = dim3(kHaloThreads); cfg.dynamicSmemBytes = hg.smem; cfg.stream = (cudaStream_t)stream;
+      cudaLaunchAttribute attr[1];
+      attr[0].id = cudaLaunchAttributeClusterDimension;
+      attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+      cfg.attrs = attr; cfg.numAttrs = 1;
+      const cudaError_t le = p.tail_w ? cudaLaunchKernelEx(&cfg, conv_tc_halo_kernel<true>, tmH, tmWh, p, tt)
+                                      : cudaLaunchKernelEx(&cfg, conv_tc_halo_kernel<false>, tmH, tmWh, p, NoTailW{});
+      if (le != cudaSuccess) { set_error("lfsr_conv2d_tc: launch failed: %s", cudaGetErrorString(le)); return LFSR_ERR_CUDA; }
+      g_halo_launches.fetch_add(1);
+      return check_launch("conv_tc_halo_kernel");
+    }
+  }
   // ---- lean path (conv_tc_lean_kernel): narrow fp16 layers run as two independent CTAs per SM -------------------------
   {
     static const bool no_lean = dbg_env("LFSR_TC_NO_LEAN") != nullptr;
@@ -2193,7 +2334,7 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
   static const bool no_t16 = dbg_env("LFSR_TC_NO_T16") != nullptr;
   // sub-pixels per cout-chunk (all r2 of them with one chunk): a multiple of 4 keeps the four warp groups balanced
   const int subs_per_chunk = p.nchunks == 1 ? ry * rx : (p.cq > 0 ? p.NC / p.cq : 0);
-  const bool t16 = p.tail_w && !no_t16 && !p.twin && !p.pair && subs_per_chunk >= 4 && subs_per_chunk % 4 == 0;
+  const bool t16 = p.tail_w && !no_t16 && !p.twin && !p.pair && subs_per_chunk >= 4 && subs_per_chunk % 4 == 0 && p.cq <= kTailMaxC;
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = smem; cfg.stream = (cudaStream_t)stream;
@@ -2204,30 +2345,31 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
   cudaError_t le;
 #ifdef LFSR_DEBUG_HOOKS
   if (p.dbg && !f16)
-    le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, true, false>, tmA, tmB, tmBh, tmO, p)
-                : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, true, false>, tmA, tmB, tmBh, tmO, p);
+    le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, true, false>, tmA, tmB, tmBh, tmO, p, NoTailW{})
+                : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, true, false>, tmA, tmB, tmBh, tmO, p, NoTailW{});
   else if (p.dbg && f16 && p.cta2 && t16) {
     cfg.blockDim = dim3(18 * 32);
-    le = cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, true, true, true>, tmA, tmB, tmBh, tmO, p);
+    le = cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, true, true, true>, tmA, tmB, tmBh, tmO, p, tt);
   } else if (p.dbg)
-    le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, true, true>, tmA, tmB, tmBh, tmO, p)
-                : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, true, true>, tmA, tmB, tmBh, tmO, p);
+    le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, true, true>, tmA, tmB, tmBh, tmO, p, NoTailW{})
+                : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, true, true>, tmA, tmB, tmBh, tmO, p, NoTailW{});
   else
 #endif
   if (t16) {     // tail projection with 16 epilogue warps: every warp group owns whole sub-pixels of the chunk
     cfg.blockDim = dim3(18 * 32);
-    if (f16) le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false, true, true>, tmA, tmB, tmBh, tmO, p)
-                         : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false, true, true>, tmA, tmB, tmBh, tmO, p);
-    else le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false, false, true>, tmA, tmB, tmBh, tmO, p)
-                     : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false, false, true>, tmA, tmB, tmBh, tmO, p);
+    if (f16) le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false, true, true>, tmA, tmB, tmBh, tmO, p, tt)
+                         : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false, true, true>, tmA, tmB, tmBh, tmO, p, tt);
+    else le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false, false, true>, tmA, tmB, tmBh, tmO, p, tt)
+                     : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false, false, true>, tmA, tmB, tmBh, tmO, p, tt);
   } else if (f16)
-    le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false, true>, tmA, tmB, tmBh, tmO, p)
-                : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false, true>, tmA, tmB, tmBh, tmO, p);
+    le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false, true>, tmA, tmB, tmBh, tmO, p, NoTailW{})
+                : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false, true>, tmA, tmB, tmBh, tmO, p, NoTailW{});
   else
-    le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false, false>, tmA, tmB, tmBh, tmO, p)
-                : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false, false>, tmA, tmB, tmBh, tmO, p);
+    le = p.cta2 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false, false>, tmA, tmB, tmBh, tmO, p, NoTailW{})
+                : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false, false>, tmA, tmB, tmBh, tmO, p, NoTailW{});
   if (le != cudaSuccess) { set_error("lfsr_conv2d_tc: launch failed: %s", cudaGetErrorString(le)); return LFSR_ERR_CUDA; }
   return check_launch("conv_tc_kernel");
 }
 
 extern "C" uint64_t lfsr_conv_tc_lean_count(void) { return lfsr::tc::g_lean_launches.load(); }
+extern "C" uint64_t lfsr_conv_tc_halo_count(void) { return lfsr::tc::g_halo_launches.load(); }

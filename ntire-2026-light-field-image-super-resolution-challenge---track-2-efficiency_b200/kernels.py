@@ -53,6 +53,17 @@ def as_tensor(t: torch.Tensor, what: str = "tensor", f16: bool = False) -> N.Ten
 _NULL_T = N.Tensor(None, 0, 0, 0, 0, 0)
 
 
+def tail_host(t: torch.Tensor) -> torch.Tensor:
+    """host copy of a tail-projection table (lfsr_conv_desc.tail_w_host: the kernels take the table by value at launch).
+    Kept on the table itself and remade only when the table has been written since (tensor version counter), so the
+    device is read once per table, not once per launch."""
+    h = getattr(t, "_lfsr_host", None)
+    if h is None or h[0] != t._version:
+        h = (t._version, t.detach().float().cpu().contiguous())
+        t._lfsr_host = h
+    return h[1]
+
+
 @dataclass
 class PackedConv:
     """One convolution's constants, packed once per weight version.
@@ -241,6 +252,7 @@ class CudaOps:
         d.res = as_tensor(res, "conv.res") if res is not None else _NULL_T
         if tail is not None:
             d.tail_w, d.tail_taps, d.tail_c = tail[0].data_ptr(), tail[1], tail[2]
+            d.tail_w_host = tail_host(tail[0]).data_ptr()
         tin, tout = as_tensor(x, "conv.in"), as_tensor(out, "conv.out")
         if x.shape[3] != pc.cin:
             raise N.LfsrError(f"conv: input has {x.shape[3]} channels, weights expect {pc.cin}")
@@ -300,6 +312,7 @@ class CudaOps:
         d.res = as_tensor(res, "conv.res") if res is not None else _NULL_T
         if tail is not None:
             d.tail_w, d.tail_taps, d.tail_c = tail[0].data_ptr(), tail[1], tail[2]
+            d.tail_w_host = tail_host(tail[0]).data_ptr()
         in16 = x.dtype == torch.float16
         d.in_f16 = 1 if in16 else 0
         w = pc.w_tc16 if in16 else pc.w_tc

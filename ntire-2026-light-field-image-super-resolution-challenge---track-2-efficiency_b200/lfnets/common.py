@@ -44,7 +44,9 @@ def tail_table(w_head: torch.Tensor, channels: int, device) -> torch.Tensor:
     w = w_head.detach().float().cpu()
     t = torch.zeros(channels, 12, dtype=torch.float32)
     t[: w.shape[1], :9] = w[0].reshape(w.shape[1], 9)
-    return t.contiguous().to(device)
+    d = t.contiguous().to(device)
+    d._lfsr_host = (d._version, t.contiguous())       # (kernels.tail_host: the host copy the launches read)
+    return d
 
 
 def upsample_tail(net, ops, pk, cur, ch, cw, Y, width, LR, shuf_mode):
