@@ -83,15 +83,11 @@ struct Params {
   // 1: stride along x, dims (c, x%s, x/s, y, image); 2: stride along y, dims (c, x, y%s, y/s, image);
   // 3: stride along both, dims (c, x%s, x/s, y%s, image*y/s))
   int amode, out_rows_per_img;
-  int pair;                            // 1: launched as 2-CTA clusters that share every weight stage via TMA multicast
   int cta2;                            // 1: 2-CTA clusters run ONE tcgen05.mma.cta_group::2 (M = 256) per K-step: each CTA stages its own
                                        //    activation tile and HALF of the weight slice; the leader CTA issues for both
-  int twin;                            // 1: a CTA walks PAIRS of M-tiles: one streamed weight stage feeds two activation tiles and both
-                                       //    TMEM accumulator stages (weights are written to / read from shared memory half as often per MMA)
   int w_img_rows;                      // >0: per-image weight sets, this many packed rows apart (streamed B only)
   short tap_off[25][4];
   long long* dbg;                      // optional per-CTA cycle counters (profiles/ experiments), else null
-  int dbg_skip_a;                      // experiment (wrong results): only tap 0 loads its activation tile
   // halo-block CTA pairs (conv_tc_halo_kernel): blocks of Rout x TWo output pixels; a CTA stages its block's (Rout + 2) x P
   // input pixels (P = TWo + 2) once and each tap's A operand is that buffer read from a row-shifted descriptor, so MMA row m of
   // tile j is the flattened padded position g = 128 j + m = ty * P + tx (tx >= TWo: halo columns, never stored)
@@ -162,18 +158,6 @@ __device__ __forceinline__ void tma_store_5d(const CUtensorMap* map, const void*
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-// weights for a CTA pair: each CTA fetches half of the rows and the TMA unit writes them into BOTH CTAs' shared
-// memory (same offset) and signals both CTAs' mbarriers
-__device__ __forceinline__ void tma_load_2d_mc(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(mask) : "memory");
-}
 __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.arrive.release.aligned;\nbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
@@ -357,30 +341,14 @@ __device__ __forceinline__ bool next_tile(const Params& p, int i, int& m, int& c
     chunk = 0;
     return true;
   }
-  if (p.twin) {           // tiles 2*pair, 2*pair + 1 of pair = blockIdx + (i / 2) * gridDim; an odd tail gets a dummy partner
-    const int pr = (int)blockIdx.x + (i >> 1) * (int)gridDim.x;
-    if (2 * pr >= p.m_tiles) return false;
-    m = 2 * pr + (i & 1);
-    if (m >= p.m_tiles) m = -1;
-    chunk = 0;
-    return true;
-  }
   if (p.resident) {
     const int b = fdiv((int)blockIdx.x, p.fd_nchunks);
     chunk = (int)blockIdx.x - b * p.nchunks;
     m = b + i * fdiv((int)gridDim.x, p.fd_nchunks);
     return m < p.m_tiles;
   }
-  int t = blockIdx.x + i * gridDim.x;
-  if (p.pair) {
-    // both CTAs of a pair must step through the same number of stages: iterate while the pair's first CTA has work
-    // and clamp the partner to the last tile (its stores are suppressed through m < 0)
-    const int t0 = (int)(blockIdx.x & ~1u) + i * gridDim.x;
-    if (t0 >= p.total_tiles) return false;
-    if (t >= p.total_tiles) { chunk = (p.total_tiles - 1) - fdiv(p.total_tiles - 1, p.fd_nchunks) * p.nchunks; m = -1; return true; }
-  } else if (t >= p.total_tiles) {
-    return false;
-  }
+  const int t = blockIdx.x + i * gridDim.x;
+  if (t >= p.total_tiles) return false;
   m = fdiv(t, p.fd_nchunks);
   chunk = t - m * p.nchunks;
   return true;
@@ -860,7 +828,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const uint32_t raw = smem_u32(smem_raw);
   uint8_t* smem = smem_raw + (((raw + 1023u) & ~1023u) - raw);
   uint8_t* sA = smem;
-  uint8_t* sB = smem + p.stages * (p.twin ? 2 : p.kps) * kABytes;
+  uint8_t* sB = smem + p.stages * p.kps * kABytes;
   const int taps = p.kh * p.kw;
   const int nks = taps * p.cgs;
   float* sEpi = reinterpret_cast<float*>(sB + (CTA2 ? p.stages * p.kps * (p.b_stage_bytes >> 1)         // (half slices)
@@ -879,7 +847,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   if (!T16)
     for (int i = threadIdx.x; i < p.tail_rows * 12; i += (int)blockDim.x) sTail[i] = i < p.cq * 12 ? __ldg(p.tail_w + i) : 0.f;
   if (threadIdx.x == 0) {
-    for (int s = 0; s < p.stages; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, p.pair ? 2 : 1); }
+    for (int s = 0; s < p.stages; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, 1); }
     for (int a = 0; a < 2; ++a) { mbar_init(tfull + a, 1); mbar_init(tempty + a, CTA2 ? 2 * kEpiW : kEpiW); }
     mbar_init(bfull, 1);
     fence_barrier_init();
@@ -890,11 +858,11 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   }
   // warp roles: 0..7 epilogue, 8 TMA producer, 9 MMA issuer. The scheduler favours the highest warp id of a
   // sub-partition, so the latency-critical single-thread roles get the top ids (B300_MICROARCH: hi-wid-first).
-  if (CTA2 || p.pair) cluster_sync_all();      // (cta2: both CTAs are resident before the paired allocation is requested)
+  if (CTA2) cluster_sync_all();      // both CTAs are resident before the paired allocation is requested
   if (warp == kMmaWarp) { if (CTA2) tmem_alloc2(tmem_slot, kTmemCols); else tmem_alloc(tmem_slot, kTmemCols); }
   tc_fence_before();
   __syncthreads();
-  if (p.pair || CTA2) cluster_sync_all();     // the partner's barriers must be initialised before anything is multicast to them
+  if (CTA2) cluster_sync_all();     // the partner's barriers must be initialised before anything is multicast to them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
@@ -903,7 +871,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     if (elect_one()) {
       int s_ring = 0;
       uint32_t ph_ring = 0;
-      const int crank = p.pair ? (int)cluster_ctarank() : 0;
       const uint32_t stage_bytes = kABytes + (p.resident ? 0 : p.NC * 128);
       int m, chunk;
       if (p.resident && next_tile(p, 0, m, chunk)) {
@@ -934,25 +901,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           }
         }
       } else
-      if (p.twin) {        // stage = {A of tile 2p, A of tile 2p+1, one (tap, channel group) of B}; amode 0, streamed B, one chunk
-        int m1, c1;
-        for (int i = 0; next_tile(p, i, m, chunk); i += 2) {
-          next_tile(p, i + 1, m1, c1);
-          const TileCoord t0 = decode_tile(p, m, 0), t1 = decode_tile(p, m1, 0);
-          int cg = 0, tap = 0;
-          for (int ks = 0; ks < nks; ++ks) {
-            if (s_ring == p.stages) { s_ring = 0; ph_ring ^= 1; }
-            const int s = s_ring++;
-            mbar_wait(empty + s, ph_ring ^ 1);
-            mbar_expect_tx(full + s, 2u * kABytes + (uint32_t)p.NC * 128u);
-            const short* to = p.tap_off[tap];
-            tma_load_5d(sA + (2 * s) * kABytes, &tmA, full + s, cg * CG, t0.x0 + to[0], t0.vx + to[1], t0.y0 + to[2], t0.nb + to[3]);
-            tma_load_5d(sA + (2 * s + 1) * kABytes, &tmA, full + s, cg * CG, t1.x0 + to[0], t1.vx + to[1], t1.y0 + to[2], t1.nb + to[3]);
-            tma_load_2d(sB + s * p.b_stage_bytes, &tmB, full + s, 0, ks * p.NC);
-            if (++cg == p.cgs) { cg = 0; ++tap; }
-          }
-        }
-      } else
       for (int i = 0; next_tile(p, i, m, chunk); ++i) {
         const TileCoord tc_ = decode_tile(p, m, chunk);
         int cg = 0, tap = 0;
@@ -967,25 +915,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           const int s = s_ring++;
           mbar_wait(empty + s, ph_ring ^ 1);
           const int nsub = nks - ks < p.kps ? nks - ks : p.kps;
-#ifdef LFSR_DEBUG_HOOKS
-          const bool skip_a = p.dbg_skip_a == 1 ? i > 0 : (p.dbg_skip_a == 2 && tap > 0);
-#else
-          const bool skip_a = false;
-#endif
-          mbar_expect_tx(full + s, (uint32_t)nsub * (stage_bytes - (skip_a ? kABytes : 0)));
+          mbar_expect_tx(full + s, (uint32_t)nsub * stage_bytes);
           for (int u = 0; u < nsub; ++u) {
             const short* to = p.tap_off[tap];
             const int slot = s * p.kps + u;
-            if (!skip_a) tma_load_5d(sA + slot * kABytes, &tmA, full + s, cg * CG, b1 + to[0], b2 + to[1], b3 + to[2], b4 + to[3]);
-            if (!p.resident) {
-              if (p.pair) {        // my half of the rows, written into both CTAs of the pair
-                const int half_rows = p.NC >> 1;
-                tma_load_2d_mc(sB + slot * p.b_stage_bytes + crank * half_rows * 128, &tmBh, full + s, 0,
-                               w_row0 + (ks + u) * p.NC + crank * half_rows, (uint16_t)3);
-              } else {
-                tma_load_2d(sB + slot * p.b_stage_bytes, &tmB, full + s, 0, w_row0 + (ks + u) * p.NC);
-              }
-            }
+            tma_load_5d(sA + slot * kABytes, &tmA, full + s, cg * CG, b1 + to[0], b2 + to[1], b3 + to[2], b4 + to[3]);
+            if (!p.resident) tma_load_2d(sB + slot * p.b_stage_bytes, &tmB, full + s, 0, w_row0 + (ks + u) * p.NC);
             if (++cg == p.cgs) { cg = 0; ++tap; }
           }
         }
@@ -1057,44 +992,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           }
         }
       } else
-      if (p.twin) {
-        for (int i = 0; next_tile(p, i, m, chunk); i += 2, tcount += 2) {
-          const uint32_t aph = (tcount >> 1) & 1;
-          int cg_i = 0;
-          for (int ks = 0; ks < nks; ++ks) {
-            if (s_ring == p.stages) { s_ring = 0; ph_ring ^= 1; }
-            const int s = s_ring++;
-            long long tw0 = 0, tw1 = 0;
-            if (ks == 0) {                       // accumulator 0 drained by the epilogue of the previous pair's first tile
-              if ((DBG && p.dbg)) tw0 = clock64();
-              mbar_wait(tempty + 0, aph ^ 1);
-              if ((DBG && p.dbg)) dbg_acc_wait += clock64() - tw0;
-            }
-            if ((DBG && p.dbg)) tw0 = clock64();
-            mbar_wait(full + s, ph_ring);
-            if ((DBG && p.dbg)) { tw1 = clock64(); dbg_full_wait += tw1 - tw0; }
-            tc_fence_after();
-            const uint64_t a_d0 = a_desc0 + (uint64_t)(2 * s) * (kABytes >> 4), a_d1 = a_d0 + (uint64_t)(kABytes >> 4);
-            const uint64_t b_d = b_desc0 + (uint64_t)s * b_step;
-            const int ksteps = (cg_i == p.cgs - 1) ? ksteps_last : 4;
-            if (ks == 0) umma_stage<true, F16>(tmem_base, a_d0, b_d, idesc, ksteps);
-            else umma_stage<false, F16>(tmem_base, a_d0, b_d, idesc, ksteps);
-            if (ks == 0) {                       // ... and accumulator 1 by the epilogue of its second tile
-              if ((DBG && p.dbg)) tw0 = clock64();
-              mbar_wait(tempty + 1, aph ^ 1);
-              if ((DBG && p.dbg)) { const long long t = clock64() - tw0; dbg_acc_wait += t; tw1 += t; }
-              tc_fence_after();
-              umma_stage<true, F16>(tmem_base + kAccStride, a_d1, b_d, idesc, ksteps);
-            } else {
-              umma_stage<false, F16>(tmem_base + kAccStride, a_d1, b_d, idesc, ksteps);
-            }
-            if (++cg_i == p.cgs) cg_i = 0;
-            umma_commit(empty + s);
-            if (ks + 1 == nks) { umma_commit(tfull + 0); umma_commit(tfull + 1); }
-            if ((DBG && p.dbg)) dbg_mma += clock64() - tw1;
-          }
-        }
-      } else
       for (int i = 0; next_tile(p, i, m, chunk); ++i, ++tcount) {
         const uint32_t a = tcount & 1, aph = (tcount >> 1) & 1;
         long long tw0 = 0;
@@ -1133,8 +1030,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               if (++cg_i == p.cgs) cg_i = 0;
             }
           }
-          if (p.pair) umma_commit_mc(empty + s, (uint16_t)3);   // both CTAs must be done before either refills the stage
-          else umma_commit(empty + s);                       // frees the smem stage when these MMAs retire
+          umma_commit(empty + s);                            // frees the smem stage when these MMAs retire
           if (ks + p.kps >= nks) umma_commit(tfull + a);     // accumulator complete -> epilogue
           if ((DBG && p.dbg)) dbg_mma += clock64() - tw1;
         }
@@ -1194,7 +1090,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     }
   }
   __syncthreads();
-  if (p.pair || CTA2) cluster_sync_all();     // no CTA may exit while its partner can still multicast into it
+  if (CTA2) cluster_sync_all();     // no CTA may exit while its partner can still multicast into it
   if (warp == kMmaWarp) {
     __syncwarp();
     if (CTA2) tmem_dealloc2(tmem_base, kTmemCols); else tmem_dealloc(tmem_base, kTmemCols);
@@ -1964,8 +1860,7 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
       break;
   }
   p.b_stage_bytes = p.NC * 128;
-#ifdef LFSR_DEBUG_HOOKS      // probe build only (liblfsr_probe.so): cycle counters / deliberately wrong experiments
-  p.dbg_skip_a = getenv("LFSR_TC_DBG_SKIP_A") ? atoi(getenv("LFSR_TC_DBG_SKIP_A")) : 0;
+#ifdef LFSR_DEBUG_HOOKS      // probe build only (liblfsr_probe.so): cycle counters
   p.dbg = getenv("LFSR_TC_DBG_PTR") ? (long long*)strtoull(getenv("LFSR_TC_DBG_PTR"), nullptr, 0) : nullptr;
 #endif
   const int sm_count = sm_count_current();
@@ -2039,9 +1934,8 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
   LFSR_REQUIRE(p.stages >= 2, "lfsr_conv2d_tc: not enough shared memory for two stages");
   // wide layers whose weights are streamed (they do not fit next to the activation stages) are bound by shared-memory
   // traffic: per K=8 MMA the weight slice is written by TMA and read by the tensor core (2 x N x 32 B) next to 2 x 4 KB
-  // of activations. Walking M-tile PAIRS halves the weight writes per MMA: one stage = two activation tiles + one slice.
-  // CTA pairs with cta_group::2 MMAs (M = 256): each SM stages its own activation tile and HALF of the weight slice, the
-  // leader's MMA thread issues for both; unlike twin tiles this keeps both accumulator stages per SM (epilogue overlapped)
+  // of activations. CTA pairs with cta_group::2 MMAs (M = 256) halve the weight writes per MMA: each SM stages its own
+  // activation tile and HALF of the weight slice, the leader's MMA thread issues for both
   static const bool use_cta2 = dbg_env("LFSR_TC_NO_CTA2") == nullptr;
   p.cta2 = 0;
   static const int cta2_min_nc = dbg_env("LFSR_TC_CTA2_MIN_NC") ? atoi(dbg_env("LFSR_TC_CTA2_MIN_NC")) : 128;
@@ -2056,12 +1950,6 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
       static const int cta2_kps = dbg_env("LFSR_TC_CTA2_KPS") ? atoi(dbg_env("LFSR_TC_CTA2_KPS")) : 2;
       if (cta2_kps > 1 && nks >= cta2_kps && avail / (cta2_kps * per) >= 3) { p.kps = cta2_kps; p.stages = avail / (cta2_kps * per); if (p.stages > kMaxStages) p.stages = kMaxStages; }
     }
-  }
-  static const bool no_twin = dbg_env("LFSR_TC_NO_TWIN") != nullptr;
-  p.twin = 0;
-  if (!p.cta2 && !no_twin && !p.resident && !per_image_w && p.kps == 1 && p.nchunks == 1 && p.amode == 0 && p.NC >= 128 && p.m_tiles >= 4) {
-    const int st = (kSmemBudget - kEpiWarps * 4096 - tail_bytes - epi16_bytes) / (2 * kABytes + p.b_stage_bytes);
-    if (st >= 2) { p.twin = 1; p.stages = st > kMaxStages ? kMaxStages : st; }
   }
   CUtensorMap tmA, tmB;
   {
@@ -2084,8 +1972,7 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
       box[1] = 1; box[2] = p.TW; box[3] = 1; box[4] = p.TH;
     }
     cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    static const bool a_trunc = dbg_env("LFSR_TC_A_TRUNC") != nullptr;   // experiment: plain fp32 loads (MMA truncates)
-    CUresult r = encode(&tmA, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : (a_trunc ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32), 5, in->ptr, dims,
+    CUresult r = encode(&tmA, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, 5, in->ptr, dims,
                         strides, box, estr,
                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -2107,25 +1994,18 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { set_error("lfsr_conv2d_tc: cuTensorMapEncodeTiled(B) failed with %d", (int)r); return LFSR_ERR_CUDA; }
   }
-  const size_t smem = 1024 + (size_t)p.stages * (p.twin ? 2 : p.kps) * kABytes +
+  const size_t smem = 1024 + (size_t)p.stages * p.kps * kABytes +
                       (p.cta2 ? (size_t)p.stages * p.kps * (p.b_stage_bytes / 2) : (size_t)(p.resident ? nks : p.stages * p.kps) * p.b_stage_bytes) +
                       kEpiWarps * 4096 + (size_t)tail_bytes + (size_t)epi16_bytes + (2 * kMaxStages + 5) * 8 + 16;
   LFSR_REQUIRE(smem <= 227 * 1024, "lfsr_conv2d_tc: shared memory plan too large");
   int grid = p.total_tiles < sm_count ? p.total_tiles : sm_count;
-  if (p.twin && grid > (p.m_tiles + 1) / 2) grid = (p.m_tiles + 1) / 2;
   if (p.cta2) { const int clusters = (p.m_tiles + 1) / 2 < sm_count / 2 ? (p.m_tiles + 1) / 2 : sm_count / 2; grid = 2 * clusters; }
   if (p.resident && p.nchunks > 1) {
     grid = grid / p.nchunks * p.nchunks;                   // every CTA owns one cout-chunk for its lifetime
     if (grid < p.nchunks) grid = p.nchunks;
   }
-  // CTA pairs with multicast weights for wide streamed layers (weights are 64 % of their L2->SM traffic)
-  // (measured on B200: parity-green but no gain - 3.90 ms with and without at batch 64, the weight stages are L2 hits
-  //  that were not the limiter - so it is opt-in: LFSR_TC_PAIR=1)
-  static const bool use_pair = dbg_env("LFSR_TC_PAIR") != nullptr;
-  p.pair = (use_pair && !p.twin && !p.cta2 && !p.resident && !per_image_w && p.NC >= 128 && p.NC % 16 == 0 && grid >= 2 && p.nchunks == 1) ? 1 : 0;
   CUtensorMap tmBh = tmB;
-  if (p.pair || p.cta2) {
-    grid &= ~1;
+  if (p.cta2) {
     cuuint64_t rows = (cuuint64_t)p.nchunks * p.kh * p.kw * p.cgs * p.NC;
     cuuint64_t dims[2] = {32, rows};
     cuuint64_t strides[1] = {128};
@@ -2266,11 +2146,11 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
     const bool act_ok = p.act == LFSR_ACT_NONE || p.act == LFSR_ACT_RELU || p.act == LFSR_ACT_LRELU;
     // (a short last block is clipped by the output tensor map; the fp16 copy is stored as 16-byte runs of 8 channels)
     const bool cout_ok = d->out_mode == 0 ? p.cout % 4 == 0 : p.cout % 8 == 0;
-    bool lean = !no_lean && !p.cta2 && !p.twin && !p.pair && !p.tail_w && p.tma_epi && ry * rx == 1 && !d->mul.ptr && act_ok &&
+    bool lean = !no_lean && !p.cta2 && !p.tail_w && p.tma_epi && ry * rx == 1 && !d->mul.ptr && act_ok &&
                 p.nchunks == 1 && p.NC <= 64 && cout_ok && !p.dbg && p.m_tiles >= 2 * sm_count;
     if (verbose && !lean)
-      fprintf(stderr, "[lfsr tc lean] not eligible: cta2 %d twin %d pair %d tail %d tma_epi %d r2 %d mul %d act %d nchunks %d NC %d cout_ok %d dbg %d tiles %d\n",
-              p.cta2, p.twin, p.pair, p.tail_w != nullptr, p.tma_epi, ry * rx, d->mul.ptr != nullptr, p.act, p.nchunks, p.NC, (int)cout_ok,
+      fprintf(stderr, "[lfsr tc lean] not eligible: cta2 %d tail %d tma_epi %d r2 %d mul %d act %d nchunks %d NC %d cout_ok %d dbg %d tiles %d\n",
+              p.cta2, p.tail_w != nullptr, p.tma_epi, ry * rx, d->mul.ptr != nullptr, p.act, p.nchunks, p.NC, (int)cout_ok,
               p.dbg != nullptr, p.m_tiles);
     int l_kps = 0, l_stages = 0, l_res = 0;
     size_t l_smem = 0;
@@ -2329,18 +2209,18 @@ extern "C" int lfsr_conv2d_tc(const lfsr_tensor* in, const float* w_packed_tc, c
     }
   }
   if (verbose)
-    fprintf(stderr, "[lfsr tc] C=%d cout=%d NC=%d k=%dx%d tiles=%d grid=%d stages=%d kps=%d resident=%d pair=%d twin=%d cta2=%d TH=%d TW=%d vec=%d tma_epi=%d smem=%zu\n",
-            p.C, p.cout, p.NC, p.kh, p.kw, p.total_tiles, grid, p.stages, p.kps, p.resident, p.pair, p.twin, p.cta2, p.TH, p.TW, p.vec, p.tma_epi, smem);
+    fprintf(stderr, "[lfsr tc] C=%d cout=%d NC=%d k=%dx%d tiles=%d grid=%d stages=%d kps=%d resident=%d cta2=%d TH=%d TW=%d vec=%d tma_epi=%d smem=%zu\n",
+            p.C, p.cout, p.NC, p.kh, p.kw, p.total_tiles, grid, p.stages, p.kps, p.resident, p.cta2, p.TH, p.TW, p.vec, p.tma_epi, smem);
   static const bool no_t16 = dbg_env("LFSR_TC_NO_T16") != nullptr;
   // sub-pixels per cout-chunk (all r2 of them with one chunk): a multiple of 4 keeps the four warp groups balanced
   const int subs_per_chunk = p.nchunks == 1 ? ry * rx : (p.cq > 0 ? p.NC / p.cq : 0);
-  const bool t16 = p.tail_w && !no_t16 && !p.twin && !p.pair && subs_per_chunk >= 4 && subs_per_chunk % 4 == 0 && p.cq <= kTailMaxC;
+  const bool t16 = p.tail_w && !no_t16 && subs_per_chunk >= 4 && subs_per_chunk % 4 == 0 && p.cq <= kTailMaxC;
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = smem; cfg.stream = (cudaStream_t)stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = (p.pair || p.cta2) ? 2 : 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  attr[0].val.clusterDim.x = p.cta2 ? 2 : 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
   cudaError_t le;
 #ifdef LFSR_DEBUG_HOOKS

@@ -19,6 +19,7 @@
 namespace lfsr {
 
 constexpr int TH_W = 32, TH_H = 16, TH_CP = 20, TH_NP = TH_CP / 2;   // tile, pixel pitch (floats), output pairs
+constexpr int TH_PPT = 2, TH_NT = 512 / TH_PPT;                       // pixels per thread, threads per CTA
 
 struct ThinArgs {
   TView in, out, mul;    // mul: optional elementwise multiplier of the activated output (20 readable floats per pixel)
@@ -47,14 +48,14 @@ __device__ __forceinline__ void th_ldw(const float* row, f32x2* w) {
   }
 }
 
-// PPT = pixels per thread (same column, TH_H / PPT rows apart): every weight row read from shared memory is used for PPT
-// pixels. ncu on the PPT = 2 version: L1/TEX (shared-memory) pipe 80 % busy, issue slots 49 % - the weight-row
-// broadcasts bound it. PPT = 4 with 128-thread CTAs has 45 % fewer LDS per FFMA2 but half the warps per SM and measured
-// no faster (LFSR_THIN_PPT=4 selects it); PPT = 2 with 256 threads is the default.
-template <int CIN, int PPT>
-__global__ void __launch_bounds__(512 / PPT)
+// TH_PPT = pixels per thread (same column, TH_H / TH_PPT rows apart): every weight row read from shared memory is used for
+// TH_PPT pixels. ncu on this version: L1/TEX (shared-memory) pipe 80 % busy, issue slots 49 % - the weight-row broadcasts
+// bound it. 4 pixels per thread with 128-thread CTAs has 45 % fewer LDS per FFMA2 but half the warps per SM and measured
+// no faster (0.273 vs 0.261 ms per layer).
+template <int CIN>
+__global__ void __launch_bounds__(TH_NT)
 conv_thin_kernel(const __grid_constant__ ThinArgs a) {
-  constexpr int NT = 512 / PPT, RSTEP = TH_H / PPT;
+  constexpr int PPT = TH_PPT, NT = TH_NT, RSTEP = TH_H / PPT;
   extern __shared__ __align__(16) float th_smem[];
   __shared__ uint64_t bar;
   const int tid = threadIdx.x;
@@ -398,28 +399,19 @@ extern "C" int lfsr_conv2d_thin(const lfsr_tensor* in, const float* w_packed, co
   const size_t smem = thin_smem(in, d);
   const int blocks = out->n * a.tiles_x * a.tiles_y;
   cudaStream_t st = (cudaStream_t)stream;
-#define LAUNCH_THIN(CIN, PPT)                                                                                       \
+#define LAUNCH_THIN(CIN)                                                                                            \
   do {                                                                                                              \
     static DevOnce once;                                                                                            \
     if (once.need()) {                                                                                              \
-      if (opt_in_smem(conv_thin_kernel<CIN, PPT>, 110 * 1024, "lfsr_conv2d_thin")) return LFSR_ERR_CUDA;            \
+      if (opt_in_smem(conv_thin_kernel<CIN>, 110 * 1024, "lfsr_conv2d_thin")) return LFSR_ERR_CUDA;                 \
       once.done();                                                                                                  \
     }                                                                                                               \
-    conv_thin_kernel<CIN, PPT><<<blocks, 512 / PPT, smem, st>>>(a);                                                 \
+    conv_thin_kernel<CIN><<<blocks, TH_NT, smem, st>>>(a);                                                          \
   } while (0)
-  static const int ppt = dbg_env("LFSR_THIN_PPT") ? atoi(dbg_env("LFSR_THIN_PPT")) : 2;   // measured: 0.261 ms (2) vs 0.273 ms (4) per layer
-  if (ppt == 2) {
-    switch (in->c) {
-      case 16: LAUNCH_THIN(16, 2); break;
-      case 18: LAUNCH_THIN(18, 2); break;
-      default: LAUNCH_THIN(20, 2); break;
-    }
-  } else {
-    switch (in->c) {
-      case 16: LAUNCH_THIN(16, 4); break;
-      case 18: LAUNCH_THIN(18, 4); break;
-      default: LAUNCH_THIN(20, 4); break;
-    }
+  switch (in->c) {
+    case 16: LAUNCH_THIN(16); break;
+    case 18: LAUNCH_THIN(18); break;
+    default: LAUNCH_THIN(20); break;
   }
 #undef LAUNCH_THIN
   return check_launch("conv_thin_kernel");

@@ -79,53 +79,6 @@ def fp16_plan(ops) -> bool:
     return bool(USE_FP16_OPERANDS and getattr(ops, "fp16_operands", getattr(ops, "use_tc", False)) and hasattr(ops, "to_f16"))
 
 
-#: LFSR_BRANCH_STREAMS=1 runs independent branches of a stage on a second stream (measured +0.6 % on the Track-2 model:
-#: the kernels already fill the GPU, so it is off by default)
-USE_BRANCH_STREAMS = os.environ.get("LFSR_BRANCH_STREAMS", "0") == "1"
-_side_streams: Dict[str, "torch.cuda.Stream"] = {}
-
-
-class SideStream:
-    """`with fork(): ...` enqueues the body on a second CUDA stream that first waits for everything already enqueued on the
-    current stream; `fork.join()` makes the current stream wait for it. Works eagerly and inside CUDA-graph capture (the
-    side stream joins the capture through the event wait). With device=None (CPU test backend) it is a no-op."""
-
-    def __init__(self, device):
-        self.device = device if USE_BRANCH_STREAMS else None
-        self._ev = None
-        if self.device is not None:
-            key = str(device)
-            if key not in _side_streams:
-                _side_streams[key] = torch.cuda.Stream(device=device)
-            self.stream = _side_streams[key]
-
-    def __call__(self):
-        return self
-
-    def __enter__(self):
-        if self.device is None:
-            return self
-        ev = torch.cuda.Event()
-        ev.record(torch.cuda.current_stream(self.device))
-        self.stream.wait_event(ev)
-        self._ctx = torch.cuda.stream(self.stream)
-        self._ctx.__enter__()
-        return self
-
-    def __exit__(self, *exc):
-        if self.device is None:
-            return False
-        self._ev = torch.cuda.Event()
-        self._ev.record(self.stream)
-        self._ctx.__exit__(*exc)
-        return False
-
-    def join(self):
-        if self.device is not None and self._ev is not None:
-            torch.cuda.current_stream(self.device).wait_event(self._ev)
-            self._ev = None
-
-
 class LFNetBase(nn.Module):
     """forward(x[B,1,A*h,A*w] float32 cuda, info=None) -> [B,1,A*h*s,A*w*s] (train.py:291-313)."""
 

@@ -24,10 +24,6 @@ from .. import _native as N
 from .. import kernels as K
 from .common import LFNetBase, L1Loss, slots, tail_table
 
-#: LFSR_EPIT_FUSED=0 keeps BasicTrans on the ten separate launches (comparison / debugging)
-import os
-USE_FUSED_BASICTRANS = os.environ.get("LFSR_EPIT_FUSED", "1") != "0"
-
 
 def _c3(cin, cout):
     return nn.Conv3d(cin, cout, kernel_size=(1, 3, 3), padding=(0, 1, 1), bias=False)
@@ -68,7 +64,7 @@ class get_model(LFNetBase):
 
     def _pack(self, device, ops):
         from . import common
-        f16 = bool(common.USE_FP16_OPERANDS and USE_FUSED_BASICTRANS and hasattr(ops, "to_f16") and hasattr(ops, "pack_basictrans") and
+        f16 = bool(common.USE_FP16_OPERANDS and hasattr(ops, "to_f16") and hasattr(ops, "pack_basictrans") and
                    getattr(ops, "fp16_operands", getattr(ops, "use_tc", False)))
         pc = lambda w, b=None, **kw: K.pack_conv(w, b, device=device, **kw)
         c3 = lambda m: pc(m.weight[:, :, 0], pad=(1, 1), tc=True, tc16=f16)          # [co, ci, 1, 3, 3] -> 2-D 3x3

@@ -21,19 +21,12 @@ torch.cat / torch.split never materialise: branches read and write channel slice
 """
 from __future__ import annotations
 
-import os
-
 import torch
 import torch.nn as nn
 
 from .. import _native as N
 from .. import kernels as K
-from .common import LFNetBase, bn_affine, slots, tail_table, upsample_tail, SideStream, fp16_plan
-
-
-#: the EPI block with its depthwise taps as shifted-row tcgen05 MMAs (persistent kernel, 0.27 ms per stage at batch 64 against 0.34
-#: for the hybrid kernel); LFSR_EPI_MMA=0 keeps the hybrid (CUDA-core taps + tensor-core 1x1s)
-USE_EPI_MMA = os.environ.get("LFSR_EPI_MMA", "1") == "1"
+from .common import LFNetBase, bn_affine, slots, tail_table, upsample_tail, fp16_plan
 
 
 def _conv(cin, cout, k, **kw):
@@ -218,14 +211,10 @@ class get_model(LFNetBase):
             s["ang_hid"] = dwp.shape[1]
             s["ang_a4"] = pc(*pad_out(ab.attention["4"].weight, to=gs_))
             s["ang_cv"] = pc(*pad_out(ab.cross_view["0"].weight, to=gs_), pad=(1, 1))
-            # expand conv + PixelShuffle(A): output channels padded 18 -> 20 per sub-pixel (nn.PixelShuffle order keeps the
-            # A*A sub-pixels innermost), so that the layer writes whole 20-float slots through the TMA-store epilogue
-            we = ab.expand["0"].weight.detach().float().cpu()
-            ce = we.shape[0] // (A * A)
-            we = torch.cat([we.view(ce, A * A, *we.shape[1:]), we.new_zeros((gs_ - ce, A * A) + tuple(we.shape[1:]))], 0)
-            s["ang_ex"] = pc(we.reshape(gs_ * A * A, *we.shape[2:]), tc=True, tc_shuffle=(A, A, N.SHUF_CHANNEL_MAJOR))
-            # the same layer for the streaming kernel (lfsr_ang_expand): [A][A][cin][cout padded to gs], nn.PixelShuffle order
+            # expand conv 1x1 + PixelShuffle(A) for the streaming kernel (lfsr_ang_expand): [A][A][cin][cout padded to gs],
+            # nn.PixelShuffle order; the padded output channels make the layer write whole 20-float slots
             wx = ab.expand["0"].weight.detach().float().cpu()[:, :, 0, 0]            # [c*A*A + i*A + j, cin]
+            ce = wx.shape[0] // (A * A)
             wx = wx.view(ce, A, A, wx.shape[1]).permute(1, 2, 3, 0)                   # [i, j, cin, c]
             s["ang_exw"] = torch.cat([wx, wx.new_zeros(A, A, wx.shape[2], gs_ - ce)], 3).contiguous().to(device)
             s["ang_scale"] = float(ab.scale.detach().item())
@@ -236,9 +225,11 @@ class get_model(LFNetBase):
                                     pw_t(eb.epi_h["1"]), pw_t(eb.epi_v["1"]), pw_t(eb.epi_diag["1"]),
                                     pw_t(eb.fuse["0"])]).to(device)
             s["epi_klen"] = eb.epi_h["0"].weight.shape[-1]
-            # fp16 operand plan: pre-swizzled tensor-core operands of the all-MMA EPI kernel (None: not available)
+            # fp16 operand plan: pre-swizzled tensor-core operands of the all-MMA EPI kernel, its depthwise taps as shifted-row
+            # tcgen05 MMAs (0.27 ms per stage at batch 64 against 0.34 for the hybrid kernel). None when the packer does not
+            # take the kernel length (2A+1 > 15) or the backend has none: the hybrid kernel runs the block then
             s["epi_img"] = (ops.mel_epi_pack(s["epi_w"], s["epi_klen"], device)
-                            if (f16 and USE_EPI_MMA and hasattr(ops, "mel_epi_pack")) else None)
+                            if (f16 and hasattr(ops, "mel_epi_pack")) else None)
             # three gate FCs as one block-diagonal 1x1 over the grouped layout (MyEfficientLFNet.py:159-173)
             sp, gs = self._groups()
             CP = gs * len(sp)
@@ -313,7 +304,7 @@ class get_model(LFNetBase):
         shallow = shallow64[..., 0:CP] if f16 else buf("shallow", H, W, CP)
         # fp16 copy of the whole trunk (64-half pixels), written by the stem / the SA tail of the previous stage: channels 0..31 feed
         # the spatial branch's tensor-core convs, 40..57 the all-MMA EPI kernel
-        epi_mma = bool(f16) and pk["stages"][0].get("epi_img") is not None and gs + 12 <= CP
+        epi_mma = bool(f16) and pk["stages"][0].get("epi_img") is not None
         trunk16 = self._buf16("trunk16", B, H, W, 64, dev) if epi_mma else None
         if epi_mma:
             ops.conv(xin, pk["stem"], shallow, out16=trunk16[..., 0:CP])      # (the stem kernel writes the copy itself)
@@ -329,7 +320,6 @@ class get_model(LFNetBase):
         ang2, ang3 = buf("ang2", hA, wA, gs), buf("ang3", hA, wA, gs)
         vmean, gmean, gate = buf("vmean", A, A, CP), buf("gmean", 1, 1, CP), buf("gate", 1, 1, CP)
         CU = pk["CU"]
-        f16 = pk.get("f16")
         # fu1 (fusion 1x1 output) feeds nothing but the 3x3 that follows: fp16 only on the fp16 operand plan
         fu1 = self._buf16("fu1", B, H, W, CU, dev) if f16 else buf("fu1", H, W, CU)
         fu2 = buf("fu2", H, W, CP)
@@ -337,11 +327,10 @@ class get_model(LFNetBase):
             xs16 = trunk16[..., 0:32] if epi_mma else self._buf16("xs16", B, H, W, 32, dev)
             t18h = self._buf16("t18h", B, H, W, 32, dev)
         pm, am1, am = buf("pm", A, A, CP), buf("am1", A, A, C // 4), buf("am", A, A, CP)
-        fork = SideStream(dev if x.is_cuda and getattr(ops, "name", "") == "cuda" else None)
         for i, st in enumerate(pk["stages"]):
             xs, xa, xe = feat[..., sl[0]], feat[..., sl[1]], feat[..., sl[2]]
             # spatial branch
-            if f16 and gs + 12 <= CP:
+            if f16:
                 if i == 0:          # later stages: the SA modulator of the previous stage wrote the copy next to the trunk
                     if not epi_mma:
                         ops.to_f16(feat[..., 0:32], xs16)
@@ -350,26 +339,18 @@ class get_model(LFNetBase):
             else:
                 ops.conv(xs, st["spa0"], t18, act=LR, slope=0.1)
                 ops.conv(t18[..., 0:c0], st["spa2"], cat[..., 0:gs])
-            # angular branch: six small launches on 32x32 maps that do not fill the GPU - on a side stream (when the backend
-            # is the CUDA one) they run under the spatial / EPI kernels; the three branches write disjoint slots of `cat`
-            with fork():
-                ops.conv(xa, st["ang_to"], ang1)
-                ops.conv(ang1[..., 0:c0], st["ang_a0"], ang2, act=N.ACT_RELU)
-                ops.dwconv(ang2, st["ang_a2"], ang3, 3, 3, act=N.ACT_RELU)
-                ops.conv(ang3[..., 0:hid], st["ang_a4"], ang4, act=N.ACT_SIGMOID, mul=ang1)
-                ops.conv(ang4[..., 0:c0], st["ang_cv"], ang5, act=LR, slope=0.1)
-                if hasattr(ops, "ang_expand"):
-                    ops.ang_expand(ang5[..., 0:c0], st["ang_exw"], feat[..., gs:2 * gs], cat[..., gs:2 * gs], A, LR, 0.1,
-                                   st["ang_scale"])
-                else:
-                    ops.conv(ang5[..., 0:c0], st["ang_ex"], cat[..., gs:2 * gs], act=LR, slope=0.1, alpha=st["ang_scale"],
-                             res=feat[..., gs:2 * gs], shuffle=(A, A, N.SHUF_CHANNEL_MAJOR))
+            # angular branch
+            ops.conv(xa, st["ang_to"], ang1)
+            ops.conv(ang1[..., 0:c0], st["ang_a0"], ang2, act=N.ACT_RELU)
+            ops.dwconv(ang2, st["ang_a2"], ang3, 3, 3, act=N.ACT_RELU)
+            ops.conv(ang3[..., 0:hid], st["ang_a4"], ang4, act=N.ACT_SIGMOID, mul=ang1)
+            ops.conv(ang4[..., 0:c0], st["ang_cv"], ang5, act=LR, slope=0.1)
+            ops.ang_expand(ang5[..., 0:c0], st["ang_exw"], feat[..., gs:2 * gs], cat[..., gs:2 * gs], A, LR, 0.1, st["ang_scale"])
             # EPI branch: three depthwise+pointwise paths and their fuse conv in one kernel
             if f16 and epi_mma:
                 ops.mel_epi_branch_mma(xe, trunk16[..., 2 * gs:2 * gs + sp[2]], st["epi_img"], cat[..., sl[2]], st["epi_klen"], A, 0.1)
             else:
                 ops.mel_epi_branch(xe, st["epi_w"], cat[..., sl[2]], st["epi_klen"], A, 0.1, tc=bool(f16))
-            fork.join()
             # gates -> per-sample channel scale of the fusion 1x1
             ops.block_mean(cat, vmean, hA, wA)
             ops.pooled_mlp(vmean, gate, st["gate"], N.ACT_SIGMOID, pool=True)      # mean over the views -> FC + sigmoid
@@ -382,7 +363,7 @@ class get_model(LFNetBase):
             ops.block_mean(fu2, pm, hA, wA)
             ops.pooled_mlp(pm, am, st["sa_c0"], N.ACT_RELU, st["sa_c2"], N.ACT_SIGMOID)
             nxt = pp[i & 1]
-            if f16 and gs + 12 <= CP and i + 1 < len(pk["stages"]):
+            if f16 and i + 1 < len(pk["stages"]):
                 ops.sa_modulate(fu2, st["sa_dw"], st["sa_bns"], st["sa_bnb"], am, st["sa_w"][0], st["sa_w"][1], feat, nxt, A,
                                 out16=trunk16[..., 0:CP] if epi_mma else xs16)
                 # (leaving the unread channels 20..39 out of the copy - skip16=(gs, 2 * gs) - was SLOWER, 0.397 vs 0.347 ms per

@@ -1,5 +1,5 @@
 """The fused EPIT BasicTrans kernel on its production shape (B patches of 5x5x32x32, 64 channels): CUDA-event time per call,
-useful TFLOP/s (SURVEY 8d: 4.8235 GMAC per call per patch), and the whole EPIT forward with / without it.
+useful TFLOP/s (SURVEY 8d: 4.8235 GMAC per call per patch), and the whole EPIT forward.
 usage: python profiles/run_basictrans.py [batch] [forward: 0|1]"""
 import os, sys, time
 import torch
@@ -49,4 +49,4 @@ if do_fwd:
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / 3
-    print(f"EPIT forward batch {B} (LFSR_EPIT_FUSED={os.environ.get('LFSR_EPIT_FUSED', '1')}): {ms:.2f} ms, {B / ms * 1e3:.0f} patches/s")
+    print(f"EPIT forward batch {B}: {ms:.2f} ms, {B / ms * 1e3:.0f} patches/s")

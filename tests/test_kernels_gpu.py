@@ -576,20 +576,6 @@ def test_conv_tc(ref, case):
     _run_tc_case(ref, case)
 
 
-@pytest.mark.parametrize("switch", ["LFSR_TC_HALO", "LFSR_TC_PAIR"])
-def test_conv_tc_halo_block_kernel(ref, switch):
-    """the opt-in variants (halo-block kernel, CTA-pair weight multicast) in a subprocess so the env switch is seen
-    at first use"""
-    import subprocess, sys, os
-    env = dict(os.environ, **{switch: "1"})
-    code = ("import sys; sys.path[:0]=['.','tests']; import torch, opref, test_kernels_gpu as t; "
-            "torch.backends.cudnn.allow_tf32=False; torch.backends.cuda.matmul.allow_tf32=False; r=opref.RefOps();\n"
-            "for c in t.TC_CASES:\n    if c['k']==(3,3) and c['cin']<=64: t._run_tc_case(r, c)\nprint('halo ok')")
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600,
-                         cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    assert out.returncode == 0 and "halo ok" in out.stdout, out.stderr[-2000:]
-
-
 def _run_tc_case(ref, case):
     tc_ops = K.CudaOps(use_tc=True)
     n = 2
@@ -1015,9 +1001,9 @@ def test_colour_tail_and_bmp_vs_reference_golden(golden_dir, tmp_path):
 
 
 @pytest.mark.parametrize("tail", [False, True])
-def test_conv_tc_twin_tiles_odd_count(ref, tail):
-    """wide streamed-weight layers walk M-tile pairs (one weight stage feeds two tiles / both accumulator stages): an odd
-    number of 128-pixel tiles leaves a dummy partner whose stores must be suppressed"""
+def test_conv_tc_cta2_odd_tile_count(ref, tail):
+    """wide streamed-weight layers run on CTA pairs (one cta_group::2 MMA over two 128-pixel tiles): an odd number of tiles
+    leaves the last pair a dummy partner, which must store nothing"""
     tc_ops = K.CudaOps(use_tc=True)
     n, h, w, cin, cq, r = 3, 20, 32, 64, 64, 2          # 3 * 5 * 1 = 15 tiles, weights 590 KB -> streamed
     g = torch.Generator().manual_seed(5)

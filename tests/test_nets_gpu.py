@@ -102,17 +102,17 @@ def test_forward_batch64_default_init_vs_oracle(name, scale):
     assert worst <= TOL and worst_dp <= 0.01, (worst, worst_dp)
 
 
-def test_epi_branch_hybrid_variant_matches_default(monkeypatch):
-    """LFSR_EPI_MMA=0 (depthwise taps of the EPI block on the CUDA cores, 1x1s on tcgen05) against the default plan (taps as
-    shifted-row tcgen05 MMAs over the fp16 trunk copy the SA tail writes): same network output to well inside the tolerance"""
-    import sys
+def test_epi_branch_packer_fallback_matches_default(monkeypatch):
+    """the hybrid EPI block (depthwise taps on the CUDA cores, 1x1s on tcgen05), which runs when the operand packer returns
+    None, against the default plan (taps as shifted-row tcgen05 MMAs over the fp16 trunk copy the SA tail writes): same
+    network output to well inside the tolerance"""
     torch.manual_seed(1234)
     net = lfsr_b200.load_net("MyEfficientLFNet", 5, 4).eval().to(DEV)
-    mod = sys.modules[type(net).__module__]          # (the package is importable under two names)
-    assert mod.USE_EPI_MMA
     x = weights.synthetic_patches(4, 5, 32, seed=9).to(DEV)
     y0 = net(x, [5, 5]).clone()
-    monkeypatch.setattr(mod, "USE_EPI_MMA", False)
+    ops = net._backend(x)          # (the package is importable under two names: patch the instance the net uses)
+    assert all(st["epi_img"] is not None for st in net._get_packed(x.device, ops)["stages"])
+    monkeypatch.setattr(ops, "mel_epi_pack", lambda *a, **k: None)
     net.invalidate()
     y1 = net(x, [5, 5]).clone()
     d = float((y0 - y1).abs().max())
